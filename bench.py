@@ -3,6 +3,7 @@
 
   python bench.py --gpus 1 --steps 20 --warmup 3            # this repo's CUDA path (one JSON line)
   python bench.py --impl reference --steps 3 --warmup 1     # CPU arm: restated reference algorithm on host cores
+  python bench.py --gpus 1 --steps 20 --dump-outputs DIR    # also write a sample of the last timed step's outputs as DIR/*.npy
   python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 --master-port P \
          bench.py --gpus 8 --steps 20 --warmup 3            # one rank per GPU, rods sharded by index, no collective
 
@@ -30,6 +31,7 @@ from pathlib import Path
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True  # the tree this runs from may be read-only; it writes nothing there
 
 import numpy as np  # noqa: E402
 
@@ -44,6 +46,7 @@ EXECUTED_NOTE = ("215 DMMA m8n8k4 (512 flop each) per rod: 176 rank-4 updates, 2
                  "(position and force share one); dead columns and padding included")
 PEAK_NOMINAL_TFLOPS = 37.2  # 148 SM x 64 FP64 FMA/clk x 2 x 1.965 GHz
 BYTES_PER_ROD = 1_992 + 3 * N_NODES * 8  # compulsory HBM traffic incl. the nodal fbar this workload supplies
+DUMP_RODS = 16_384  # rods in the --dump-outputs sample: 16384 x (Q, r, n, m, info) = 26 MB of float64
 
 
 def _config(rods: int, world: int) -> dict:
@@ -65,7 +68,15 @@ def _parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="target CPU time of the cpu_baseline sample")
     ap.add_argument("--no-side-configs", action="store_true", help="skip other_configs (cfg2, cfg3_strong, cfg4, cfg5)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write Q, r, n, m and info of the last step for a fixed, seeded sample of rank 0's "
+                         f"rods (at most {DUMP_RODS}; rod_index names them) as DIR/<name>.npy in float64")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU arm (--impl b200)")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------------------------
@@ -252,6 +263,21 @@ def _bind_to_gpu_numa_node(torch, local_rank: int):
         return None
 
 
+def dump_outputs(out_dir: str, torch, outs: dict, first_rod: int) -> None:
+    """Writes the rows of a fixed, seeded sample of the batch (all of it when it has at most DUMP_RODS rods) as
+    out_dir/<name>.npy in float64, with rod_index = the global rod index of each row.  The sample depends on the batch
+    size alone, so two builds run with the same arguments can be compared output for output."""
+    any_out = next(iter(outs.values()))
+    B = any_out.shape[0]
+    rows = np.sort(np.random.default_rng(SEED).choice(B, size=min(B, DUMP_RODS), replace=False))
+    sel = torch.from_numpy(rows).to(any_out.device)
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    for name, t in outs.items():
+        np.save(out / f"{name}.npy", t.index_select(0, sel).cpu().numpy().astype(np.float64))
+    np.save(out / "rod_index.npy", (first_rod + rows).astype(np.float64))
+
+
 def _max_over_ranks(torch, dist, world, dev, x: float) -> float:
     if world == 1:
         return x
@@ -329,6 +355,8 @@ def run_b200(args, rank: int, world: int, local_rank: int):
     ms_step = mx(e0.elapsed_time(e1)) / args.steps
     value = world * B / (ms_step * 1e-3)
     assert int(info.abs().sum().item()) == 0, "zero pivot reported on the synthetic workload"
+    if args.dump_outputs is not None and rank == 0:  # before the legs below reuse Q, r, n, m
+        dump_outputs(args.dump_outputs, torch, {"Q": Q, "r": r, "n": n, "m": m, "info": info}, first)
 
     # ---- end to end through the C ABI with HOST buffers (pinned), H2D + D2H inside the timed region, and beside it the bare
     #      concurrent copies of the very same buffers on all ranks (the ceiling the host platform allows this call)

@@ -4,10 +4,12 @@ Build products go to oracle/_ref/ (git-ignored, shipped to the GPU box with the 
 """
 from __future__ import annotations
 
+import atexit
 import ctypes
 import os
 import shutil
 import subprocess
+import tempfile
 from ctypes import c_double, c_int, c_long, c_void_p
 from pathlib import Path
 
@@ -16,23 +18,31 @@ import numpy as np
 ORACLE_DIR = Path(__file__).resolve().parent
 REF_DIR = ORACLE_DIR / "_ref"
 SRC = ORACLE_DIR / "sri_oracle.c"
+_native_dir = None
 
 
 def oracle_lib_path(native: bool = False) -> Path:
-    return REF_DIR / ("libsri_oracle_native.so" if native else "libsri_oracle.so")
+    if not native:
+        return REF_DIR / "libsri_oracle.so"
+    global _native_dir
+    if _native_dir is None:
+        _native_dir = Path(tempfile.mkdtemp(prefix="sri_oracle_native_"))
+        atexit.register(shutil.rmtree, _native_dir, True)
+    return _native_dir / "libsri_oracle_native.so"
 
 
 def build_oracle(force: bool = False, native: bool = False) -> Path:
-    """gcc on oracle/sri_oracle.c -> oracle/_ref/libsri_oracle[_native].so.
+    """gcc on oracle/sri_oracle.c -> oracle/_ref/libsri_oracle.so.
 
     The default (checker) build is portable: generic x86-64, no FMA contraction, so its arithmetic is plain IEEE
-    and identical on the build container and on the GPU box.  native=True adds -march=native and is rebuilt on
-    the host that runs it; bench.py uses it for the timed CPU baseline only.
+    and identical on every x86-64 host.  native=True adds -march=native and is rebuilt on the host that runs it,
+    in a temporary directory of this process (the tree it runs from may be read-only); bench.py uses it for the
+    timed CPU baseline only.
     """
     out = oracle_lib_path(native)
     if not force and not native and out.exists() and out.stat().st_mtime >= SRC.stat().st_mtime:
         return out
-    REF_DIR.mkdir(exist_ok=True)
+    out.parent.mkdir(exist_ok=True)
     gcc = shutil.which("gcc") or "gcc"
     flags = ["-O3", "-march=native"] if native else ["-O3", "-ffp-contract=off"]
     cmd = [gcc, *flags, "-fopenmp", "-fPIC", "-shared", "-o", str(out), str(SRC), "-lm"]

