@@ -39,6 +39,16 @@ class RodBatch(ctypes.Structure):
     ]
 
 
+class RodBatchGrad(ctypes.Structure):
+    """struct sri_rod_batch_grad (include/sri.h)."""
+
+    _fields_ = [
+        ("gQ", c_void_p), ("gr", c_void_p), ("gn", c_void_p), ("gm", c_void_p),
+        ("gK", c_void_p), ("gq0", c_void_p), ("gr0", c_void_p), ("gGamma", c_void_p),
+        ("gfbar", c_void_p), ("glbar", c_void_p), ("gF_tip", c_void_p), ("gM_tip", c_void_p),
+    ]
+
+
 class NewtonReport(ctypes.Structure):
     """struct sri_newton_report (include/sri.h)."""
 
@@ -65,6 +75,7 @@ SYMBOLS = {
     "sri_get_N": (c_int, [c_void_p, POINTER(c_int)]),
     "sri_get_operator": (c_int, [c_void_p, c_int, c_void_p]),
     "sri_strain_from_modes": (c_int, [c_void_p, c_int64, c_int, c_void_p, c_void_p]),
+    "sri_strain_from_modes_transpose": (c_int, [c_void_p, c_int64, c_int, c_void_p, c_void_p]),
     "sri_assemble_A": (c_int, [c_void_p, c_int64, c_void_p, c_void_p]),
     "sri_scale_for_length": (c_int, [c_void_p, c_int64, c_void_p, c_double, c_void_p, c_void_p, c_void_p, c_void_p]),
     "sri_device_count": (c_int, [POINTER(c_int)]),
@@ -86,6 +97,7 @@ SYMBOLS = {
     "sri_integrate_stress": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p]),
     "sri_integrate_couple": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "sri_integrate_all": (c_int, [c_void_p, POINTER(RodBatch)]),
+    "sri_integrate_all_vjp": (c_int, [c_void_p, POINTER(RodBatch), POINTER(RodBatchGrad)]),
     "sri_shape_residual": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "sri_wrench_local": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "sri_integrate_wrench_local": (c_int, [c_void_p, c_int64] + [c_void_p] * 10),

@@ -183,6 +183,16 @@ class SpectralRodIntegrator:
         _lib.check(self._lib.sri_strain_from_modes(self._h, batch, ne, _ptr(qe, "qe"), _ptr(K, "K")), "sri_strain_from_modes")
         return K
 
+    def strain_from_modes_transpose(self, gK, ne: int, out=None):
+        """gK [batch][3][N] -> gqe [batch][3*ne] = sum_i P_k(2 x_i - 1) gK[b][c][i] (the transpose of strain_from_modes,
+        no quadrature weights), 1 <= ne <= 8."""
+        self._follow_torch(gK)
+        batch = gK.shape[0]
+        gqe = out if out is not None else _empty_like_kind(gK, (batch, 3 * int(ne)))
+        _lib.check(self._lib.sri_strain_from_modes_transpose(self._h, batch, int(ne), _ptr(gK, "gK"), _ptr(gqe, "gqe")),
+                   "sri_strain_from_modes_transpose")
+        return gqe
+
     def scale_for_length_(self, length, K=None, Gamma=None, fbar=None, lbar=None) -> None:
         """sri_scale_for_length: scales the given [batch][3][N] arrays IN PLACE by the rod length (a float, or one value per rod as
         an array / tensor).  See scale_for_length() for the out-of-place convenience form."""
@@ -290,6 +300,26 @@ class SpectralRodIntegrator:
         )
         _lib.check(self._lib.sri_integrate_all(self._h, ctypes.byref(rb)), "sri_integrate_all")
         return {k: v for k, v in outs.items() if v is not None}
+
+    def integrate_all_vjp(self, K, Q, n=None, q0=None, Gamma=None, gQ=None, gr=None, gn=None, gm=None, info=None,
+                          want=("K", "q0", "r0", "Gamma", "fbar", "lbar", "F_tip", "M_tip"), out=None):
+        """sri_integrate_all_vjp: gradients of <gQ,Q> + <gr,r> + <gn,n> + <gm,m> with respect to the inputs named in `want`,
+        from the forward's Q (and n, needed with gm).  Cotangents may be None (zero).  Returns a dict of the requested
+        gradients (allocated unless given in the dict `out`)."""
+        self._follow_torch(K)
+        batch, N = K.shape[0], self.N
+        shapes = {"K": (batch, 3, N), "q0": (batch, 4), "r0": (batch, 3), "Gamma": (batch, 3, N), "fbar": (batch, 3, N),
+                  "lbar": (batch, 3, N), "F_tip": (batch, 3), "M_tip": (batch, 3)}
+        given = out or {}
+        grads = {key: given[key] if given.get(key) is not None else _empty_like_kind(K, shapes[key]) for key in want}
+        rb = _lib.RodBatch(batch=batch, K=_ptr(K, "K"), q0=_ptr(q0, "q0"), Gamma=_ptr(Gamma, "Gamma"), Q=_ptr(Q, "Q"),
+                           n=_ptr(n, "n"), info=_ptr(info, "info", np.int32))
+        g = lambda key: _ptr(grads.get(key), "grad " + key)
+        gb = _lib.RodBatchGrad(gQ=_ptr(gQ, "gQ"), gr=_ptr(gr, "gr"), gn=_ptr(gn, "gn"), gm=_ptr(gm, "gm"), gK=g("K"),
+                               gq0=g("q0"), gr0=g("r0"), gGamma=g("Gamma"), gfbar=g("fbar"), glbar=g("lbar"),
+                               gF_tip=g("F_tip"), gM_tip=g("M_tip"))
+        _lib.check(self._lib.sri_integrate_all_vjp(self._h, ctypes.byref(rb), ctypes.byref(gb)), "sri_integrate_all_vjp")
+        return {k: v for k, v in grads.items() if v is not None}
 
     def shape_residual(self, K, H_diag, Q, m, M_tip, K0=None, q0=None, rho=None, reduce=None):
         self._follow_torch(K)

@@ -30,6 +30,8 @@
 #include "sri_stage_tma.cuh"
 #include "sri_tiled.cuh"
 #include "sri_tiled_dmma.cuh"
+#include "sri_vjp16.cuh"
+#include "sri_vjp_tiled.cuh"
 #include "sri_wrench_generic.cuh"
 #include "sri_wrench_gj.cuh"
 #include "sri_wrench_gj_multi.cuh"
@@ -84,8 +86,10 @@ struct sri_context {
     double* d_reduce = nullptr;  // 2 doubles: sum rho^2, max |rho|
     double* d_ccw = nullptr;     // Clenshaw-Curtis weights of the nodes, [N]
     double* d_ptab = nullptr;    // Legendre polynomials at the nodes, P_k(2 x_i - 1), [8][N]
-    double* d_jac = nullptr;     // S = Dn_NN^-1 and S_T = D_TT^-1, row-major [M][M] each (sri_shape_jacobian), built on first use
+    double* d_jac = nullptr;     // S = Dn_NN^-1 and S_T = D_TT^-1, row-major [M][M] each (sri_shape_jacobian, sri_integrate_all_vjp), built on first use
     double* d_dnn = nullptr;     // Dn_NN, column-major [M][M] (sri_assemble_A), built on first use
+    double* d_dnin = nullptr;    // Dn_IN [M] (sri_integrate_all_vjp), built on first use
+    int vjp_occ = 0;             // resident CTAs per SM of the reverse-mode kernel of this N
     double* d_wrench_scratch = nullptr;  // 58 <= N <= 64: per-CTA operator of sri_integrate_wrench_local (L2-resident)
     size_t wrench_scratch_cap = 0;
     int wrench_gen_occ = 0;
@@ -916,6 +920,7 @@ int sri_destroy(sri_handle h) {
     if (h->d_ccw) cudaFree(h->d_ccw);
     if (h->d_ptab) cudaFree(h->d_ptab);
     if (h->d_jac) cudaFree(h->d_jac);
+    if (h->d_dnin) cudaFree(h->d_dnin);
     if (h->d_partial) cudaFree(h->d_partial);
     if (h->d_counter) cudaFree(h->d_counter);
     if (h->newton.graph) cudaGraphExecDestroy(h->newton.graph);
@@ -1455,6 +1460,111 @@ int sri_generalised_forces(sri_handle h, int64_t batch, int ne, const double* La
     return st.finish();
 }
 
+// S = Dn_NN^-1 and S_T = D_TT^-1, row-major [M][M] each (h->d_jac: the scalar kernel of sri_shape_jacobian and the
+// reverse-mode kernels), built on first use
+static int ensure_rowmajor_ops(sri_context* h) {
+    if (h->d_jac) return SRI_OK;
+    const int M = h->M;
+    std::vector<double> t((size_t)2 * M * M);
+    for (int i = 0; i < M; ++i)
+        for (int j = 0; j < M; ++j) {
+            t[(size_t)i * M + j] = h->ops.S[(size_t)j * M + i];
+            t[(size_t)M * M + (size_t)i * M + j] = h->ops.ST[(size_t)j * M + i];
+        }
+    SRI_CUDA(cudaMalloc(&h->d_jac, t.size() * sizeof(double)));
+    SRI_CUDA(cudaMemcpy(h->d_jac, t.data(), t.size() * sizeof(double), cudaMemcpyHostToDevice));
+    return SRI_OK;
+}
+
+// device pointers, handle's device current: N <= 16 two rods per warp (sri_vjp16.cuh), else one rod per CTA
+static int launch_vjp(sri_context* h, const sri::VjpParams& p) {
+    if (h->N <= 16) {
+        constexpr size_t smem = (sri::VjpTables16::total + (size_t)(kFusedThreads / 32) * 2 * sri::VjpScratch16::total) * sizeof(double);
+        if (h->vjp_occ == 0) {
+            if (h->M == 15) SRI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->vjp_occ, sri::vjp16_kernel<15>, kFusedThreads, smem));
+            else SRI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->vjp_occ, sri::vjp16_kernel<0>, kFusedThreads, smem));
+            if (h->vjp_occ < 1) return fail(SRI_ERR_CUDA, "sri_integrate_all_vjp: kernel does not fit on this device");
+        }
+        const long long want = ((p.batch + 1) / 2 + (kFusedThreads / 32) - 1) / (kFusedThreads / 32);
+        const long long cap = (long long)h->sm_count * h->vjp_occ;
+        const int grid = (int)(want < cap ? want : cap);
+        if (h->M == 15) sri::vjp16_kernel<15><<<grid, kFusedThreads, smem, h->stream>>>(p);
+        else sri::vjp16_kernel<0><<<grid, kFusedThreads, smem, h->stream>>>(p);
+    } else {
+        const size_t smem = sri::VjpTiledSmem{h->M}.bytes();
+        SRI_TRY(ensure_dynamic_smem(sri::vjp_tiled_kernel, h->device, smem));
+        if (h->vjp_occ == 0) {
+            SRI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->vjp_occ, sri::vjp_tiled_kernel, sri::kVjpTiledThreads, smem));
+            if (h->vjp_occ < 1) return fail(SRI_ERR_CUDA, "sri_integrate_all_vjp: kernel does not fit on this device");
+        }
+        const long long cap = (long long)h->sm_count * h->vjp_occ;
+        sri::vjp_tiled_kernel<<<(int)(p.batch < cap ? p.batch : cap), sri::kVjpTiledThreads, smem, h->stream>>>(p);
+    }
+    g_launches.fetch_add(1);
+    SRI_CUDA(cudaGetLastError());
+    return SRI_OK;
+}
+
+int sri_integrate_all_vjp(sri_handle h, const sri_rod_batch* rods, const sri_rod_batch_grad* grads) {
+    SRI_ENTER(h);
+    if (!rods || !grads) return fail(SRI_ERR_INVALID_ARGUMENT, "sri_integrate_all_vjp: rods and grads are required");
+    const int64_t B = rods->batch;
+    if (B < 0) return fail(SRI_ERR_INVALID_ARGUMENT, "sri_integrate_all_vjp: negative batch");
+    if (B == 0) return SRI_OK;
+    if (!rods->K) return fail(SRI_ERR_INVALID_ARGUMENT, "sri_integrate_all_vjp: K is required");
+    if (!rods->Q) return fail(SRI_ERR_INVALID_ARGUMENT, "sri_integrate_all_vjp: Q (the forward's output) is required");
+    if (grads->gm && !rods->n) return fail(SRI_ERR_INVALID_ARGUMENT, "sri_integrate_all_vjp: n (the forward's output) is required with gm");
+    const int N = h->N, M = h->M;
+    SRI_TRY(ensure_rowmajor_ops(h));
+    if (!h->d_dnin) {
+        SRI_CUDA(cudaMalloc(&h->d_dnin, sizeof(double) * M));
+        SRI_CUDA(cudaMemcpy(h->d_dnin, h->ops.Dn_IN.data(), sizeof(double) * M, cudaMemcpyHostToDevice));
+    }
+    Staging st(h);
+    sri::VjpParams p{};
+    p.batch = B; p.N = N; p.M = M;
+    p.S_rm = h->d_jac; p.ST_rm = h->d_jac + (size_t)M * M; p.DTI = h->d_dtt + (size_t)M * M; p.DnIN = h->d_dnin;
+    SRI_TRY(st.in(rods->K, (size_t)B * 3 * N, &p.K));
+    SRI_TRY(st.in(rods->q0, (size_t)B * 4, &p.q0));
+    SRI_TRY(st.in(rods->Gamma, (size_t)B * 3 * N, &p.Gamma));
+    SRI_TRY(st.in<double>(rods->Q, (size_t)B * 4 * M, &p.Q));
+    if (grads->gm) SRI_TRY(st.in<double>(rods->n, (size_t)B * 3 * M, &p.n));
+    SRI_TRY(st.in(grads->gQ, (size_t)B * 4 * M, &p.gQ));
+    SRI_TRY(st.in(grads->gr, (size_t)B * 3 * M, &p.gr));
+    SRI_TRY(st.in(grads->gn, (size_t)B * 3 * M, &p.gn));
+    SRI_TRY(st.in(grads->gm, (size_t)B * 3 * M, &p.gm));
+    SRI_TRY(st.out(grads->gK, (size_t)B * 3 * N, &p.gK));
+    SRI_TRY(st.out(grads->gq0, (size_t)B * 4, &p.gq0));
+    SRI_TRY(st.out(grads->gr0, (size_t)B * 3, &p.gr0));
+    SRI_TRY(st.out(grads->gGamma, (size_t)B * 3 * N, &p.gGamma));
+    SRI_TRY(st.out(grads->gfbar, (size_t)B * 3 * N, &p.gfbar));
+    SRI_TRY(st.out(grads->glbar, (size_t)B * 3 * N, &p.glbar));
+    SRI_TRY(st.out(grads->gF_tip, (size_t)B * 3, &p.gF_tip));
+    SRI_TRY(st.out(grads->gM_tip, (size_t)B * 3, &p.gM_tip));
+    SRI_TRY(st.out(rods->info, (size_t)B, &p.info));
+    SRI_TRY(launch_vjp(h, p));
+    SRI_TRY(st.finish());
+    if (rods->info && !is_device_pointer(rods->info)) return singular_status(rods->info, B, "sri_integrate_all_vjp");
+    return SRI_OK;
+}
+
+int sri_strain_from_modes_transpose(sri_handle h, int64_t batch, int ne, const double* gK, double* gqe) {
+    SRI_ENTER(h);
+    if (batch < 0 || ne < 1 || ne > 8 || (batch > 0 && (!gK || !gqe)))
+        return fail(SRI_ERR_INVALID_ARGUMENT, "sri_strain_from_modes_transpose: bad arguments (1 <= ne <= 8)");
+    if (batch == 0) return SRI_OK;
+    Staging st(h);
+    const double* dgK; double* dgqe;
+    SRI_TRY(st.in(gK, (size_t)batch * 3 * h->N, &dgK));
+    SRI_TRY(st.out(gqe, (size_t)batch * 3 * ne, &dgqe));
+    const long long total = (long long)batch * 3;
+    // the projection kernel without quadrature weights: gqe[b][c*ne+k] = sum_i P_k(t_i) gK[b][c][i]
+    project_onto_modes_kernel<<<(unsigned)((total + 127) / 128), 128, 0, h->stream>>>(batch, h->N, ne, 3LL * h->N, 1.0, h->d_ptab, nullptr, dgK, dgqe);
+    g_launches.fetch_add(1);
+    SRI_CUDA(cudaGetLastError());
+    return st.finish();
+}
+
 // device pointers, H on the host, handle's device current
 static int shape_jacobian_dev(sri_context* h, int64_t batch, int ne, const double* H, const double* dQ, const double* dq0,
                               const double* dG, const double* dn, const double* dm, const double* dMt, double* dJ) {
@@ -1485,16 +1595,7 @@ static int shape_jacobian_dev(sri_context* h, int64_t batch, int ne, const doubl
         SRI_CUDA(cudaGetLastError());
         return SRI_OK;
     }
-    if (!h->d_jac) {
-        std::vector<double> t((size_t)2 * M * M);
-        for (int i = 0; i < M; ++i)
-            for (int j = 0; j < M; ++j) {
-                t[(size_t)i * M + j] = h->ops.S[(size_t)j * M + i];
-                t[(size_t)M * M + (size_t)i * M + j] = h->ops.ST[(size_t)j * M + i];
-            }
-        SRI_CUDA(cudaMalloc(&h->d_jac, t.size() * sizeof(double)));
-        SRI_CUDA(cudaMemcpy(h->d_jac, t.data(), t.size() * sizeof(double), cudaMemcpyHostToDevice));
-    }
+    SRI_TRY(ensure_rowmajor_ops(h));
     constexpr int kWarps = 4;
     const size_t smem = ((size_t)2 * M * M + (size_t)9 * N + (size_t)kWarps * JacobianScratch::total(N)) * sizeof(double);
     SRI_TRY(ensure_dynamic_smem(shape_jacobian_kernel, h->device, smem));

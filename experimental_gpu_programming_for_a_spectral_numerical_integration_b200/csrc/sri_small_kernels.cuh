@@ -163,7 +163,7 @@ __global__ void wrench_local_kernel(long long batch, int N, const double* __rest
 
 // out[b][c*ne+k] = scale * sum_i w_i P_k(t_i) f[b*rod_stride + c*N + i]: one thread per (rod, component), cached Legendre
 // table.  rod_stride = 3 N, scale = 1: projection of a nodal field; rod_stride = 6 N, scale = -1: generalised forces of the
-// couple part of a wrench field.
+// couple part of a wrench field.  ccw == NULL: w_i = 1, the transpose of the modal strain adapter.
 __global__ void project_onto_modes_kernel(long long batch, int N, int ne, long long rod_stride, double scale,
                                           const double* __restrict__ ptab, const double* __restrict__ ccw,
                                           const double* __restrict__ f, double* __restrict__ out) {
@@ -175,7 +175,7 @@ __global__ void project_onto_modes_kernel(long long batch, int N, int ne, long l
     for (int k = 0; k < ne; ++k) acc[k] = 0.0;
     const double* fi = f + b * rod_stride + c * N;
     for (int i = 0; i < N; ++i) {
-        const double wf = ccw[i] * fi[i];
+        const double wf = ccw ? ccw[i] * fi[i] : fi[i];
 #pragma unroll
         for (int k = 0; k < 8; ++k)
             if (k < ne) acc[k] = fma(wf, ptab[k * N + i], acc[k]);

@@ -32,7 +32,7 @@ extern "C" {
 #endif
 
 #define SRI_VERSION_MAJOR 0
-#define SRI_VERSION_MINOR 2
+#define SRI_VERSION_MINOR 3
 
 typedef enum sri_status {
     SRI_OK = 0,
@@ -79,6 +79,10 @@ int sri_get_operator(sri_handle h, int which, double* out);
 
 /* K = Phi<3,ne>(x_i) * qe at every node (main.cpp:69).  qe [batch][3*ne] -> K [batch][3][N]. */
 int sri_strain_from_modes(sri_handle h, int64_t batch, int ne, const double* qe, double* K);
+/* Its transpose (no quadrature weights, unlike sri_project_onto_modes): gqe[b][c*ne+k] = sum_i P_k(2 x_i - 1) gK[b][c][i],
+ * the gradient with respect to qe of a function of K = Phi qe whose K-gradient is gK.  gK [batch][3][N] -> gqe [batch][3*ne],
+ * 1 <= ne <= 8. */
+int sri_strain_from_modes_transpose(sri_handle h, int64_t batch, int ne, const double* gK, double* gqe);
 
 /* Rod length (SURVEY 8 f3).  The reference integrates on X in [0,1] with an implicit length of 1 (ComputeChebyshevPoints<N, 1>,
  * main.cpp:15).  For a rod of length l every ODE is multiplied by l (rod_modeling.pdf eq. 2.17): Q' = l/2 Q (x) (0,K),
@@ -143,6 +147,32 @@ typedef struct sri_rod_batch {
     int* info;           /* [batch] or NULL */
 } sri_rod_batch;
 int sri_integrate_all(sri_handle h, const sri_rod_batch* rods);
+
+/* Reverse mode of sri_integrate_all (vector-Jacobian product of the discrete four-stage map): given cotangents of the
+ * outputs, the gradients of  <gQ,Q> + <gr,r> + <gn,n> + <gm,m>  with respect to the eight inputs, in one launch.
+ * rods: the struct of the forward call.  Its inputs are read as in sri_integrate_all (NULL defaults q0 = identity,
+ * Gamma = e1; r0, fbar, lbar, F_tip, M_tip enter linearly and are not read); rods->Q, the forward's output, is required;
+ * rods->n is required when gm is given; rods->r and rods->m are not read.  rods->info (or NULL) receives the zero /
+ * non-finite pivot step of the transposed stage-1 solve A_NN(K)^T lam = gQ (0 when no K / q0 gradient is wanted).
+ * Cotangents have the shapes of the outputs (NULL = zero); every non-NULL gradient has the shape of its input and is
+ * written, not accumulated (K and fbar/lbar gradients are 0 at the node whose sample the forward does not use).  Host or
+ * device pointers, errors and SRI_ERR_SINGULAR as for sri_integrate_all.  N <= 16: two rods per warp, register-resident
+ * Gauss-Jordan with row pivoting; 17 <= N <= 64: one rod per CTA. */
+typedef struct sri_rod_batch_grad {
+    const double* gQ;  /* [batch][4][M] or NULL */
+    const double* gr;  /* [batch][3][M] or NULL */
+    const double* gn;  /* [batch][3][M] or NULL */
+    const double* gm;  /* [batch][3][M] or NULL */
+    double* gK;        /* [batch][3][N] or NULL */
+    double* gq0;       /* [batch][4]    or NULL */
+    double* gr0;       /* [batch][3]    or NULL */
+    double* gGamma;    /* [batch][3][N] or NULL */
+    double* gfbar;     /* [batch][3][N] or NULL */
+    double* glbar;     /* [batch][3][N] or NULL */
+    double* gF_tip;    /* [batch][3]    or NULL */
+    double* gM_tip;    /* [batch][3]    or NULL */
+} sri_rod_batch_grad;
+int sri_integrate_all_vjp(sri_handle h, const sri_rod_batch* rods, const sri_rod_batch_grad* grads);
 
 /* ---- several devices in one process (SURVEY 8b/8e: one host thread and one stream per GPU, contiguous rod ranges) -------- */
 
