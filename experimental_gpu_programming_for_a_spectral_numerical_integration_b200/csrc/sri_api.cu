@@ -17,6 +17,7 @@
 #include <mutex>
 #include <string>
 #include <thread>
+#include <tuple>
 #include <utility>
 #include <vector>
 
@@ -37,18 +38,6 @@
 #include "sri_wrench_gj_multi.cuh"
 #include "sri_wrench_gj_static.cuh"
 #include "sri_wrench_solve.cuh"
-
-// <row tiles per warp, column tiles, warps> of the N <= 32 instantiation of the multi-warp DMMA kernel
-#ifndef SRI_T32_RT
-#define SRI_T32_RT 4
-#define SRI_T32_W 4
-#endif
-#define SRI_T32 SRI_T32_RT, 4, SRI_T32_W
-#ifndef SRI_T64_RT
-#define SRI_T64_RT 2
-#define SRI_T64_W 16
-#endif
-#define SRI_T64 SRI_T64_RT, 8, SRI_T64_W
 #include "sri_host_math.hpp"
 
 namespace {
@@ -78,8 +67,6 @@ struct sri_context {
     sri_host::OperatorSet ops;
     double* d_ops16 = nullptr;   // OpsLayout16 tables (N <= 16) or OpsLayoutGeneric tables (N > 16)
     int R = 0;                   // generic kernel: row lanes (32 or 64); 0 for the N <= 16 kernel
-    size_t generic_smem = 0;
-    int generic_blocks_per_sm = 0;
     double* d_ops2 = nullptr;    // N > 16: tables of the DMMA kernel (Stx | AS | AT, TiledDmmaCfg)
     double* d_dtt = nullptr;     // D_TT (M x M, column-major), D_TI (M), D_TT^-1 (M x M): operator of the local-frame statics solve and its preconditioner
     double* d_tnodes = nullptr;  // 2 x_i - 1, i = 0..N-1
@@ -89,24 +76,17 @@ struct sri_context {
     double* d_jac = nullptr;     // S = Dn_NN^-1 and S_T = D_TT^-1, row-major [M][M] each (sri_shape_jacobian, sri_integrate_all_vjp), built on first use
     double* d_dnn = nullptr;     // Dn_NN, column-major [M][M] (sri_assemble_A), built on first use
     double* d_dnin = nullptr;    // Dn_IN [M] (sri_integrate_all_vjp), built on first use
-    int vjp_occ = 0;             // resident CTAs per SM of the reverse-mode kernel of this N
     double* d_wrench_scratch = nullptr;  // 58 <= N <= 64: per-CTA operator of sri_integrate_wrench_local (L2-resident)
     size_t wrench_scratch_cap = 0;
-    int wrench_gen_occ = 0;
-    int wrench_gj_occ = 0;
     int wrench_impl = 0;         // SRI_WRENCH_IMPL: 0 = default (register-resident rolled Gauss-Jordan, N <= 33: one row per lane over 1-3 warps, two rows per lane for 12 <= N <= 16), 1 = blocked (N <= 16: shared-memory blocked LU with DMMA), 2 = generic (N > 16: CTA-wide LU), 3 = multi (one row per lane also for 12 <= N <= 16), 4 = warp (two rows per lane for every N <= 16)
-    int jac_occ[9] = {};         // resident CTAs per SM of shape_jacobian_dmma_kernel<ne>
     int jac_impl = 0;            // 0: DMMA kernel for N <= 16 (default), 1: SRI_JACOBIAN_IMPL=scalar everywhere (A/B measurements)
     const int* skip = nullptr;   // Newton loop with the device-side convergence flag: kernels launched while this is set take
                                  // it as their "already converged, do nothing" flag (NULL everywhere else)
     void* nccl_comm = nullptr;   // ncclComm_t attached by sri_nccl_init
     int nccl_nranks = 1, nccl_rank = 0;
     double* d_gather = nullptr;  // [2 * nccl_nranks] all-gathered norms
-    int fused_blocks_per_sm = 0;
-    int stage_blocks_per_sm = 0;
-    int dmma_blocks_per_sm = 0;
     double dmma_growth = sri::kDmmaGrowthDefault;
-    bool use_dmma = false;
+    bool use_dmma = false;       // DMMA elimination first, row-pivoting kernel for the rods it hands back (SRI_FUSED16_IMPL)
     struct NewtonWorkspace {  // buffers of sri_newton_static_shape, kept for the next call of the same shape
         int64_t B = -1; int ne = 0; bool has_K0 = false, analytic = false;
         double* block = nullptr;
@@ -125,10 +105,6 @@ struct sri_context {
     double* d_partial = nullptr;  // block partials of galerkin_residual_kernel's norms, and its ticket counter
     size_t partial_cap = 0;
     unsigned* d_counter = nullptr;
-    size_t tma_smem[3] = {0, 0, 0};  // shared-memory size the cached occupancy of each TMA stage kernel was computed for
-    int tma_occ[3] = {0, 0, 0};
-    size_t gtma_smem[3] = {0, 0, 0};  // the same for the 17 <= N <= 64 TMA stage kernels
-    int gtma_occ[3] = {0, 0, 0};
     cudaEvent_t pipe_event = nullptr;  // orders the host-buffer pipeline after the work already queued on `stream`
     // tracing: every API call is an NVTX range; with sri_set_timing a CUDA-event pair brackets its work on `stream`
     bool timing = false;
@@ -136,7 +112,7 @@ struct sri_context {
     cudaEvent_t t0 = nullptr, t1 = nullptr;
     const char* timed_call = nullptr;
     int stage_impl = 0;          // N <= 16 separate-stage entry points: 0 = measured best per stage (position, couple: TMA-staged;
-                                 // stress: direct loads), 1 = SRI_STAGE_IMPL=tma everywhere, 2 = SRI_STAGE_IMPL=ldg everywhere       // N <= 16: DMMA elimination first, row-pivoting scalar kernel for the rods it hands back
+                                 // stress: direct loads), 1 = SRI_STAGE_IMPL=tma everywhere, 2 = SRI_STAGE_IMPL=ldg everywhere
     // rods handed back by the DMMA kernel: [0] = count, entries from [4]; one list per pipeline slot + the handle stream
     int* d_list[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};   // hand-back lists: pipeline slots 0-2, handle stream 3, local-frame statics 4
     size_t list_cap[5] = {0, 0, 0, 0, 0};
@@ -237,6 +213,41 @@ int ensure_dynamic_smem(Kernel kernel, int device, size_t bytes) {
     return SRI_OK;
 }
 
+// Resident CTAs per SM of `kernel` at this block size and dynamic shared memory (0: it does not fit), with the kernel's
+// shared-memory limit raised first.  Like that limit, the answer belongs to (kernel, device), so it is cached process-wide.
+template <typename Kernel>
+int resident_ctas(const sri_context* h, Kernel kernel, int threads, size_t smem, int* occ) {
+    SRI_TRY(ensure_dynamic_smem(kernel, h->device, smem));
+    static std::mutex mu;
+    static std::map<std::tuple<const void*, int, int, size_t>, int> cache;
+    std::lock_guard<std::mutex> lock(mu);
+    const auto key = std::make_tuple(reinterpret_cast<const void*>(kernel), h->device, threads, smem);
+    auto it = cache.find(key);
+    if (it == cache.end()) {
+        int n = 0;
+        SRI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, kernel, threads, smem));
+        it = cache.emplace(key, n).first;
+    }
+    *occ = it->second;
+    return SRI_OK;
+}
+
+// Every kernel launch that sri_kernel_launch_count counts goes through here.
+template <typename... Params, typename... Args>
+int launch(void (*kernel)(Params...), dim3 grid, int threads, size_t smem, cudaStream_t stream, Args&&... args) {
+    kernel<<<grid, threads, smem, stream>>>(std::forward<Args>(args)...);
+    g_launches.fetch_add(1);
+    SRI_CUDA(cudaGetLastError());
+    return SRI_OK;
+}
+
+// the diagonal stiffness H_diag (3 doubles) from a host or device pointer
+int read_H(const double* H_diag, double* H) {
+    if (is_device_pointer(H_diag)) SRI_CUDA(cudaMemcpy(H, H_diag, 3 * sizeof(double), cudaMemcpyDeviceToHost));
+    else std::memcpy(H, H_diag, 3 * sizeof(double));
+    return SRI_OK;
+}
+
 // Makes the handle's device current for the duration of one API call and restores the caller's device afterwards.
 class DeviceGuard {
 public:
@@ -299,52 +310,7 @@ namespace {
 
 // ---- launch helpers --------------------------------------------------------------------------------------------
 
-constexpr int kFusedThreads = SRI_THREADS;
-constexpr size_t kFusedSmem = (sri::OpsLayout16::total + (kFusedThreads / 32) * sri::kWarpScratch16) * sizeof(double);
-
-int list_reserve(sri_context* h, int slot, long long batch);
-
-template <bool SOLVE>
-int launch_generic(sri_context* h, const sri::FusedParams& p_in, cudaStream_t stream, int list_slot = 3) {
-    sri::FusedParams p = p_in;
-    if (SOLVE && h->use_dmma) {
-        // first pass: static-order elimination on the FP64 tensor cores, one rod per CTA
-        if (p.batch > 0x7fffffffLL) return fail(SRI_ERR_INVALID_ARGUMENT, "batch too large for one call (2^31 rods)");
-        SRI_TRY(list_reserve(h, list_slot, p.batch));
-        {
-            const double g2 = h->dmma_growth * h->dmma_growth;
-            const double lg = (g2 > 0.0) ? std::log2(g2) * 1048576.0 : -2.0e9;
-            p.growth_log = (int)std::lround(std::max(-2.0e9, std::min(2.0e9, lg)));
-        }
-        p.ops2 = h->d_ops2;
-        p.rod_count = h->d_list[list_slot];
-        p.rod_list = h->d_list[list_slot] + 4;
-        SRI_CUDA(cudaMemsetAsync(p.rod_count, 0, sizeof(int), stream));
-        if (list_slot == 3) h->last_handback_slot = 3;
-        const long long dcap = (long long)h->sm_count * h->dmma_blocks_per_sm;
-        const int dgrid = (int)(p.batch < dcap ? p.batch : dcap);
-        if (h->R == 32) {
-            using Cfg = sri::TiledDmmaCfg<SRI_T32>;
-            sri::tiled_dmma_kernel<SRI_T32><<<dgrid, Cfg::threads, Cfg::smem_bytes, stream>>>(p);
-        } else {
-            using Cfg = sri::TiledDmmaCfg<SRI_T64>;
-            sri::tiled_dmma_kernel<SRI_T64><<<dgrid, Cfg::threads, Cfg::smem_bytes, stream>>>(p);
-        }
-        g_launches.fetch_add(1);
-        SRI_CUDA(cudaGetLastError());
-        // second pass (row pivoting) over the rods handed back; CTAs without work exit at once
-    }
-    const long long cap = (long long)h->sm_count * h->generic_blocks_per_sm;
-    const long long groups = (h->R == 32) ? (p.batch + 1) / 2 : p.batch;  // rods per CTA iteration: 2 (N <= 32) or 1
-    const int grid = (int)(groups < cap ? groups : cap);
-    if (h->R == 32)
-        sri::tiled_kernel<16, 4, SOLVE><<<grid, 128, h->generic_smem, stream>>>(p);
-    else
-        sri::tiled_kernel<32, 8, SOLVE><<<grid, 256, h->generic_smem, stream>>>(p);
-    g_launches.fetch_add(1);
-    SRI_CUDA(cudaGetLastError());
-    return SRI_OK;
-}
+constexpr size_t kFusedSmem = (sri::OpsLayout16::total + (sri::kFusedThreads / 32) * sri::kWarpScratch16) * sizeof(double);
 
 int list_reserve(sri_context* h, int slot, long long batch) {
     size_t need = (size_t)batch + 4;
@@ -360,54 +326,66 @@ int list_reserve(sri_context* h, int slot, long long batch) {
     return SRI_OK;
 }
 
+// Points p.rod_count / p.rod_list at the emptied hand-back list `slot` (pipeline slots 0-2, handle stream 3, local-frame
+// statics 4) for a first pass over `batch` rods; sri_get_handback_count reports the last list used on the handle's stream.
+template <typename Params>
+int handback_list(sri_context* h, int slot, long long batch, cudaStream_t stream, Params& p) {
+    if (batch > 0x7fffffffLL) return fail(SRI_ERR_INVALID_ARGUMENT, "batch too large for one call (2^31 rods)");
+    SRI_TRY(list_reserve(h, slot, batch));
+    p.rod_count = h->d_list[slot];
+    p.rod_list = h->d_list[slot] + 4;
+    SRI_CUDA(cudaMemsetAsync(p.rod_count, 0, sizeof(int), stream));
+    if (slot >= 3) h->last_handback_slot = slot;
+    return SRI_OK;
+}
+
+// The fused four-stage integration runs in two passes: static-order elimination on the FP64 tensor cores, then the
+// row-pivoting kernel over the rods that the first pass hands back (over every rod with SRI_FUSED16_IMPL=scalar).
+// Kernel, block size, dynamic shared memory and rods per CTA of each pass for this handle's N:
+struct FusedPass {
+    void (*kernel)(sri::FusedParams);
+    int threads;
+    size_t smem;
+    int rods_per_cta;
+};
+FusedPass fused_first_pass(const sri_context* h) {
+    using C32 = sri::TiledDmmaCfg<4, 4, 4>;   // <row tiles per warp, column tiles, warps> for N <= 32
+    using C64 = sri::TiledDmmaCfg<2, 8, 16>;  // and for N <= 64
+    if (h->R == 0)  // one rod per warp
+        return {h->M == 15 ? sri::fused16_dmma_kernel<15> : sri::fused16_dmma_kernel<0>, sri::kDmmaThreads, sri::kDmmaSmem, sri::kDmmaThreads / 32};
+    if (h->R == 32) return {sri::tiled_dmma_kernel<4, 4, 4>, C32::threads, C32::smem_bytes, 1};
+    return {sri::tiled_dmma_kernel<2, 8, 16>, C64::threads, C64::smem_bytes, 1};
+}
+FusedPass fused_second_pass(const sri_context* h) {
+    if (h->R == 0)  // two rods per warp
+        return {h->M == 15 ? sri::fused16_kernel<15> : sri::fused16_kernel<0>, sri::kFusedThreads, kFusedSmem, 2 * (sri::kFusedThreads / 32)};
+    if (h->R == 32) return {sri::tiled_kernel<16, 4>, 128, sri::TiledSmem<16, 4>::total() * sizeof(double), 2};
+    return {sri::tiled_kernel<32, 8>, 256, sri::TiledSmem<32, 8>::total() * sizeof(double), 1};
+}
+
 // list_slot: which hand-back list to use (pipeline slot, or 3 for the handle stream)
-template <bool SOLVE>
-int launch_fused16(sri_context* h, const sri::FusedParams& p_in, cudaStream_t stream = nullptr, bool use_handle_stream = true,
-                   int list_slot = 3) {
+int launch_fused(sri_context* h, const sri::FusedParams& p_in, cudaStream_t stream = nullptr, bool use_handle_stream = true,
+                 int list_slot = 3) {
     if (p_in.batch <= 0) return SRI_OK;
     sri::FusedParams p = p_in;
     if (use_handle_stream) { stream = h->stream; p.skip = h->skip; }
-    if (h->R != 0) return launch_generic<SOLVE>(h, p, stream, list_slot);
-    const long long pairs = (p.batch + 1) / 2;
-    const long long want = (pairs + (kFusedThreads / 32) - 1) / (kFusedThreads / 32);
-    const int per_sm = SOLVE ? h->fused_blocks_per_sm : h->stage_blocks_per_sm;
-    const long long cap = (long long)h->sm_count * per_sm;
-    const int grid = (int)(want < cap ? want : cap);
-    if constexpr (!SOLVE) {
-        return fail(SRI_ERR_INVALID_ARGUMENT, "internal: the N <= 16 stage entry points use the DMMA stage kernels");
-    } else {
-        if (h->use_dmma) {
-            if (p.batch > 0x7fffffffLL) return fail(SRI_ERR_INVALID_ARGUMENT, "batch too large for one call (2^31 rods)");
-            SRI_TRY(list_reserve(h, list_slot, p.batch));
-            {
-                const double g2 = h->dmma_growth * h->dmma_growth;
-                const double lg = (g2 > 0.0) ? std::log2(g2) * 1048576.0 : -2.0e9;
-                p.growth_log = (int)std::lround(std::max(-2.0e9, std::min(2.0e9, lg)));
-            }
-            p.rod_count = h->d_list[list_slot];
-            p.rod_list = h->d_list[list_slot] + 4;
-            SRI_CUDA(cudaMemsetAsync(p.rod_count, 0, sizeof(int), stream));
-            if (list_slot == 3) h->last_handback_slot = 3;
-            constexpr int wpc = sri::kDmmaThreads / 32;
-            const long long dwant = (p.batch + wpc - 1) / wpc;
-            const long long dcap = (long long)h->sm_count * h->dmma_blocks_per_sm;
-            const int dgrid = (int)(dwant < dcap ? dwant : dcap);
-            if (h->M == 15)
-                sri::fused16_dmma_kernel<15><<<dgrid, sri::kDmmaThreads, sri::kDmmaSmem, stream>>>(p);
-            else
-                sri::fused16_dmma_kernel<0><<<dgrid, sri::kDmmaThreads, sri::kDmmaSmem, stream>>>(p);
-            g_launches.fetch_add(1);
-            SRI_CUDA(cudaGetLastError());
-            // second pass (row pivoting) over the rods handed back; CTAs without work exit at once
-        }
-        if (h->M == 15)
-            sri::fused16_kernel<15, true><<<grid, kFusedThreads, kFusedSmem, stream>>>(p);
-        else
-            sri::fused16_kernel<0, true><<<grid, kFusedThreads, kFusedSmem, stream>>>(p);
+    // grid: one CTA per rods_per_cta rods, at most as many as are resident at once
+    auto run = [&](const FusedPass& k) -> int {
+        int occ = 0;
+        SRI_TRY(resident_ctas(h, k.kernel, k.threads, k.smem, &occ));
+        const long long want = (p.batch + k.rods_per_cta - 1) / k.rods_per_cta;
+        return launch(k.kernel, (int)std::min(want, (long long)h->sm_count * occ), k.threads, k.smem, stream, p);
+    };
+    if (h->use_dmma) {
+        SRI_TRY(handback_list(h, list_slot, p.batch, stream, p));
+        const double g2 = h->dmma_growth * h->dmma_growth;
+        const double lg = (g2 > 0.0) ? std::log2(g2) * 1048576.0 : -2.0e9;
+        p.growth_log = (int)std::lround(std::max(-2.0e9, std::min(2.0e9, lg)));
+        p.ops2 = h->d_ops2;
+        SRI_TRY(run(fused_first_pass(h)));
+        // second pass (row pivoting) over the rods handed back; CTAs without work exit at once
     }
-    g_launches.fetch_add(1);
-    SRI_CUDA(cudaGetLastError());
-    return SRI_OK;
+    return run(fused_second_pass(h));
 }
 
 // ---- host-buffer pipeline --------------------------------------------------------------------------------------
@@ -503,7 +481,7 @@ int integrate_all_host_pipeline_body(sri_context* h, const sri_rod_batch* r) {
         p.F_tip = static_cast<const double*>(din[6]); p.M_tip = static_cast<const double*>(din[7]);
         p.Q = static_cast<double*>(dout[0]); p.r = static_cast<double*>(dout[1]); p.n = static_cast<double*>(dout[2]);
         p.m = static_cast<double*>(dout[3]); p.info = static_cast<int*>(dout[4]);
-        SRI_TRY(launch_fused16<true>(h, p, st, false, slot));
+        SRI_TRY(launch_fused(h, p, st, false, slot));
         for (int a = 0; a < 5; ++a) {
             if (!outs[a].dst) continue;
             SRI_CUDA(cudaMemcpyAsync(static_cast<char*>(outs[a].dst) + (size_t)first * outs[a].per_rod, dout[a],
@@ -519,12 +497,7 @@ int launch_stage_dmma(sri_context* h, const sri::FusedParams& p) {
     if (p.batch <= 0) return SRI_OK;
     const long long tiles = (p.batch + 7) / 8;
     const long long want = (tiles + 3) / 4;
-    const long long cap = (long long)h->sm_count * 8;
-    const int grid = (int)(want < cap ? want : cap);
-    sri::stage_dmma_kernel<STAGE><<<grid, 128, 0, h->stream>>>(p);
-    g_launches.fetch_add(1);
-    SRI_CUDA(cudaGetLastError());
-    return SRI_OK;
+    return launch(sri::stage_dmma_kernel<STAGE>, (int)std::min(want, (long long)h->sm_count * 8), 128, 0, h->stream, p);
 }
 
 // the rods [done, batch) of a separate-stage call
@@ -584,18 +557,12 @@ int launch_stage(sri_context* h, const sri::FusedParams& p_in) {
     L.out = 2 * off;
     L.warp_bytes = 2 * off + 8 * 3 * M * 8;
     const size_t smem = (size_t)sri::kStageTmaWarps * L.warp_bytes;
-    SRI_TRY(ensure_dynamic_smem(sri::stage_tma_kernel<STAGE>, h->device, smem));
-    if (h->tma_smem[STAGE] != smem) {  // the layout depends on which optional inputs are present
-        SRI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->tma_occ[STAGE], sri::stage_tma_kernel<STAGE>, 32 * sri::kStageTmaWarps, smem));
-        h->tma_smem[STAGE] = smem;
-    }
-    const int occ = h->tma_occ[STAGE];
+    constexpr int threads = 32 * sri::kStageTmaWarps;
+    int occ = 0;
+    SRI_TRY(resident_ctas(h, sri::stage_tma_kernel<STAGE>, threads, smem, &occ));
     if (occ < 1) return launch_stage_dmma<STAGE>(h, p);
     const long long want = (tiles + sri::kStageTmaWarps - 1) / sri::kStageTmaWarps;
-    const long long cap = (long long)h->sm_count * occ;
-    sri::stage_tma_kernel<STAGE><<<(int)(want < cap ? want : cap), 32 * sri::kStageTmaWarps, smem, h->stream>>>(p, L, tiles);
-    g_launches.fetch_add(1);
-    SRI_CUDA(cudaGetLastError());
+    SRI_TRY(launch(sri::stage_tma_kernel<STAGE>, (int)std::min(want, (long long)h->sm_count * occ), threads, smem, h->stream, p, L, tiles));
     if (tiles * 8 < p.batch) return launch_stage_dmma<STAGE>(h, stage_tail(p, tiles * 8));
     return SRI_OK;
 }
@@ -608,20 +575,11 @@ int launch_stage_generic_direct(sri_context* h, const sri::FusedParams& p) {
     const long long tiles = (p.batch + 7) / 8;
     const long long want = (tiles + 3) / 4;
     const size_t smem = (size_t)h->R * h->R * sizeof(double);
+    auto* kernel = h->R == 32 ? sri::stage_generic_kernel<STAGE, 32> : sri::stage_generic_kernel<STAGE, 64>;
     int occ = 0;
-    if (h->R == 32) {
-        SRI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, sri::stage_generic_kernel<STAGE, 32>, 128, smem));
-    } else {
-        SRI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, sri::stage_generic_kernel<STAGE, 64>, 128, smem));
-    }
+    SRI_TRY(resident_ctas(h, kernel, 128, smem, &occ));
     if (occ < 1) return fail(SRI_ERR_CUDA, "stage kernel does not fit on this device");
-    const long long cap = (long long)h->sm_count * occ;
-    const int grid = (int)(want < cap ? want : cap);
-    if (h->R == 32) sri::stage_generic_kernel<STAGE, 32><<<grid, 128, smem, h->stream>>>(p);
-    else sri::stage_generic_kernel<STAGE, 64><<<grid, 128, smem, h->stream>>>(p);
-    g_launches.fetch_add(1);
-    SRI_CUDA(cudaGetLastError());
-    return SRI_OK;
+    return launch(kernel, (int)std::min(want, (long long)h->sm_count * occ), 128, smem, h->stream, p);
 }
 
 template <int STAGE>
@@ -653,27 +611,35 @@ int launch_stage_generic(sri_context* h, const sri::FusedParams& p_in) {
     if (off == 0) return launch_stage_generic_direct<STAGE>(h, p);  // nothing to stage (force stage without inputs)
     const size_t smem = (size_t)h->R * h->R * sizeof(double) + (size_t)4 * off;
     if (smem > 220 * 1024) return launch_stage_generic_direct<STAGE>(h, p);
-    if (h->R == 32) SRI_TRY(ensure_dynamic_smem(sri::stage_generic_tma_kernel<STAGE, 32>, h->device, smem));
-    else SRI_TRY(ensure_dynamic_smem(sri::stage_generic_tma_kernel<STAGE, 64>, h->device, smem));
-    if (h->gtma_smem[STAGE] != smem) {
-        if (h->R == 32) {
-            SRI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->gtma_occ[STAGE], sri::stage_generic_tma_kernel<STAGE, 32>, 128, smem));
-        } else {
-            SRI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->gtma_occ[STAGE], sri::stage_generic_tma_kernel<STAGE, 64>, 128, smem));
-        }
-        h->gtma_smem[STAGE] = smem;
-    }
-    const int occ = h->gtma_occ[STAGE];
+    auto* kernel = h->R == 32 ? sri::stage_generic_tma_kernel<STAGE, 32> : sri::stage_generic_tma_kernel<STAGE, 64>;
+    int occ = 0;
+    SRI_TRY(resident_ctas(h, kernel, 128, smem, &occ));
     if (occ < 1) return launch_stage_generic_direct<STAGE>(h, p);
     const long long want = (tiles + 3) / 4;
-    const long long cap = (long long)h->sm_count * occ;
-    const int grid = (int)(want < cap ? want : cap);
-    if (h->R == 32) sri::stage_generic_tma_kernel<STAGE, 32><<<grid, 128, smem, h->stream>>>(p, L, tiles);
-    else sri::stage_generic_tma_kernel<STAGE, 64><<<grid, 128, smem, h->stream>>>(p, L, tiles);
-    g_launches.fetch_add(1);
-    SRI_CUDA(cudaGetLastError());
+    SRI_TRY(launch(kernel, (int)std::min(want, (long long)h->sm_count * occ), 128, smem, h->stream, p, L, tiles));
     if (tiles * 8 < p.batch) return launch_stage_generic_direct<STAGE>(h, stage_tail(p, tiles * 8));
     return SRI_OK;
+}
+
+// Tables of the DMMA kernels for row capacity R (16, 32 or 64; zero-filled by the caller): Stx [R][R] row-major =
+// -1/2 S with g in the last column, and the stage operators S and -S_T as A fragments [R/8][R/4][32] with the boundary
+// terms g and g_T as the last k index.
+void dmma_tables(const sri_host::OperatorSet& ops, int M, int R, double* Stx, double* AS, double* AT) {
+    const int KT = R / 4;
+    for (int i = 0; i < M; ++i) {
+        for (int j = 0; j < M; ++j) Stx[(size_t)i * R + j] = -0.5 * ops.S[j * M + i];
+        Stx[(size_t)i * R + R - 1] = ops.g[i];
+    }
+    for (int mt = 0; mt < R / 8; ++mt)
+        for (int kt = 0; kt < KT; ++kt)
+            for (int lane = 0; lane < 32; ++lane) {
+                const int i = 8 * mt + lane / 4, j = 4 * kt + lane % 4;
+                double s = 0.0, t = 0.0;
+                if (i < M && j < M) { s = ops.S[j * M + i]; t = -ops.ST[j * M + i]; }
+                if (i < M && j == R - 1) { s = ops.g[i]; t = ops.gT[i]; }
+                AS[(mt * KT + kt) * 32 + lane] = s;
+                AT[(mt * KT + kt) * 32 + lane] = t;
+            }
 }
 
 }  // namespace
@@ -761,21 +727,7 @@ int sri_create(int N, int device, sri_handle* out) {
             t[L::DnIN + i] = h->ops.Dn_IN[i];
         }
         t.resize(sri::DmmaTables::total, 0.0);
-        for (int i = 0; i < M; ++i) {
-            for (int j = 0; j < M; ++j) t[sri::DmmaTables::Stx + i * 16 + j] = -0.5 * h->ops.S[j * M + i];
-            t[sri::DmmaTables::Stx + i * 16 + 15] = h->ops.g[i];
-        }
-        // stage operators in DMMA A-fragment order, boundary term as k index 15
-        for (int mt = 0; mt < 2; ++mt)
-            for (int kt = 0; kt < 4; ++kt)
-                for (int lane = 0; lane < 32; ++lane) {
-                    const int i = 8 * mt + lane / 4, j = 4 * kt + lane % 4;
-                    double s = 0.0, tt = 0.0;
-                    if (i < M && j < M) { s = h->ops.S[j * M + i]; tt = -h->ops.ST[j * M + i]; }
-                    if (i < M && j == 15) { s = h->ops.g[i]; tt = h->ops.gT[i]; }
-                    t[sri::DmmaTables::AS + (mt * 4 + kt) * 32 + lane] = s;
-                    t[sri::DmmaTables::AT + (mt * 4 + kt) * 32 + lane] = tt;
-                }
+        dmma_tables(h->ops, M, 16, t.data() + sri::DmmaTables::Stx, t.data() + sri::DmmaTables::AS, t.data() + sri::DmmaTables::AT);
         SRI_CUDA(cudaMalloc(&h->d_ops16, sizeof(double) * sri::DmmaTables::total));
         SRI_CUDA(cudaMemcpy(h->d_ops16, t.data(), sizeof(double) * sri::DmmaTables::total, cudaMemcpyHostToDevice));
     } else {
@@ -794,48 +746,16 @@ int sri_create(int N, int device, sri_handle* out) {
         }
         SRI_CUDA(cudaMalloc(&h->d_ops16, sizeof(double) * L.total()));
         SRI_CUDA(cudaMemcpy(h->d_ops16, t.data(), sizeof(double) * L.total(), cudaMemcpyHostToDevice));
-        {
-            // tables of the DMMA kernel: Stx [QR][NC] | AS | AT (A fragments of the stage operators, last k index =
-            // boundary term), QR = NC = R
-            const int R = h->R, KT = R / 4;
-            std::vector<double> t2((size_t)3 * R * R, 0.0);
-            for (int i = 0; i < M; ++i) {
-                for (int j = 0; j < M; ++j) t2[(size_t)i * R + j] = -0.5 * h->ops.S[j * M + i];
-                t2[(size_t)i * R + R - 1] = h->ops.g[i];
-            }
-            for (int mt = 0; mt < R / 8; ++mt)
-                for (int kt = 0; kt < KT; ++kt)
-                    for (int lane = 0; lane < 32; ++lane) {
-                        const int i = 8 * mt + lane / 4, j = 4 * kt + lane % 4;
-                        double sv = 0.0, tv = 0.0;
-                        if (i < M && j < M) { sv = h->ops.S[j * M + i]; tv = -h->ops.ST[j * M + i]; }
-                        if (i < M && j == R - 1) { sv = h->ops.g[i]; tv = h->ops.gT[i]; }
-                        t2[(size_t)R * R + (size_t)(mt * KT + kt) * 32 + lane] = sv;
-                        t2[(size_t)2 * R * R + (size_t)(mt * KT + kt) * 32 + lane] = tv;
-                    }
-            SRI_CUDA(cudaMalloc(&h->d_ops2, sizeof(double) * t2.size()));
-            SRI_CUDA(cudaMemcpy(h->d_ops2, t2.data(), sizeof(double) * t2.size(), cudaMemcpyHostToDevice));
-            if (R == 32) {
-                using Cfg = sri::TiledDmmaCfg<SRI_T32>;
-                SRI_TRY(ensure_dynamic_smem(sri::tiled_dmma_kernel<SRI_T32>, h->device, Cfg::smem_bytes));
-                SRI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->dmma_blocks_per_sm, sri::tiled_dmma_kernel<SRI_T32>, Cfg::threads, Cfg::smem_bytes));
-            } else {
-                using Cfg = sri::TiledDmmaCfg<SRI_T64>;
-                SRI_TRY(ensure_dynamic_smem(sri::tiled_dmma_kernel<SRI_T64>, h->device, Cfg::smem_bytes));
-                SRI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->dmma_blocks_per_sm, sri::tiled_dmma_kernel<SRI_T64>, Cfg::threads, Cfg::smem_bytes));
-            }
-            if (h->dmma_blocks_per_sm < 1) { return fail(SRI_ERR_CUDA, "sri_create: DMMA kernel does not fit on this device"); }
-        }
-        if (h->R == 32) {
-            h->generic_smem = sri::TiledSmem<16, 4>::total() * sizeof(double);
-            SRI_TRY(ensure_dynamic_smem(sri::tiled_kernel<16, 4, true>, h->device, h->generic_smem));
-            SRI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->generic_blocks_per_sm, sri::tiled_kernel<16, 4, true>, 128, h->generic_smem));
-        } else {
-            h->generic_smem = sri::TiledSmem<32, 8>::total() * sizeof(double);
-            SRI_TRY(ensure_dynamic_smem(sri::tiled_kernel<32, 8, true>, h->device, h->generic_smem));
-            SRI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->generic_blocks_per_sm, sri::tiled_kernel<32, 8, true>, 256, h->generic_smem));
-        }
-        if (h->generic_blocks_per_sm < 1) { return fail(SRI_ERR_CUDA, "sri_create: generic kernel does not fit on this device"); }
+        const int R = h->R;
+        std::vector<double> t2((size_t)3 * R * R, 0.0);  // tables of the DMMA kernel
+        dmma_tables(h->ops, M, R, t2.data(), t2.data() + (size_t)R * R, t2.data() + (size_t)2 * R * R);
+        SRI_CUDA(cudaMalloc(&h->d_ops2, sizeof(double) * t2.size()));
+        SRI_CUDA(cudaMemcpy(h->d_ops2, t2.data(), sizeof(double) * t2.size(), cudaMemcpyHostToDevice));
+    }
+    for (const FusedPass& k : {fused_first_pass(h), fused_second_pass(h)}) {
+        int occ = 0;
+        SRI_TRY(resident_ctas(h, k.kernel, k.threads, k.smem, &occ));
+        if (occ < 1) return fail(SRI_ERR_CUDA, "sri_create: kernel does not fit on this device");
     }
     {
         std::vector<double> t(N);
@@ -861,23 +781,6 @@ int sri_create(int N, int device, sri_handle* out) {
         sri_host::clenshaw_curtis_weights(N, w.data());
         SRI_CUDA(cudaMalloc(&h->d_ccw, sizeof(double) * N));
         SRI_CUDA(cudaMemcpy(h->d_ccw, w.data(), sizeof(double) * N, cudaMemcpyHostToDevice));
-    }
-    if (N > 16) {
-        h->fused_blocks_per_sm = h->stage_blocks_per_sm = h->generic_blocks_per_sm;
-    } else if (M == 15) {
-        SRI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->fused_blocks_per_sm, sri::fused16_kernel<15, true>, kFusedThreads, kFusedSmem));
-        h->stage_blocks_per_sm = h->fused_blocks_per_sm;
-    } else {
-        SRI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->fused_blocks_per_sm, sri::fused16_kernel<0, true>, kFusedThreads, kFusedSmem));
-        h->stage_blocks_per_sm = h->fused_blocks_per_sm;
-    }
-    if (h->fused_blocks_per_sm < 1 || h->stage_blocks_per_sm < 1) { return fail(SRI_ERR_CUDA, "sri_create: kernel does not fit on this device"); }
-    if (N <= 16) {
-        if (M == 15) SRI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->dmma_blocks_per_sm, sri::fused16_dmma_kernel<15>, sri::kDmmaThreads, sri::kDmmaSmem));
-        else SRI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->dmma_blocks_per_sm, sri::fused16_dmma_kernel<0>, sri::kDmmaThreads, sri::kDmmaSmem));
-        if (h->dmma_blocks_per_sm < 1) { return fail(SRI_ERR_CUDA, "sri_create: DMMA kernel does not fit on this device"); }
-        // Both are sm_100a kernels of this library; SRI_FUSED16_IMPL=scalar selects the row-pivoting scalar kernel for
-        // every rod (A/B measurements), the default is the DMMA elimination with the scalar kernel as its second pass.
     }
     {
         const char* impl = std::getenv("SRI_FUSED16_IMPL");
@@ -1002,18 +905,14 @@ int sri_get_operator(sri_handle h, int which, double* out) {
 
 // device pointers, handle's device current
 static int strain_from_modes_dev(sri_context* h, int64_t batch, int ne, const double* dqe, double* dK) {
-    const long long total = (long long)batch * 3 * h->N;
     if (ne <= 8) {
         const long long rows = (long long)batch * 3;
-        if (h->N <= 16) strain_from_modes_table_kernel<16><<<(unsigned)((rows + 15) / 16), 256, 0, h->stream>>>(rows, h->N, ne, h->d_ptab, dqe, dK, h->skip);
-        else if (h->N <= 32) strain_from_modes_table_kernel<32><<<(unsigned)((rows + 7) / 8), 256, 0, h->stream>>>(rows, h->N, ne, h->d_ptab, dqe, dK, h->skip);
-        else strain_from_modes_table_kernel<64><<<(unsigned)((rows + 3) / 4), 256, 0, h->stream>>>(rows, h->N, ne, h->d_ptab, dqe, dK, h->skip);
-    } else {
-        strain_from_modes_kernel<<<(unsigned)((total + 255) / 256), 256, 0, h->stream>>>(batch, h->N, ne, h->d_tnodes, dqe, dK, h->skip);
+        const int per_cta = h->N <= 16 ? 16 : (h->N <= 32 ? 8 : 4);  // rows per CTA of 256 threads
+        auto* kernel = h->N <= 16 ? strain_from_modes_table_kernel<16> : (h->N <= 32 ? strain_from_modes_table_kernel<32> : strain_from_modes_table_kernel<64>);
+        return launch(kernel, (unsigned)((rows + per_cta - 1) / per_cta), 256, 0, h->stream, rows, h->N, ne, h->d_ptab, dqe, dK, h->skip);
     }
-    g_launches.fetch_add(1);
-    SRI_CUDA(cudaGetLastError());
-    return SRI_OK;
+    const long long total = (long long)batch * 3 * h->N;
+    return launch(strain_from_modes_kernel, (unsigned)((total + 255) / 256), 256, 0, h->stream, batch, h->N, ne, h->d_tnodes, dqe, dK, h->skip);
 }
 
 int sri_strain_from_modes(sri_handle h, int64_t batch, int ne, const double* qe, double* K) {
@@ -1048,10 +947,8 @@ int sri_scale_for_length(sri_handle h, int64_t batch, const double* length, doub
         st.copy_back(arr[i], dev[i], (size_t)batch * per_rod * sizeof(double));
     }
     const long long total = (long long)batch * per_rod;
-    scale_for_length_kernel<<<(unsigned)std::min<long long>((total + 255) / 256, (long long)h->sm_count * 16), 256, 0, h->stream>>>(
-        batch, per_rod, dl, uniform_length, dev[0], dev[1], dev[2], dev[3]);
-    g_launches.fetch_add(1);
-    SRI_CUDA(cudaGetLastError());
+    SRI_TRY(launch(scale_for_length_kernel, (unsigned)std::min<long long>((total + 255) / 256, (long long)h->sm_count * 16), 256, 0,
+                   h->stream, batch, per_rod, dl, uniform_length, dev[0], dev[1], dev[2], dev[3]));
     return st.finish();
 }
 
@@ -1068,10 +965,7 @@ int sri_assemble_A(sri_handle h, int64_t batch, const double* K, double* A_NN) {
     const double* dK; double* dA;
     SRI_TRY(st.in(K, (size_t)batch * 3 * N, &dK));
     SRI_TRY(st.out(A_NN, (size_t)batch * n * n, &dA));
-    const long long cap = (long long)h->sm_count * 8;
-    assemble_A_kernel<<<(unsigned)(batch < cap ? batch : cap), 256, 0, h->stream>>>(batch, N, h->d_dnn, dK, dA);
-    g_launches.fetch_add(1);
-    SRI_CUDA(cudaGetLastError());
+    SRI_TRY(launch(assemble_A_kernel, (unsigned)std::min<long long>(batch, (long long)h->sm_count * 8), 256, 0, h->stream, batch, N, h->d_dnn, dK, dA));
     return st.finish();
 }
 
@@ -1102,7 +996,7 @@ int sri_integrate_all(sri_handle h, const sri_rod_batch* rods) {
     SRI_TRY(st.out(rods->n, (size_t)B * 3 * M, &p.n));
     SRI_TRY(st.out(rods->m, (size_t)B * 3 * M, &p.m));
     SRI_TRY(st.out(rods->info, (size_t)B, &p.info));
-    SRI_TRY(launch_fused16<true>(h, p));
+    SRI_TRY(launch_fused(h, p));
     SRI_TRY(st.finish());
     if (rods->info && !is_device_pointer(rods->info)) return singular_status(rods->info, B, "sri_integrate_all");
     return SRI_OK;
@@ -1149,9 +1043,8 @@ int sri_integrate_stress(sri_handle h, int64_t batch, const double* fbar, const 
         const long long total = (long long)batch * 3 * M, chunks = (total + 255) / 256 * 32;  // 32 lanes per 2 KB tile
         const double* gT = h->d_ops16 + (h->R == 0 ? sri::OpsLayout16::gT : sri::OpsLayoutGeneric{h->R}.gT());
         const bool aligned = (reinterpret_cast<uintptr_t>(p.n) & 15u) == 0;
-        sri::stress_noload_kernel<<<(unsigned)std::min<long long>((chunks + 255) / 256, (long long)h->sm_count * 8), 256, 0, h->stream>>>(total, M, gT, p.F_tip, p.n, aligned ? 1 : 0);
-        g_launches.fetch_add(1);
-        SRI_CUDA(cudaGetLastError());
+        SRI_TRY(launch(sri::stress_noload_kernel, (unsigned)std::min<long long>((chunks + 255) / 256, (long long)h->sm_count * 8), 256, 0,
+                       h->stream, total, M, gT, p.F_tip, p.n, aligned ? 1 : 0));
     } else if (h->R == 0) {
         SRI_TRY(launch_stage<sri::kStageStress>(h, p));
     } else {
@@ -1190,8 +1083,7 @@ int sri_shape_residual(sri_handle h, int64_t batch, const double* K, const doubl
     if (batch == 0) return SRI_OK;
     const int N = h->N, M = h->M;
     double H[3];
-    if (is_device_pointer(H_diag)) SRI_CUDA(cudaMemcpy(H, H_diag, sizeof(H), cudaMemcpyDeviceToHost));
-    else std::memcpy(H, H_diag, sizeof(H));
+    SRI_TRY(read_H(H_diag, H));
     Staging st(h);
     const double *dK, *dK0, *dQ, *dq0, *dm, *dMt; double* drho; double* dred = nullptr;
     SRI_TRY(st.in(K, (size_t)batch * 3 * N, &dK));
@@ -1206,9 +1098,8 @@ int sri_shape_residual(sri_handle h, int64_t batch, const double* K, const doubl
         SRI_CUDA(cudaMemsetAsync(dred, 0, 2 * sizeof(double), h->stream));
     }
     const long long total = (long long)batch * N;
-    shape_residual_kernel<<<(unsigned)((total + 255) / 256), 256, 0, h->stream>>>(batch, N, dK, dK0, H[0], H[1], H[2], dQ, dq0, dm, dMt, drho, dred);
-    g_launches.fetch_add(1);
-    SRI_CUDA(cudaGetLastError());
+    SRI_TRY(launch(shape_residual_kernel, (unsigned)((total + 255) / 256), 256, 0, h->stream, batch, N, dK, dK0, H[0], H[1], H[2], dQ, dq0,
+                   dm, dMt, drho, dred));
     return st.finish();
 }
 
@@ -1228,9 +1119,7 @@ int sri_wrench_local(sri_handle h, int64_t batch, const double* Q, const double*
     SRI_TRY(st.in(M_tip, (size_t)batch * 3, &dMt));
     SRI_TRY(st.out(Lambda, (size_t)batch * 6 * N, &dL));
     const long long total = (long long)batch * N;
-    wrench_local_kernel<<<(unsigned)((total + 255) / 256), 256, 0, h->stream>>>(batch, N, dQ, dq0, dn, dm, dF, dMt, dL);
-    g_launches.fetch_add(1);
-    SRI_CUDA(cudaGetLastError());
+    SRI_TRY(launch(wrench_local_kernel, (unsigned)((total + 255) / 256), 256, 0, h->stream, batch, N, dQ, dq0, dn, dm, dF, dMt, dL));
     return st.finish();
 }
 
@@ -1242,25 +1131,19 @@ int launch_wrench_gjm(sri_context* h, const sri::WrenchParams& p, int64_t batch)
     using C = sri::WrenchGjMultiCfg<NW, WMAX>;
     static_assert(C::NODES <= 33, "node capacity");
     auto* kern = sri::wrench_local_solve_gj_multi_kernel<NW, WMAX, MINB>;
-    SRI_TRY(ensure_dynamic_smem(kern, h->device, C::smem_bytes));
     int occ = 0;
-    SRI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, 32 * NW, C::smem_bytes));
+    SRI_TRY(resident_ctas(h, kern, 32 * NW, C::smem_bytes, &occ));
     if (occ < 1) return fail(SRI_ERR_CUDA, "sri_integrate_wrench_local: kernel does not fit on this device");
-    const long long cap = (long long)h->sm_count * occ;
-    kern<<<(int)(batch < cap ? batch : cap), 32 * NW, C::smem_bytes, h->stream>>>(p);
-    return SRI_OK;
+    return launch(kern, (int)std::min<long long>(batch, (long long)h->sm_count * occ), 32 * NW, C::smem_bytes, h->stream, p);
 }
 template <int NW, int WMAX, int MINB>
 int launch_wrench_gjs(sri_context* h, const sri::WrenchParams& p, int64_t batch) {
     using C = sri::WrenchGjStaticCfg<NW, WMAX>;
     auto* kern = sri::wrench_local_solve_gj_static_kernel<NW, WMAX, MINB>;
-    SRI_TRY(ensure_dynamic_smem(kern, h->device, C::smem_bytes));
     int occ = 0;
-    SRI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, 32 * NW, C::smem_bytes));
+    SRI_TRY(resident_ctas(h, kern, 32 * NW, C::smem_bytes, &occ));
     if (occ < 1) return fail(SRI_ERR_CUDA, "sri_integrate_wrench_local: kernel does not fit on this device");
-    const long long cap = (long long)h->sm_count * occ;
-    kern<<<(int)(batch < cap ? batch : cap), 32 * NW, C::smem_bytes, h->stream>>>(p);
-    return SRI_OK;
+    return launch(kern, (int)std::min<long long>(batch, (long long)h->sm_count * occ), 32 * NW, C::smem_bytes, h->stream, p);
 }
 }  // namespace
 }  // extern "C++"
@@ -1290,22 +1173,15 @@ int sri_integrate_wrench_local(sri_handle h, int64_t batch, const double* K, con
     // back are re-solved with partial pivoting by the second pass
     const bool two_pass = h->wrench_impl == 0 && (N == 17 || (N >= 23 && N <= 33));
     if (two_pass) {
-        if (batch > 0x7fffffffLL) return fail(SRI_ERR_INVALID_ARGUMENT, "batch too large for one call (2^31 rods)");
-        SRI_TRY(list_reserve(h, 4, batch));
+        SRI_TRY(handback_list(h, 4, batch, h->stream, p));
         p.S = h->d_dtt + (size_t)M * M + M;
-        p.rod_count = h->d_list[4];
-        p.rod_list = h->d_list[4] + 4;
         {
             const double g = h->dmma_growth;
             long long bits; std::memcpy(&bits, &g, sizeof bits);
             p.growth_hi = g > 0.0 ? (int)(bits >> 32) : -1;   // (bound 0: every rod goes to the row-pivoting pass)
         }
-        SRI_CUDA(cudaMemsetAsync(p.rod_count, 0, sizeof(int), h->stream));
-        h->last_handback_slot = 4;
         if (N == 17) SRI_TRY((launch_wrench_gjs<2, 48, 6>(h, p, batch)));
         else SRI_TRY((launch_wrench_gjs<3, 96, 1>(h, p, batch)));
-        g_launches.fetch_add(1);
-        SRI_CUDA(cudaGetLastError());
         p.from_list = 1;   // second pass: CTAs without work exit at once
     }
     // row-pivoting kernels: register-resident rolled Gauss-Jordan, one row per lane over 1-3 warps, or (12 <= N <= 16, where it
@@ -1324,9 +1200,8 @@ int sri_integrate_wrench_local(sri_handle h, int64_t batch, const double* K, con
         bool in_smem = (size_t)L.total() * sizeof(double) <= 227 * 1024;
         if (!in_smem) L.in_smem = false;
         const size_t smem = (size_t)L.total() * sizeof(double);
-        SRI_TRY(ensure_dynamic_smem(sri::wrench_local_solve_generic_kernel, h->device, smem));
         int occ = 0;
-        SRI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, sri::wrench_local_solve_generic_kernel, sri::kWrenchGenThreads, smem));
+        SRI_TRY(resident_ctas(h, sri::wrench_local_solve_generic_kernel, sri::kWrenchGenThreads, smem, &occ));
         if (occ < 1) return fail(SRI_ERR_CUDA, "sri_integrate_wrench_local: kernel does not fit on this device");
         const long long capg = (long long)h->sm_count * occ;
         const int grid = (int)(batch < capg ? batch : capg);
@@ -1340,25 +1215,21 @@ int sri_integrate_wrench_local(sri_handle h, int64_t batch, const double* K, con
                 h->wrench_scratch_cap = (size_t)capg * n * ld * sizeof(double);
             }
         }
-        sri::wrench_local_solve_generic_kernel<<<grid, sri::kWrenchGenThreads, smem, h->stream>>>(p, h->d_wrench_scratch, in_smem ? 1 : 0);
+        SRI_TRY(launch(sri::wrench_local_solve_generic_kernel, grid, sri::kWrenchGenThreads, smem, h->stream, p, h->d_wrench_scratch, in_smem ? 1 : 0));
     } else if (h->wrench_impl != 1) {
         // one rod per warp, the whole operator in registers: rolled Gauss-Jordan with implicit partial pivoting
-        SRI_TRY(ensure_dynamic_smem(sri::wrench_local_solve_gj_kernel, h->device, sri::kWrenchGjSmem));
-        if (h->wrench_gj_occ == 0)
-            SRI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->wrench_gj_occ, sri::wrench_local_solve_gj_kernel,
-                                                                   32 * sri::kWrenchGjWarps, sri::kWrenchGjSmem));
-        if (h->wrench_gj_occ < 1) return fail(SRI_ERR_CUDA, "sri_integrate_wrench_local: kernel does not fit on this device");
+        int occ = 0;
+        SRI_TRY(resident_ctas(h, sri::wrench_local_solve_gj_kernel, 32 * sri::kWrenchGjWarps, sri::kWrenchGjSmem, &occ));
+        if (occ < 1) return fail(SRI_ERR_CUDA, "sri_integrate_wrench_local: kernel does not fit on this device");
         const long long want = (batch + sri::kWrenchGjWarps - 1) / sri::kWrenchGjWarps;
-        const long long cap = (long long)h->sm_count * h->wrench_gj_occ;
-        sri::wrench_local_solve_gj_kernel<<<(int)(want < cap ? want : cap), 32 * sri::kWrenchGjWarps, sri::kWrenchGjSmem, h->stream>>>(p);
+        SRI_TRY(launch(sri::wrench_local_solve_gj_kernel, (int)std::min(want, (long long)h->sm_count * occ), 32 * sri::kWrenchGjWarps,
+                       sri::kWrenchGjSmem, h->stream, p));
     } else {
         SRI_TRY(ensure_dynamic_smem(sri::wrench_local_solve_kernel, h->device, sri::kWrenchSmem));
         const long long want = (batch + sri::kWrenchWarps - 1) / sri::kWrenchWarps;
-        const long long cap = (long long)h->sm_count;  // one CTA of 8 warps per SM (24 KB of shared memory per rod)
-        sri::wrench_local_solve_kernel<<<(int)(want < cap ? want : cap), 32 * sri::kWrenchWarps, sri::kWrenchSmem, h->stream>>>(p);
+        // one CTA of 8 warps per SM (24 KB of shared memory per rod)
+        SRI_TRY(launch(sri::wrench_local_solve_kernel, (int)std::min(want, (long long)h->sm_count), 32 * sri::kWrenchWarps, sri::kWrenchSmem, h->stream, p));
     }
-    g_launches.fetch_add(1);
-    SRI_CUDA(cudaGetLastError());
     SRI_TRY(st.finish());
     if (info && !is_device_pointer(info)) return singular_status(info, batch, "sri_integrate_wrench_local");
     return SRI_OK;
@@ -1387,22 +1258,14 @@ static int galerkin_residual_dev(sri_context* h, int64_t batch, int ne, const do
             h->partial_cap = cap;
         }
     }
-#define SRI_GALERKIN(GG, NE_)                                                                                            \
-    galerkin_residual_kernel<GG, NE_><<<(unsigned)blocks, 256, 0, h->stream>>>(batch, N, h->d_ptab, h->d_ccw, dK, dK0, H[0], \
-                                                                                 H[1], H[2], dQ, dq0, dm, dMt, dg,          \
-                                                                                 h->d_partial, h->d_counter, dred, h->skip)
-#define SRI_GALERKIN_NE(GG)                                                                                              \
-    switch (ne) {                                                                                                        \
-        case 1: SRI_GALERKIN(GG, 1); break; case 2: SRI_GALERKIN(GG, 2); break; case 3: SRI_GALERKIN(GG, 3); break;      \
-        case 4: SRI_GALERKIN(GG, 4); break; case 5: SRI_GALERKIN(GG, 5); break; case 6: SRI_GALERKIN(GG, 6); break;      \
-        case 7: SRI_GALERKIN(GG, 7); break; default: SRI_GALERKIN(GG, 8); break;                                        \
-    }
-    if (G == 16) { SRI_GALERKIN_NE(16) } else { SRI_GALERKIN_NE(32) }
-#undef SRI_GALERKIN_NE
+    auto* kernel = G == 16 ? galerkin_residual_kernel<16, 8> : galerkin_residual_kernel<32, 8>;
+    switch (ne) {
+#define SRI_GALERKIN(NE_) case NE_: kernel = G == 16 ? galerkin_residual_kernel<16, NE_> : galerkin_residual_kernel<32, NE_>; break;
+        SRI_GALERKIN(1) SRI_GALERKIN(2) SRI_GALERKIN(3) SRI_GALERKIN(4) SRI_GALERKIN(5) SRI_GALERKIN(6) SRI_GALERKIN(7)
 #undef SRI_GALERKIN
-    g_launches.fetch_add(1);
-    SRI_CUDA(cudaGetLastError());
-    return SRI_OK;
+    }
+    return launch(kernel, (unsigned)blocks, 256, 0, h->stream, batch, N, h->d_ptab, h->d_ccw, dK, dK0, H[0], H[1], H[2], dQ, dq0, dm,
+                  dMt, dg, h->d_partial, h->d_counter, dred, h->skip);
 }
 
 int sri_galerkin_residual(sri_handle h, int64_t batch, int ne, const double* K, const double* K0, const double* H_diag,
@@ -1414,8 +1277,7 @@ int sri_galerkin_residual(sri_handle h, int64_t batch, int ne, const double* K, 
     if (batch == 0) return SRI_OK;
     const int N = h->N, M = h->M;
     double H[3];
-    if (is_device_pointer(H_diag)) SRI_CUDA(cudaMemcpy(H, H_diag, sizeof(H), cudaMemcpyDeviceToHost));
-    else std::memcpy(H, H_diag, sizeof(H));
+    SRI_TRY(read_H(H_diag, H));
     Staging st(h);
     const double *dK, *dK0, *dQ, *dq0, *dm, *dMt; double* dg; double* dred = nullptr;
     SRI_TRY(st.in(K, (size_t)batch * 3 * N, &dK));
@@ -1439,9 +1301,8 @@ int sri_project_onto_modes(sri_handle h, int64_t batch, int ne, const double* f,
     SRI_TRY(st.in(f, (size_t)batch * 3 * h->N, &df));
     SRI_TRY(st.out(out, (size_t)batch * 3 * ne, &dout));
     const long long total = (long long)batch * 3;
-    project_onto_modes_kernel<<<(unsigned)((total + 127) / 128), 128, 0, h->stream>>>(batch, h->N, ne, 3LL * h->N, 1.0, h->d_ptab, h->d_ccw, df, dout);
-    g_launches.fetch_add(1);
-    SRI_CUDA(cudaGetLastError());
+    SRI_TRY(launch(project_onto_modes_kernel, (unsigned)((total + 127) / 128), 128, 0, h->stream, batch, h->N, ne, 3LL * h->N, 1.0,
+                   h->d_ptab, h->d_ccw, df, dout));
     return st.finish();
 }
 
@@ -1454,9 +1315,8 @@ int sri_generalised_forces(sri_handle h, int64_t batch, int ne, const double* La
     SRI_TRY(st.in(Lambda, (size_t)batch * 6 * h->N, &dL));
     SRI_TRY(st.out(Qad, (size_t)batch * 3 * ne, &dout));
     const long long total = (long long)batch * 3;
-    project_onto_modes_kernel<<<(unsigned)((total + 127) / 128), 128, 0, h->stream>>>(batch, h->N, ne, 6LL * h->N, -1.0, h->d_ptab, h->d_ccw, dL, dout);
-    g_launches.fetch_add(1);
-    SRI_CUDA(cudaGetLastError());
+    SRI_TRY(launch(project_onto_modes_kernel, (unsigned)((total + 127) / 128), 128, 0, h->stream, batch, h->N, ne, 6LL * h->N, -1.0,
+                   h->d_ptab, h->d_ccw, dL, dout));
     return st.finish();
 }
 
@@ -1478,31 +1338,17 @@ static int ensure_rowmajor_ops(sri_context* h) {
 
 // device pointers, handle's device current: N <= 16 two rods per warp (sri_vjp16.cuh), else one rod per CTA
 static int launch_vjp(sri_context* h, const sri::VjpParams& p) {
-    if (h->N <= 16) {
-        constexpr size_t smem = (sri::VjpTables16::total + (size_t)(kFusedThreads / 32) * 2 * sri::VjpScratch16::total) * sizeof(double);
-        if (h->vjp_occ == 0) {
-            if (h->M == 15) SRI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->vjp_occ, sri::vjp16_kernel<15>, kFusedThreads, smem));
-            else SRI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->vjp_occ, sri::vjp16_kernel<0>, kFusedThreads, smem));
-            if (h->vjp_occ < 1) return fail(SRI_ERR_CUDA, "sri_integrate_all_vjp: kernel does not fit on this device");
-        }
-        const long long want = ((p.batch + 1) / 2 + (kFusedThreads / 32) - 1) / (kFusedThreads / 32);
-        const long long cap = (long long)h->sm_count * h->vjp_occ;
-        const int grid = (int)(want < cap ? want : cap);
-        if (h->M == 15) sri::vjp16_kernel<15><<<grid, kFusedThreads, smem, h->stream>>>(p);
-        else sri::vjp16_kernel<0><<<grid, kFusedThreads, smem, h->stream>>>(p);
-    } else {
-        const size_t smem = sri::VjpTiledSmem{h->M}.bytes();
-        SRI_TRY(ensure_dynamic_smem(sri::vjp_tiled_kernel, h->device, smem));
-        if (h->vjp_occ == 0) {
-            SRI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->vjp_occ, sri::vjp_tiled_kernel, sri::kVjpTiledThreads, smem));
-            if (h->vjp_occ < 1) return fail(SRI_ERR_CUDA, "sri_integrate_all_vjp: kernel does not fit on this device");
-        }
-        const long long cap = (long long)h->sm_count * h->vjp_occ;
-        sri::vjp_tiled_kernel<<<(int)(p.batch < cap ? p.batch : cap), sri::kVjpTiledThreads, smem, h->stream>>>(p);
-    }
-    g_launches.fetch_add(1);
-    SRI_CUDA(cudaGetLastError());
-    return SRI_OK;
+    const bool small = h->N <= 16;  // two rods per warp, else one rod per CTA
+    auto* kernel = !small ? sri::vjp_tiled_kernel : (h->M == 15 ? sri::vjp16_kernel<15> : sri::vjp16_kernel<0>);
+    const int threads = small ? sri::kFusedThreads : sri::kVjpTiledThreads;
+    const size_t smem = small ? (sri::VjpTables16::total + (size_t)(sri::kFusedThreads / 32) * 2 * sri::VjpScratch16::total) * sizeof(double)
+                              : sri::VjpTiledSmem{h->M}.bytes();
+    const long long rods_per_cta = small ? 2 * (sri::kFusedThreads / 32) : 1;
+    int occ = 0;
+    SRI_TRY(resident_ctas(h, kernel, threads, smem, &occ));
+    if (occ < 1) return fail(SRI_ERR_CUDA, "sri_integrate_all_vjp: kernel does not fit on this device");
+    const long long want = (p.batch + rods_per_cta - 1) / rods_per_cta;
+    return launch(kernel, (int)std::min(want, (long long)h->sm_count * occ), threads, smem, h->stream, p);
 }
 
 int sri_integrate_all_vjp(sri_handle h, const sri_rod_batch* rods, const sri_rod_batch_grad* grads) {
@@ -1559,9 +1405,8 @@ int sri_strain_from_modes_transpose(sri_handle h, int64_t batch, int ne, const d
     SRI_TRY(st.out(gqe, (size_t)batch * 3 * ne, &dgqe));
     const long long total = (long long)batch * 3;
     // the projection kernel without quadrature weights: gqe[b][c*ne+k] = sum_i P_k(t_i) gK[b][c][i]
-    project_onto_modes_kernel<<<(unsigned)((total + 127) / 128), 128, 0, h->stream>>>(batch, h->N, ne, 3LL * h->N, 1.0, h->d_ptab, nullptr, dgK, dgqe);
-    g_launches.fetch_add(1);
-    SRI_CUDA(cudaGetLastError());
+    SRI_TRY(launch(project_onto_modes_kernel, (unsigned)((total + 127) / 128), 128, 0, h->stream, batch, h->N, ne, 3LL * h->N, 1.0,
+                   h->d_ptab, nullptr, dgK, dgqe));
     return st.finish();
 }
 
@@ -1571,40 +1416,28 @@ static int shape_jacobian_dev(sri_context* h, int64_t batch, int ne, const doubl
     const int N = h->N, M = h->M;
     if (N <= 16 && h->jac_impl == 0) {
         // two [16 x 16] x [16 x 9 ne] contractions + the projection on the FP64 tensor cores, one rod per warp
-        int occ = 0;
-        const long long want = (batch + sri::kJacWarps - 1) / sri::kJacWarps;
-#define SRI_JAC(NE_)                                                                                                        \
-    {                                                                                                                       \
-        const size_t smem = (256 + (size_t)sri::kJacWarps * sri::JacDmmaScratch<NE_>::total) * sizeof(double);              \
-        SRI_TRY(ensure_dynamic_smem(sri::shape_jacobian_dmma_kernel<NE_>, h->device, smem));                                \
-        if (h->jac_occ[NE_] == 0)                                                                                            \
-            SRI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->jac_occ[NE_], sri::shape_jacobian_dmma_kernel<NE_>,   \
-                                                                   32 * sri::kJacWarps, smem));                              \
-        occ = h->jac_occ[NE_];                                                                                               \
-        if (occ < 1) return fail(SRI_ERR_CUDA, "sri_shape_jacobian: kernel does not fit on this device");                    \
-        const long long cap = (long long)h->sm_count * occ;                                                                 \
-        sri::shape_jacobian_dmma_kernel<NE_><<<(unsigned)(want < cap ? want : cap), 32 * sri::kJacWarps, smem, h->stream>>>( \
-            batch, N, h->d_ops16, h->d_ptab, h->d_ccw, H[0], H[1], H[2], dQ, dq0, dG, dn, dm, dMt, dJ, h->skip);             \
-    }
+        auto* kernel = sri::shape_jacobian_dmma_kernel<8>;
+        size_t scratch = sri::JacDmmaScratch<8>::total;
         switch (ne) {
-            case 1: SRI_JAC(1) break; case 2: SRI_JAC(2) break; case 3: SRI_JAC(3) break; case 4: SRI_JAC(4) break;
-            case 5: SRI_JAC(5) break; case 6: SRI_JAC(6) break; case 7: SRI_JAC(7) break; default: SRI_JAC(8) break;
-        }
+#define SRI_JAC(NE_) case NE_: kernel = sri::shape_jacobian_dmma_kernel<NE_>; scratch = sri::JacDmmaScratch<NE_>::total; break;
+            SRI_JAC(1) SRI_JAC(2) SRI_JAC(3) SRI_JAC(4) SRI_JAC(5) SRI_JAC(6) SRI_JAC(7)
 #undef SRI_JAC
-        g_launches.fetch_add(1);
-        SRI_CUDA(cudaGetLastError());
-        return SRI_OK;
+        }
+        const size_t smem = (256 + sri::kJacWarps * scratch) * sizeof(double);
+        int occ = 0;
+        SRI_TRY(resident_ctas(h, kernel, 32 * sri::kJacWarps, smem, &occ));
+        if (occ < 1) return fail(SRI_ERR_CUDA, "sri_shape_jacobian: kernel does not fit on this device");
+        const long long want = (batch + sri::kJacWarps - 1) / sri::kJacWarps;
+        return launch(kernel, (unsigned)std::min(want, (long long)h->sm_count * occ), 32 * sri::kJacWarps, smem, h->stream,
+                      batch, N, h->d_ops16, h->d_ptab, h->d_ccw, H[0], H[1], H[2], dQ, dq0, dG, dn, dm, dMt, dJ, h->skip);
     }
     SRI_TRY(ensure_rowmajor_ops(h));
     constexpr int kWarps = 4;
     const size_t smem = ((size_t)2 * M * M + (size_t)9 * N + (size_t)kWarps * JacobianScratch::total(N)) * sizeof(double);
     SRI_TRY(ensure_dynamic_smem(shape_jacobian_kernel, h->device, smem));
-    const long long want = (batch + kWarps - 1) / kWarps, cap = (long long)h->sm_count * 8;
-    shape_jacobian_kernel<<<(unsigned)(want < cap ? want : cap), 32 * kWarps, smem, h->stream>>>(
-        batch, N, ne, h->d_jac, h->d_jac + (size_t)M * M, h->d_ptab, h->d_ccw, H[0], H[1], H[2], dQ, dq0, dG, dn, dm, dMt, dJ, h->skip);
-    g_launches.fetch_add(1);
-    SRI_CUDA(cudaGetLastError());
-    return SRI_OK;
+    const long long want = (batch + kWarps - 1) / kWarps;
+    return launch(shape_jacobian_kernel, (unsigned)std::min(want, (long long)h->sm_count * 8), 32 * kWarps, smem, h->stream,
+                  batch, N, ne, h->d_jac, h->d_jac + (size_t)M * M, h->d_ptab, h->d_ccw, H[0], H[1], H[2], dQ, dq0, dG, dn, dm, dMt, dJ, h->skip);
 }
 
 int sri_shape_jacobian(sri_handle h, int64_t batch, int ne, const double* H_diag, const double* Q, const double* q0,
@@ -1615,8 +1448,7 @@ int sri_shape_jacobian(sri_handle h, int64_t batch, int ne, const double* H_diag
     if (batch == 0) return SRI_OK;
     const int N = h->N, M = h->M, nq = 3 * ne;
     double H[3];
-    if (is_device_pointer(H_diag)) SRI_CUDA(cudaMemcpy(H, H_diag, sizeof(H), cudaMemcpyDeviceToHost));
-    else std::memcpy(H, H_diag, sizeof(H));
+    SRI_TRY(read_H(H_diag, H));
     Staging st(h);
     const double *dQ, *dq0, *dG, *dn, *dm, *dMt; double* dJ;
     SRI_TRY(st.in(Q, (size_t)batch * 4 * M, &dQ));
@@ -1632,21 +1464,13 @@ int sri_shape_jacobian(sri_handle h, int64_t batch, int ne, const double* H_diag
 
 static int solve_small_dev(sri_context* h, int64_t batch, int n, double* A, const double* b, double* x, int* info) {
     if (n == 3 || n == 6 || n == 9) {  // ne <= 3: the whole system lives in the thread's registers
-        const unsigned blocks = (unsigned)((batch + 63) / 64);
-        if (n == 3) solve_small_reg_kernel<3><<<blocks, 64, 0, h->stream>>>(batch, A, b, x, info, h->skip);
-        else if (n == 6) solve_small_reg_kernel<6><<<blocks, 64, 0, h->stream>>>(batch, A, b, x, info, h->skip);
-        else solve_small_reg_kernel<9><<<blocks, 64, 0, h->stream>>>(batch, A, b, x, info, h->skip);
-        g_launches.fetch_add(1);
-        SRI_CUDA(cudaGetLastError());
-        return SRI_OK;
+        auto* kernel = n == 3 ? solve_small_reg_kernel<3> : (n == 6 ? solve_small_reg_kernel<6> : solve_small_reg_kernel<9>);
+        return launch(kernel, (unsigned)((batch + 63) / 64), 64, 0, h->stream, batch, A, b, x, info, h->skip);
     }
     const int T = n <= 13 ? 128 : (n <= 19 ? 64 : 32);
     const size_t smem = (size_t)(n * n + n) * (T + 1) * sizeof(double);
     SRI_TRY(ensure_dynamic_smem(solve_small_kernel, h->device, smem));
-    solve_small_kernel<<<(unsigned)((batch + T - 1) / T), T, smem, h->stream>>>(batch, n, A, b, x, info, h->skip);
-    g_launches.fetch_add(1);
-    SRI_CUDA(cudaGetLastError());
-    return SRI_OK;
+    return launch(solve_small_kernel, (unsigned)((batch + T - 1) / T), T, smem, h->stream, batch, n, A, b, x, info, h->skip);
 }
 
 int sri_solve_small_batched(sri_handle h, int64_t batch, int n, double* A, const double* b, double* x, int* info) {
@@ -1762,10 +1586,7 @@ int sri_nccl_allreduce_norms(sri_handle h, double* norm2_and_max) {
     SRI_ENTER(h);
     if (!norm2_and_max || !is_device_pointer(norm2_and_max)) return fail(SRI_ERR_INVALID_ARGUMENT, "sri_nccl_allreduce_norms: device pointer required");
     SRI_TRY(gather_norms(h, norm2_and_max));
-    fold_norms_kernel<<<1, 32, 0, h->stream>>>(h->d_gather, std::max(1, h->nccl_nranks), norm2_and_max);
-    g_launches.fetch_add(1);
-    SRI_CUDA(cudaGetLastError());
-    return SRI_OK;
+    return launch(fold_norms_kernel, 1, 32, 0, h->stream, h->d_gather, std::max(1, h->nccl_nranks), norm2_and_max);
 }
 
 // Newton iteration of the static shape problem, host loop in this library (no torch, no Python in the loop).  Per
@@ -1793,8 +1614,7 @@ int sri_newton_static_shape(sri_handle h, int64_t batch, int ne, const double* H
     const int N = h->N, M = h->M, n = 3 * ne;
     const int64_t B = batch, W = analytic ? 0 : (int64_t)n * B;
     double H[3];
-    if (is_device_pointer(H_diag)) SRI_CUDA(cudaMemcpy(H, H_diag, sizeof(H), cudaMemcpyDeviceToHost));
-    else std::memcpy(H, H_diag, sizeof(H));
+    SRI_TRY(read_H(H_diag, H));
     auto& ws = h->newton;
     if (ws.B != B || ws.ne != ne || ws.has_K0 != (K0 != nullptr) || ws.analytic != analytic || !ws.block) {
         SRI_CUDA(cudaStreamSynchronize(h->stream));
@@ -1864,7 +1684,7 @@ int sri_newton_static_shape(sri_handle h, int64_t batch, int ne, const double* H
         sri::FusedParams p{};
         p.batch = rods; p.N = N; p.M = M; p.ops = h->d_ops16;
         p.K = K; p.F_tip = F; p.M_tip = Mt; p.Q = Q; p.m = m; p.n = nout;
-        SRI_TRY(launch_fused16<true>(h, p));
+        SRI_TRY(launch_fused(h, p));
         return galerkin_residual_dev(h, rods, ne, K, k0, H, Q, nullptr, m, Mt, g, red);
     };
     // one Newton update + re-evaluation of the base point, all asynchronous on the handle's stream
@@ -1874,16 +1694,12 @@ int sri_newton_static_shape(sri_handle h, int64_t batch, int ne, const double* H
         if (analytic) {
             SRI_TRY(shape_jacobian_dev(h, B, ne, H, ws.Q, nullptr, nullptr, ws.nn, ws.m, ws.Mt, ws.J));
         } else {
-            fd_perturb_kernel<<<(unsigned)((tq + 255) / 256), 256, 0, st>>>(B, n, fd_step, ws.qe, ws.qw, h->skip);
-            g_launches.fetch_add(1);
+            SRI_TRY(launch(fd_perturb_kernel, (unsigned)((tq + 255) / 256), 256, 0, st, B, n, fd_step, ws.qe, ws.qw, h->skip));
             SRI_TRY(evaluate(W, ws.qw, ws.Kw, ws.Qw, ws.mw, ws.Fw, ws.Mtw, ws.K0w, ws.gw, nullptr));
-            fd_jacobian_kernel<<<(unsigned)((tj + 255) / 256), 256, 0, st>>>(B, n, fd_step, ws.gw, ws.g0, ws.J, h->skip);
-            g_launches.fetch_add(1);
+            SRI_TRY(launch(fd_jacobian_kernel, (unsigned)((tj + 255) / 256), 256, 0, st, B, n, fd_step, ws.gw, ws.g0, ws.J, h->skip));
         }
         SRI_TRY(solve_small_dev(h, B, n, ws.J, ws.g0, ws.delta, ws.sinfo));
-        newton_update_kernel<<<(unsigned)((tu + 255) / 256), 256, 0, st>>>(B, n, ws.qe, ws.delta, ws.sinfo, ws.state, h->skip);
-        g_launches.fetch_add(1);
-        SRI_CUDA(cudaGetLastError());
+        SRI_TRY(launch(newton_update_kernel, (unsigned)((tu + 255) / 256), 256, 0, st, B, n, ws.qe, ws.delta, ws.sinfo, ws.state, h->skip));
         return evaluate(B, ws.qe, ws.K, ws.Q, ws.m, ws.F, ws.Mt, ws.K0, ws.g0, ws.red, analytic ? ws.nn : nullptr);
     };
     const double dof = (double)(total_dof > 0 ? total_dof : (int64_t)n * B);
@@ -1891,10 +1707,7 @@ int sri_newton_static_shape(sri_handle h, int64_t batch, int ne, const double* H
     // device-side convergence test number `t` and the asynchronous copy of its outcome to the pinned mirror
     auto test_device = [&]() -> int {
         SRI_TRY(gather_norms(h, ws.red));
-        newton_check_kernel<<<1, 32, 0, st>>>(h->d_gather, nranks, dof, tol, ws.state);
-        g_launches.fetch_add(1);
-        SRI_CUDA(cudaGetLastError());
-        return SRI_OK;
+        return launch(newton_check_kernel, 1, 32, 0, st, h->d_gather, nranks, dof, tol, ws.state);
     };
     auto test_mirror = [&](int t) -> int {
         SRI_CUDA(cudaMemcpyAsync(ws.host_state + (t & 1), ws.state, sizeof(NewtonState), cudaMemcpyDeviceToHost, st));
@@ -2229,10 +2042,8 @@ int sri_generate_rods(sri_handle h, uint64_t seed, int64_t first_rod, int64_t ba
     if (batch == 0) return SRI_OK;
     for (const void* p : {(const void*)K, (const void*)F_tip, (const void*)M_tip, (const void*)fbar})
         if (p && !is_device_pointer(p)) return fail(SRI_ERR_INVALID_ARGUMENT, "sri_generate_rods: device pointers only");
-    generate_rods_kernel<<<(unsigned)((batch + 127) / 128), 128, 0, h->stream>>>(seed, first_rod, batch, h->N, h->d_tnodes, K, F_tip, M_tip, fbar);
-    g_launches.fetch_add(1);
-    SRI_CUDA(cudaGetLastError());
-    return SRI_OK;
+    return launch(generate_rods_kernel, (unsigned)((batch + 127) / 128), 128, 0, h->stream, seed, first_rod, batch, h->N, h->d_tnodes, K,
+                  F_tip, M_tip, fbar);
 }
 
 int sri_get_handback_count(sri_handle h, int64_t* count) {
@@ -2258,9 +2069,7 @@ static int measure_peak(sri_handle h, bool tensor, double* tflops) {
     float best = 1e30f;
     for (int rep = 0; rep < 6; ++rep) {
         SRI_CUDA(cudaEventRecord(e0, h->stream));
-        if (tensor) dmma_peak_kernel<<<blocks, threads, 0, h->stream>>>(d, iters, 0.5);
-        else fp64_peak_kernel<<<blocks, threads, 0, h->stream>>>(d, iters, 0.5);
-        g_launches.fetch_add(1);
+        SRI_TRY(launch(tensor ? dmma_peak_kernel : fp64_peak_kernel, blocks, threads, 0, h->stream, d, iters, 0.5));
         SRI_CUDA(cudaEventRecord(e1, h->stream));
         SRI_CUDA(cudaEventSynchronize(e1));
         float ms = 0;

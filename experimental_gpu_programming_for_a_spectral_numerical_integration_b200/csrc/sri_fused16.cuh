@@ -29,12 +29,8 @@ namespace sri {
 
 constexpr int MP16 = 16;  // padded rows per rod in this kernel
 
-#ifndef SRI_MINBLOCKS
-#define SRI_MINBLOCKS 3
-#endif
-#ifndef SRI_THREADS
-#define SRI_THREADS 128  // threads per CTA of the fused kernel
-#endif
+constexpr int kFusedThreads = 128;  // threads per CTA of the fused kernel
+constexpr int kFusedMinBlocks = 3;
 
 // Packed operator tables (doubles), stride MP16, zero padded.  Built on the host by sri_api.cu.
 struct OpsLayout16 {
@@ -285,10 +281,9 @@ __device__ __forceinline__ void contract16(const double* T, const double* v, int
     o2 = (a[0][2] + a[1][2]) + a[2][2];
 }
 
-// SOLVE = true: all stages starting from the strain samples K.  SOLVE = false: the cached-operator stages only
-// (position / stress / couple), reading Q (and optionally n) produced by an earlier call.
-template <int MS, bool SOLVE>
-__global__ void __launch_bounds__(SRI_THREADS, SOLVE ? SRI_MINBLOCKS : 4) fused16_kernel(const FusedParams p) {
+// All four stages starting from the strain samples K.  MS = M when it is fixed at compile time (15), else 0.
+template <int MS>
+__global__ void __launch_bounds__(kFusedThreads, kFusedMinBlocks) fused16_kernel(const FusedParams p) {
     if (p.skip && *p.skip) return;  // Newton loop: the solve has already converged (device-side flag), nothing to do
     extern __shared__ __align__(16) double smem[];
     double* tab = smem;  // OpsLayout16::total doubles
@@ -300,7 +295,7 @@ __global__ void __launch_bounds__(SRI_THREADS, SOLVE ? SRI_MINBLOCKS : 4) fused1
     double* vec2 = scr + RodScratch::vec2;
     double* misc = scr + RodScratch::misc;
 
-    const bool listed = SOLVE && p.rod_list != nullptr;  // second pass over the rods the DMMA kernel handed back
+    const bool listed = p.rod_list != nullptr;  // second pass over the rods the DMMA kernel handed back
     const long long batch = listed ? (long long)*p.rod_count : p.batch;
     const long long pairs = (batch + 1) >> 1;
     if ((long long)blockIdx.x * (blockDim.x >> 5) >= pairs) return;  // whole CTA idle (the usual case of a second pass)
@@ -318,13 +313,11 @@ __global__ void __launch_bounds__(SRI_THREADS, SOLVE ? SRI_MINBLOCKS : 4) fused1
         double* kb = scr + RodScratch::kbuf + slot * 64;
         const bool ok = idx_ < batch;
         const long long rod_ = (ok && listed) ? (long long)p.rod_list[idx_] : idx_;
-        if (SOLVE) {
-            if (ok && row < N) {
-                const double* s = p.K + rod_ * 3 * N + row;
-                cp_async8(kb + row, s); cp_async8(kb + 16 + row, s + N); cp_async8(kb + 32 + row, s + 2 * N);
-            } else {
-                kb[row] = 0.0; kb[16 + row] = 0.0; kb[32 + row] = 0.0;
-            }
+        if (ok && row < N) {
+            const double* s = p.K + rod_ * 3 * N + row;
+            cp_async8(kb + row, s); cp_async8(kb + 16 + row, s + N); cp_async8(kb + 32 + row, s + 2 * N);
+        } else {
+            kb[row] = 0.0; kb[16 + row] = 0.0; kb[32 + row] = 0.0;
         }
         if (row < 4) {
             if (ok && p.q0) cp_async8(kb + 48 + row, p.q0 + rod_ * 4 + row);
@@ -369,43 +362,33 @@ __global__ void __launch_bounds__(SRI_THREADS, SOLVE ? SRI_MINBLOCKS : 4) fused1
             q0.w = a.x; q0.x = a.y; q0.y = c2.x; q0.z = c2.y;
         }
         quat q; q.w = 1.0; q.x = 0.0; q.y = 0.0; q.z = 0.0;
-        if (SOLVE) {
-            // ---- stage 1: assemble c_ij = delta_ij - 1/2 S_ij (0,K_j) and eliminate ---------------------
-            int sing;
-            {
-                quat c[15], b;
+        // ---- stage 1: assemble c_ij = delta_ij - 1/2 S_ij (0,K_j) and eliminate -------------------------
+        int sing;
+        {
+            quat c[15], b;
 #pragma unroll
-                for (int j = 0; j < 15; ++j) {
-                    const double s = tab[OpsLayout16::St + j * MP16 + row];  // -1/2 S_ij
-                    c[j].w = (j == row) ? 1.0 : 0.0;
-                    c[j].x = s * kb[j]; c[j].y = s * kb[16 + j]; c[j].z = s * kb[32 + j];
-                }
-                {
-                    const double gi = tab[OpsLayout16::g + row];
-                    b.w = gi * q0.w; b.x = gi * q0.x; b.y = gi * q0.y; b.z = gi * q0.z;
-                }
-                int mycol;
-                gauss_jordan16(c, b, M, row, scr + RodScratch::pbuf, mycol, sing);
-                __syncwarp();
-                if (row < M) st_quat(qnode + 4 * mycol, b);
+            for (int j = 0; j < 15; ++j) {
+                const double s = tab[OpsLayout16::St + j * MP16 + row];  // -1/2 S_ij
+                c[j].w = (j == row) ? 1.0 : 0.0;
+                c[j].x = s * kb[j]; c[j].y = s * kb[16 + j]; c[j].z = s * kb[32 + j];
             }
-            if (row == M) st_quat(qnode + 4 * M, q0);
-            if (p.info && live && row == 0) p.info[rod] = sing;
-            cp_async_wait<0>();
+            {
+                const double gi = tab[OpsLayout16::g + row];
+                b.w = gi * q0.w; b.x = gi * q0.x; b.y = gi * q0.y; b.z = gi * q0.z;
+            }
+            int mycol;
+            gauss_jordan16(c, b, M, row, scr + RodScratch::pbuf, mycol, sing);
             __syncwarp();
-            if (row <= M) q = ld_quat(qnode + 4 * row);
-            if (p.Q && live && row < M) {
-                double* d = p.Q + rod * 4 * M + row;
-                d[0] = q.w; d[M] = q.x; d[2 * M] = q.y; d[3 * M] = q.z;
-            }
-        } else {
-            if (row == M) q = q0;
-            if (p.Qin && live && row < M) {
-                const double* s = p.Qin + rod * 4 * M + row;
-                q.w = s[0]; q.x = s[M]; q.y = s[2 * M]; q.z = s[3 * M];
-            }
-            cp_async_wait<0>();
-            __syncwarp();
+            if (row < M) st_quat(qnode + 4 * mycol, b);
+        }
+        if (row == M) st_quat(qnode + 4 * M, q0);
+        if (p.info && live && row == 0) p.info[rod] = sing;
+        cp_async_wait<0>();
+        __syncwarp();
+        if (row <= M) q = ld_quat(qnode + 4 * row);
+        if (p.Q && live && row < M) {
+            double* d = p.Q + rod * 4 * M + row;
+            d[0] = q.w; d[M] = q.x; d[2 * M] = q.y; d[3 * M] = q.z;
         }
 
         if (p.r || p.n || p.m) {
@@ -426,7 +409,7 @@ __global__ void __launch_bounds__(SRI_THREADS, SOLVE ? SRI_MINBLOCKS : 4) fused1
             // ---- stage 3 right-hand side (independent of stage 2; issued before the barrier) -----------
             double F0 = 0.0, F1 = 0.0, F2 = 0.0;
             if ((p.n || p.m) && live && p.F_tip) { F0 = misc[0]; F1 = misc[1]; F2 = misc[2]; }
-            const bool contract3 = (p.n || p.m) && p.fbar && !(!SOLVE && p.nin);
+            const bool contract3 = (p.n || p.m) && p.fbar;
             if (contract3) {
                 const double dti = tab[OpsLayout16::DTI + row];
                 double f0 = 0.0, f1 = 0.0, f2 = 0.0;
@@ -450,10 +433,7 @@ __global__ void __launch_bounds__(SRI_THREADS, SOLVE ? SRI_MINBLOCKS : 4) fused1
             if (p.n || p.m) {
                 // ---- stage 3: n = D_TT^-1 (-fbar - D_TI F_tip^T); lane `row` = reduced index (node row+1)
                 double n0, n1, n2;
-                if (!SOLVE && p.nin) {
-                    n0 = 0.0; n1 = 0.0; n2 = 0.0;
-                    if (live && row < M) { const double* s = p.nin + rod * 3 * M + row; n0 = s[0]; n1 = s[M]; n2 = s[2 * M]; }
-                } else if (contract3) {
+                if (contract3) {
                     contract16<MS>(tab + OpsLayout16::STt, vec2, M, row, n0, n1, n2);
                 } else {
                     const double gi = tab[OpsLayout16::gT + row];

@@ -41,7 +41,7 @@ struct TiledSmem {
     __host__ __device__ static int total() { return ints() + 128; }
 };
 
-template <int LPR, int H, bool SOLVE>
+template <int LPR, int H>
 __global__ void __launch_bounds__(32 * H, (LPR == 16 ? 3 : 1)) tiled_kernel(const FusedParams p) {
     using SM = TiledSmem<LPR, H>;
     constexpr int RPW = SM::RPW, ROWS = SM::ROWS, SC = SM::SC;
@@ -68,7 +68,7 @@ __global__ void __launch_bounds__(32 * H, (LPR == 16 ? 3 : 1)) tiled_kernel(cons
     double* misc_t = smem + SM::misc() + tsub * 16;
 
     // second pass over the rods the DMMA kernel (sri_tiled_dmma.cuh) handed back: rods rod_list[0 .. *rod_count)
-    const bool listed = SOLVE && p.rod_list != nullptr;
+    const bool listed = p.rod_list != nullptr;
     const long long batch = listed ? (long long)*p.rod_count : p.batch;
     const long long groups = (batch + RPW - 1) / RPW;
     if ((long long)blockIdx.x >= groups) return;  // whole CTA idle (the usual case of a second pass)
@@ -79,7 +79,7 @@ __global__ void __launch_bounds__(32 * H, (LPR == 16 ? 3 : 1)) tiled_kernel(cons
         const long long tidx = grp * RPW + tsub;
         const bool tlive = tidx < batch;
         const long long trod = (tlive && listed) ? (long long)p.rod_list[tidx] : tidx;
-        if (SOLVE && tn < 64) {
+        if (tn < 64) {
             double k0 = 0.0, k1 = 0.0, k2 = 0.0;
             if (tlive && tn < N) { const double* s = p.K + trod * 3 * N + tn; k0 = s[0]; k1 = s[N]; k2 = s[2 * N]; }
             Kb_t[tn] = k0; Kb_t[64 + tn] = k1; Kb_t[128 + tn] = k2;
@@ -95,7 +95,7 @@ __global__ void __launch_bounds__(32 * H, (LPR == 16 ? 3 : 1)) tiled_kernel(cons
         quat q0t; q0t.w = misc_t[9]; q0t.x = misc_t[10]; q0t.y = misc_t[11]; q0t.z = misc_t[12];
 
         quat q; q.w = 1.0; q.x = 0.0; q.y = 0.0; q.z = 0.0;
-        if (SOLVE) {
+        {
             // ---- stage 1: assemble this lane's 2 rows x 8 column slots ---------------------------------------
             const double* Kb = smem + SM::Kb() + sub * 192;
             const double* misc = smem + SM::misc() + sub * 16;
@@ -234,12 +234,6 @@ __global__ void __launch_bounds__(32 * H, (LPR == 16 ? 3 : 1)) tiled_kernel(cons
                 double* d = p.Q + trod * 4 * M + tn;
                 d[0] = q.w; d[M] = q.x; d[2 * M] = q.y; d[3 * M] = q.z;
             }
-        } else {
-            if (tn == M) q = q0t;
-            if (p.Qin && tlive && tn < M) {
-                const double* s = p.Qin + trod * 4 * M + tn;
-                q.w = s[0]; q.x = s[M]; q.y = s[2 * M]; q.z = s[3 * M];
-            }
         }
 
         if (p.r || p.n || p.m) {
@@ -251,7 +245,7 @@ __global__ void __launch_bounds__(32 * H, (LPR == 16 ? 3 : 1)) tiled_kernel(cons
                 quat v; v.w = b0; v.x = b1; v.y = b2; v.z = 0.0;
                 st_quat(vec + 4 * tn, v);
             }
-            const bool contract3 = (p.n || p.m) && p.fbar && !(!SOLVE && p.nin);
+            const bool contract3 = (p.n || p.m) && p.fbar;
             const double F0 = misc_t[0], F1 = misc_t[1], F2 = misc_t[2];
             if (contract3 && tn < M) {
                 const double dti = tab[L.DTI() + tn];
@@ -281,9 +275,7 @@ __global__ void __launch_bounds__(32 * H, (LPR == 16 ? 3 : 1)) tiled_kernel(cons
                 // ---- stage 3: thread tn = reduced row (node tn+1) ------------------------------------------------
                 double n0 = 0.0, n1 = 0.0, n2 = 0.0;
                 if (tn < M) {
-                    if (!SOLVE && p.nin) {
-                        if (tlive) { const double* s = p.nin + trod * 3 * M + tn; n0 = s[0]; n1 = s[M]; n2 = s[2 * M]; }
-                    } else if (contract3) {
+                    if (contract3) {
                         double e0 = 0.0, e1 = 0.0, e2 = 0.0;
                         for (int j = 0; j + 1 < M; j += 2) {
                             const double s0 = tab[L.STt() + j * ROWS + tn], s1 = tab[L.STt() + (j + 1) * ROWS + tn];

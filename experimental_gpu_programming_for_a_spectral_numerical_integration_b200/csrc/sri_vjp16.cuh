@@ -16,7 +16,7 @@
 // the nodal quantities, reduced row `row` = node row+1 for the stage 3/4 quantities).
 #pragma once
 #include "sri_device.cuh"
-#include "sri_fused16.cuh"  // MP16, gauss_jordan16, contract16, SRI_THREADS, SRI_MINBLOCKS
+#include "sri_fused16.cuh"  // MP16, gauss_jordan16, contract16, kFusedThreads, kFusedMinBlocks
 
 namespace sri {
 
@@ -114,7 +114,7 @@ __device__ __forceinline__ quat contract16_quat(const double* T, const double* v
 }
 
 template <int MS>
-__global__ void __launch_bounds__(SRI_THREADS, SRI_MINBLOCKS) vjp16_kernel(const VjpParams p) {
+__global__ void __launch_bounds__(kFusedThreads, kFusedMinBlocks) vjp16_kernel(const VjpParams p) {
     extern __shared__ __align__(16) double smem[];
     double* tab = smem;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
