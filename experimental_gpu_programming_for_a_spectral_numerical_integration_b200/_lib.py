@@ -103,6 +103,8 @@ SYMBOLS = {
     "sri_integrate_wrench_local": (c_int, [c_void_p, c_int64] + [c_void_p] * 10),
     "sri_project_onto_modes": (c_int, [c_void_p, c_int64, c_int, c_void_p, c_void_p]),
     "sri_galerkin_residual": (c_int, [c_void_p, c_int64, c_int] + [c_void_p] * 9),
+    "sri_galerkin_residual_vjp": (c_int, [c_void_p, c_int64, c_int] + [c_void_p] * 15),
+    "sri_static_shape_vjp": (c_int, [c_void_p, c_int64, c_int] + [c_void_p] * 6 + [c_int] + [c_void_p] * 7),
     "sri_generalised_forces": (c_int, [c_void_p, c_int64, c_int, c_void_p, c_void_p]),
     "sri_shape_jacobian": (c_int, [c_void_p, c_int64, c_int] + [c_void_p] * 8),
     "sri_solve_small_batched": (c_int, [c_void_p, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),

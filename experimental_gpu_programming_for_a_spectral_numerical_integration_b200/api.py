@@ -387,6 +387,47 @@ class SpectralRodIntegrator:
         )
         return out
 
+    def galerkin_residual_vjp(self, K, H_diag, Q, m, M_tip, gg, K0=None, q0=None,
+                              want=("K", "K0", "H", "Q", "q0", "m", "M_tip"), out=None):
+        """sri_galerkin_residual_vjp: gradients of <gg, g> (g = galerkin_residual, gg [batch][3*ne]) with respect to the inputs
+        named in `want`; "H" is per rod, [batch][3].  Returns a dict of the requested gradients (allocated unless given in the
+        dict `out`)."""
+        self._follow_torch(K)
+        batch, N, M = K.shape[0], self.N, self.M
+        ne = gg.shape[1] // 3
+        H = np.ascontiguousarray(np.asarray(H_diag, dtype=np.float64))
+        shapes = {"K": (batch, 3, N), "K0": (batch, 3, N), "H": (batch, 3), "Q": (batch, 4, M), "q0": (batch, 4),
+                  "m": (batch, 3, M), "M_tip": (batch, 3)}
+        given = out or {}
+        grads = {key: given[key] if given.get(key) is not None else _empty_like_kind(K, shapes[key]) for key in want}
+        g = lambda key: _ptr(grads.get(key), "grad " + key)
+        _lib.check(self._lib.sri_galerkin_residual_vjp(
+            self._h, batch, int(ne), _ptr(K, "K"), _ptr(K0, "K0"), H.ctypes.data, _ptr(Q, "Q"), _ptr(q0, "q0"), _ptr(m, "m"),
+            _ptr(M_tip, "M_tip"), _ptr(gg, "gg"), g("K"), g("K0"), g("H"), g("Q"), g("q0"), g("m"), g("M_tip")),
+            "sri_galerkin_residual_vjp")
+        return grads
+
+    def static_shape_vjp(self, F_tip, M_tip, qe, gqe, H_diag=(1.0, 1.0, 0.77), K0=None, refine_steps: int = 3, info=None,
+                         want=("F_tip", "M_tip", "K0", "H"), out=None):
+        """sri_static_shape_vjp: gradients -(dg/dtheta)^T lam of the equilibrium qe [batch][3*ne] (the caller's converged
+        newton_static_shape solution) for the cotangent gqe, with respect to the parameters named in `want` among F_tip,
+        M_tip, K0, H (per rod, [batch][3]); "lambda" ([batch][3*ne], the adjoint solution) and "resid" ([batch], its relative
+        residual) may be requested too.  info: optional int32 [batch] pivot report.  Returns a dict of the requested arrays
+        (allocated unless given in the dict `out`)."""
+        self._follow_torch(qe)
+        batch, n = qe.shape[0], qe.shape[1]
+        H = np.ascontiguousarray(np.asarray(H_diag, dtype=np.float64))
+        shapes = {"F_tip": (batch, 3), "M_tip": (batch, 3), "K0": (batch, 3, self.N), "H": (batch, 3), "lambda": (batch, n),
+                  "resid": (batch,)}
+        given = out or {}
+        res = {key: given[key] if given.get(key) is not None else _empty_like_kind(qe, shapes[key]) for key in want}
+        g = lambda key: _ptr(res.get(key), key)
+        _lib.check(self._lib.sri_static_shape_vjp(
+            self._h, batch, n // 3, H.ctypes.data, _ptr(F_tip, "F_tip"), _ptr(M_tip, "M_tip"), _ptr(K0, "K0"), _ptr(qe, "qe"),
+            _ptr(gqe, "gqe"), int(refine_steps), g("F_tip"), g("M_tip"), g("K0"), g("H"), g("lambda"), g("resid"),
+            _ptr(info, "info", np.int32)), "sri_static_shape_vjp")
+        return res
+
     def generalised_forces(self, Lambda, ne: int, out=None):
         """Q_ad = -int Phi^T (couple part of the local-frame wrench) dX  (rod_modeling.pdf eqs. 2.16, 2.20)."""
         self._follow_torch(Lambda)

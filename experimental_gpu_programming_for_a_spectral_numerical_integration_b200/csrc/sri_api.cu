@@ -102,6 +102,12 @@ struct sri_context {
         long long graph_kernels = 0;     // kernel nodes per replay (for sri_kernel_launch_count)
         bool graph_off = false;          // SRI_NEWTON_GRAPH=0, or a capture failed on this handle
     } newton;
+    struct AdjointWorkspace {  // buffers of sri_static_shape_vjp, kept for the next call of the same shape
+        int64_t B = -1; int ne = 0;
+        double* block = nullptr;
+        double *K, *Q, *n, *m, *J, *rhs, *delta, *gKd, *gKi, *gQ, *gm, *gMd, *gMi, *gFi, *gHw, *lam;
+        int *sinfo, *vinfo;      // [B] pivot reports of the J_a^T solve and of the transposed stage-1 solve
+    } adjoint;
     double* d_partial = nullptr;  // block partials of galerkin_residual_kernel's norms, and its ticket counter
     size_t partial_cap = 0;
     unsigned* d_counter = nullptr;
@@ -828,6 +834,7 @@ int sri_destroy(sri_handle h) {
     if (h->d_counter) cudaFree(h->d_counter);
     if (h->newton.graph) cudaGraphExecDestroy(h->newton.graph);
     if (h->newton.block) cudaFree(h->newton.block);
+    if (h->adjoint.block) cudaFree(h->adjoint.block);
     for (int sl = 0; sl < 5; ++sl)
         if (h->d_list[sl]) cudaFree(h->d_list[sl]);
     for (int sl = 0; sl < sri_context::kPipeSlots; ++sl) {
@@ -1292,6 +1299,70 @@ int sri_galerkin_residual(sri_handle h, int64_t batch, int ne, const double* K, 
     return st.finish();
 }
 
+extern "C++" {
+namespace {
+// the instantiation <G, ne> (1 <= ne <= 8) of one of the per-rod lane-group kernels, G = 16 for N <= 16, else 32
+template <template <int, int> class Pick>
+auto pick_lanes_ne(int N, int ne) {
+    const bool g16 = N <= 16;
+    switch (ne) {
+#define SRI_PICK(NE_) case NE_: return g16 ? Pick<16, NE_>::get() : Pick<32, NE_>::get();
+        SRI_PICK(1) SRI_PICK(2) SRI_PICK(3) SRI_PICK(4) SRI_PICK(5) SRI_PICK(6) SRI_PICK(7)
+#undef SRI_PICK
+        default: return g16 ? Pick<16, 8>::get() : Pick<32, 8>::get();
+    }
+}
+template <int G, int NE> struct PickResidualVjp { static auto get() { return galerkin_residual_vjp_kernel<G, NE>; } };
+template <int G, int NE> struct PickAdjointRefine { static auto get() { return static_adjoint_refine_kernel<G, NE>; } };
+}  // namespace
+}  // extern "C++"
+
+// persistent grid of the lane-group kernels: 256 threads, at most 4 resident blocks per SM
+static unsigned lane_group_blocks(const sri_context* h, int64_t batch) {
+    const int G = h->N <= 16 ? 16 : 32;
+    const long long chunks = ((long long)batch * G + 255) / 256;
+    return (unsigned)std::min<long long>(chunks, (long long)h->sm_count * 4);
+}
+
+// device pointers, H on the host, handle's device current
+static int galerkin_residual_vjp_dev(sri_context* h, int64_t batch, int ne, const double* dK, const double* dK0, const double* H,
+                                     const double* dQ, const double* dq0, const double* dm, const double* dMt, const double* dgg,
+                                     double* gK, double* gK0, double* gH, double* gQ, double* gq0, double* gm, double* gMt) {
+    return launch(pick_lanes_ne<PickResidualVjp>(h->N, ne), lane_group_blocks(h, batch), 256, 0, h->stream, batch, h->N, h->d_ptab,
+                  h->d_ccw, dK, dK0, H[0], H[1], H[2], dQ, dq0, dm, dMt, dgg, gK, gK0, gH, gQ, gq0, gm, gMt);
+}
+
+int sri_galerkin_residual_vjp(sri_handle h, int64_t batch, int ne, const double* K, const double* K0, const double* H_diag,
+                              const double* Q, const double* q0, const double* m, const double* M_tip, const double* gg,
+                              double* gK, double* gK0, double* gH, double* gQ, double* gq0, double* gm, double* gM_tip) {
+    SRI_ENTER(h);
+    if (batch < 0 || ne < 1 || ne > 8 || !H_diag || (batch > 0 && (!K || !Q || !m || !M_tip || !gg)))
+        return fail(SRI_ERR_INVALID_ARGUMENT, "sri_galerkin_residual_vjp: bad arguments (1 <= ne <= 8)");
+    if (batch == 0) return SRI_OK;
+    const int N = h->N, M = h->M;
+    double H[3];
+    SRI_TRY(read_H(H_diag, H));
+    Staging st(h);
+    const double *dK, *dK0, *dQ, *dq0, *dm, *dMt, *dgg;
+    double *dgK, *dgK0, *dgH, *dgQ, *dgq0, *dgm, *dgMt;
+    SRI_TRY(st.in(K, (size_t)batch * 3 * N, &dK));
+    SRI_TRY(st.in(K0, (size_t)batch * 3 * N, &dK0));
+    SRI_TRY(st.in(Q, (size_t)batch * 4 * M, &dQ));
+    SRI_TRY(st.in(q0, (size_t)batch * 4, &dq0));
+    SRI_TRY(st.in(m, (size_t)batch * 3 * M, &dm));
+    SRI_TRY(st.in(M_tip, (size_t)batch * 3, &dMt));
+    SRI_TRY(st.in(gg, (size_t)batch * 3 * ne, &dgg));
+    SRI_TRY(st.out(gK, (size_t)batch * 3 * N, &dgK));
+    SRI_TRY(st.out(gK0, (size_t)batch * 3 * N, &dgK0));
+    SRI_TRY(st.out(gH, (size_t)batch * 3, &dgH));
+    SRI_TRY(st.out(gQ, (size_t)batch * 4 * M, &dgQ));
+    SRI_TRY(st.out(gq0, (size_t)batch * 4, &dgq0));
+    SRI_TRY(st.out(gm, (size_t)batch * 3 * M, &dgm));
+    SRI_TRY(st.out(gM_tip, (size_t)batch * 3, &dgMt));
+    SRI_TRY(galerkin_residual_vjp_dev(h, batch, ne, dK, dK0, H, dQ, dq0, dm, dMt, dgg, dgK, dgK0, dgH, dgQ, dgq0, dgm, dgMt));
+    return st.finish();
+}
+
 int sri_project_onto_modes(sri_handle h, int64_t batch, int ne, const double* f, double* out) {
     SRI_ENTER(h);
     if (batch < 0 || ne < 1 || ne > 8 || (batch > 0 && (!f || !out))) return fail(SRI_ERR_INVALID_ARGUMENT, "sri_project_onto_modes: bad arguments (1 <= ne <= 8)");
@@ -1336,6 +1407,20 @@ static int ensure_rowmajor_ops(sri_context* h) {
     return SRI_OK;
 }
 
+// VjpParams with the handle's operator tables (built on first use) and the batch shape; every data pointer NULL
+static int vjp_params(sri_context* h, int64_t batch, sri::VjpParams* p) {
+    const int M = h->M;
+    SRI_TRY(ensure_rowmajor_ops(h));
+    if (!h->d_dnin) {
+        SRI_CUDA(cudaMalloc(&h->d_dnin, sizeof(double) * M));
+        SRI_CUDA(cudaMemcpy(h->d_dnin, h->ops.Dn_IN.data(), sizeof(double) * M, cudaMemcpyHostToDevice));
+    }
+    *p = sri::VjpParams{};
+    p->batch = batch; p->N = h->N; p->M = M;
+    p->S_rm = h->d_jac; p->ST_rm = h->d_jac + (size_t)M * M; p->DTI = h->d_dtt + (size_t)M * M; p->DnIN = h->d_dnin;
+    return SRI_OK;
+}
+
 // device pointers, handle's device current: N <= 16 two rods per warp (sri_vjp16.cuh), else one rod per CTA
 static int launch_vjp(sri_context* h, const sri::VjpParams& p) {
     const bool small = h->N <= 16;  // two rods per warp, else one rod per CTA
@@ -1361,15 +1446,9 @@ int sri_integrate_all_vjp(sri_handle h, const sri_rod_batch* rods, const sri_rod
     if (!rods->Q) return fail(SRI_ERR_INVALID_ARGUMENT, "sri_integrate_all_vjp: Q (the forward's output) is required");
     if (grads->gm && !rods->n) return fail(SRI_ERR_INVALID_ARGUMENT, "sri_integrate_all_vjp: n (the forward's output) is required with gm");
     const int N = h->N, M = h->M;
-    SRI_TRY(ensure_rowmajor_ops(h));
-    if (!h->d_dnin) {
-        SRI_CUDA(cudaMalloc(&h->d_dnin, sizeof(double) * M));
-        SRI_CUDA(cudaMemcpy(h->d_dnin, h->ops.Dn_IN.data(), sizeof(double) * M, cudaMemcpyHostToDevice));
-    }
     Staging st(h);
     sri::VjpParams p{};
-    p.batch = B; p.N = N; p.M = M;
-    p.S_rm = h->d_jac; p.ST_rm = h->d_jac + (size_t)M * M; p.DTI = h->d_dtt + (size_t)M * M; p.DnIN = h->d_dnin;
+    SRI_TRY(vjp_params(h, B, &p));
     SRI_TRY(st.in(rods->K, (size_t)B * 3 * N, &p.K));
     SRI_TRY(st.in(rods->q0, (size_t)B * 4, &p.q0));
     SRI_TRY(st.in(rods->Gamma, (size_t)B * 3 * N, &p.Gamma));
@@ -1462,15 +1541,18 @@ int sri_shape_jacobian(sri_handle h, int64_t batch, int ne, const double* H_diag
     return st.finish();
 }
 
-static int solve_small_dev(sri_context* h, int64_t batch, int n, double* A, const double* b, double* x, int* info) {
+// trans: solve A^T x = b instead (A read transposed, not copied)
+static int solve_small_dev(sri_context* h, int64_t batch, int n, double* A, const double* b, double* x, int* info, bool trans = false) {
     if (n == 3 || n == 6 || n == 9) {  // ne <= 3: the whole system lives in the thread's registers
-        auto* kernel = n == 3 ? solve_small_reg_kernel<3> : (n == 6 ? solve_small_reg_kernel<6> : solve_small_reg_kernel<9>);
+        auto* kernel = trans ? (n == 3 ? solve_small_reg_kernel<3, true> : (n == 6 ? solve_small_reg_kernel<6, true> : solve_small_reg_kernel<9, true>))
+                             : (n == 3 ? solve_small_reg_kernel<3, false> : (n == 6 ? solve_small_reg_kernel<6, false> : solve_small_reg_kernel<9, false>));
         return launch(kernel, (unsigned)((batch + 63) / 64), 64, 0, h->stream, batch, A, b, x, info, h->skip);
     }
     const int T = n <= 13 ? 128 : (n <= 19 ? 64 : 32);
     const size_t smem = (size_t)(n * n + n) * (T + 1) * sizeof(double);
-    SRI_TRY(ensure_dynamic_smem(solve_small_kernel, h->device, smem));
-    return launch(solve_small_kernel, (unsigned)((batch + T - 1) / T), T, smem, h->stream, batch, n, A, b, x, info, h->skip);
+    auto* kernel = trans ? solve_small_kernel<true> : solve_small_kernel<false>;
+    SRI_TRY(ensure_dynamic_smem(kernel, h->device, smem));
+    return launch(kernel, (unsigned)((batch + T - 1) / T), T, smem, h->stream, batch, n, A, b, x, info, h->skip);
 }
 
 int sri_solve_small_batched(sri_handle h, int64_t batch, int n, double* A, const double* b, double* x, int* info) {
@@ -1480,6 +1562,112 @@ int sri_solve_small_batched(sri_handle h, int64_t batch, int n, double* A, const
     for (const void* p : {(const void*)A, (const void*)b, (const void*)x, (const void*)info})
         if (p && !is_device_pointer(p)) return fail(SRI_ERR_INVALID_ARGUMENT, "sri_solve_small_batched: device pointers only");
     return solve_small_dev(h, batch, n, A, b, x, info);
+}
+
+// Implicit adjoint of the static shape solve (DESIGN section 5e).  At the caller's qe (one integration and one analytic
+// Jacobian J_a), solve J_d^T lam = gqe by iterative refinement preconditioned with J_a^T:
+//     lam_0 = J_a^-T gqe,   lam_{k+1} = lam_k + J_a^-T (gqe - J_d^T lam_k)   (refine_steps times),
+// where J_d^T lam = Phi^T (gK_dir + gK_int) comes from chain(lam): the residual's VJP (cotangent lam) followed by the
+// integration's VJP of its (gQ, gm).  A final chain(lam) gives the parameter gradients -(dg/dtheta)^T lam and the residual.
+int sri_static_shape_vjp(sri_handle h, int64_t batch, int ne, const double* H_diag, const double* F_tip, const double* M_tip,
+                         const double* K0, const double* qe, const double* gqe, int refine_steps, double* gF_tip,
+                         double* gM_tip, double* gK0, double* gH, double* lambda, double* resid, int* info) {
+    SRI_ENTER(h);
+    if (batch < 0 || ne < 1 || ne > 8 || !H_diag || refine_steps < 0 || refine_steps > 1000 ||
+        (batch > 0 && (!F_tip || !M_tip || !qe || !gqe)))
+        return fail(SRI_ERR_INVALID_ARGUMENT, "sri_static_shape_vjp: bad arguments (1 <= ne <= 8, 0 <= refine_steps <= 1000)");
+    if (batch == 0) return SRI_OK;
+    const int N = h->N, M = h->M, n = 3 * ne;
+    const int64_t B = batch;
+    double H[3];
+    SRI_TRY(read_H(H_diag, H));
+    auto& ws = h->adjoint;
+    if (ws.B != B || ws.ne != ne || !ws.block) {
+        SRI_CUDA(cudaStreamSynchronize(h->stream));
+        if (ws.block) SRI_CUDA(cudaFree(ws.block));
+        ws.block = nullptr; ws.B = -1;
+        auto up = [](size_t v) { return (v + 1) & ~(size_t)1; };  // 16-byte aligned pieces
+        const size_t sz[] = {up((size_t)3 * N * B), up((size_t)4 * M * B), up((size_t)3 * M * B), up((size_t)3 * M * B),
+                             up((size_t)n * n * B), up((size_t)n * B), up((size_t)n * B), up((size_t)3 * N * B), up((size_t)3 * N * B),
+                             up((size_t)4 * M * B), up((size_t)3 * M * B), up((size_t)3 * B), up((size_t)3 * B), up((size_t)3 * B),
+                             up((size_t)3 * B), up((size_t)n * B)};
+        double** fields[] = {&ws.K, &ws.Q, &ws.n, &ws.m, &ws.J, &ws.rhs, &ws.delta, &ws.gKd, &ws.gKi, &ws.gQ, &ws.gm, &ws.gMd,
+                             &ws.gMi, &ws.gFi, &ws.gHw, &ws.lam};
+        static_assert(sizeof(sz) / sizeof(sz[0]) == sizeof(fields) / sizeof(fields[0]), "one size per workspace field");
+        size_t total = 2 * up(((size_t)B + 1) / 2);
+        for (size_t v : sz) total += v;
+        SRI_CUDA(cudaMalloc(&ws.block, total * sizeof(double)));
+        size_t off = 0;
+        for (size_t i = 0; i < sizeof(sz) / sizeof(sz[0]); ++i) { *fields[i] = ws.block + off; off += sz[i]; }
+        ws.sinfo = reinterpret_cast<int*>(ws.block + off);
+        ws.vinfo = ws.sinfo + 2 * up(((size_t)B + 1) / 2);
+        ws.B = B; ws.ne = ne;
+    }
+    Staging st(h);
+    const double *dF, *dMt, *dK0, *dqe, *dgqe;
+    double *dgF, *dgMt, *dgK0, *dgH, *dlam, *dres;
+    int* dinfo;
+    SRI_TRY(st.in(F_tip, (size_t)B * 3, &dF));
+    SRI_TRY(st.in(M_tip, (size_t)B * 3, &dMt));
+    SRI_TRY(st.in(K0, (size_t)B * 3 * N, &dK0));
+    SRI_TRY(st.in(qe, (size_t)B * n, &dqe));
+    SRI_TRY(st.in(gqe, (size_t)B * n, &dgqe));
+    SRI_TRY(st.out(gF_tip, (size_t)B * 3, &dgF));
+    SRI_TRY(st.out(gM_tip, (size_t)B * 3, &dgMt));
+    SRI_TRY(st.out(gK0, (size_t)B * 3 * N, &dgK0));
+    SRI_TRY(st.out(gH, (size_t)B * 3, &dgH));
+    SRI_TRY(st.out(lambda, (size_t)B * n, &dlam));
+    SRI_TRY(st.out(resid, (size_t)B, &dres));
+    SRI_TRY(st.out(info, (size_t)B, &dinfo));
+    double* lam = dlam ? dlam : ws.lam;
+
+    // forward state at qe: K = Phi qe, the four stages (Q, n, m), the analytic Jacobian J_a
+    SRI_TRY(strain_from_modes_dev(h, B, ne, dqe, ws.K));
+    {
+        sri::FusedParams p{};
+        p.batch = B; p.N = N; p.M = M; p.ops = h->d_ops16;
+        p.K = ws.K; p.F_tip = dF; p.M_tip = dMt; p.Q = ws.Q; p.n = ws.n; p.m = ws.m;
+        SRI_TRY(launch_fused(h, p));
+    }
+    SRI_TRY(shape_jacobian_dev(h, B, ne, H, ws.Q, nullptr, nullptr, ws.n, ws.m, dMt, ws.J));
+    SRI_TRY(solve_small_dev(h, B, n, ws.J, dgqe, lam, ws.sinfo, true));
+
+    sri::VjpParams vp{};
+    SRI_TRY(vjp_params(h, B, &vp));
+    vp.K = ws.K; vp.Q = ws.Q; vp.n = ws.n; vp.gQ = ws.gQ; vp.gm = ws.gm; vp.gK = ws.gKi; vp.info = ws.vinfo;
+    auto refine_kernel = pick_lanes_ne<PickAdjointRefine>(N, ne);
+    const unsigned blocks = lane_group_blocks(h, B);
+    const long long tu = (long long)n * B;
+    for (int step = 0; step <= refine_steps; ++step) {
+        const bool last = step == refine_steps;
+        // chain(lam): K0-gradient = H rho_bar = gK_dir, so the last chain writes gK_dir straight into that output
+        double* gKd = last && dgK0 ? dgK0 : ws.gKd;
+        SRI_TRY(galerkin_residual_vjp_dev(h, B, ne, ws.K, dK0, H, ws.Q, nullptr, ws.m, dMt, lam, gKd, nullptr,
+                                          last && dgH ? ws.gHw : nullptr, ws.gQ, nullptr, ws.gm, last && dgMt ? ws.gMd : nullptr));
+        vp.gF_tip = last && dgF ? ws.gFi : nullptr;
+        vp.gM_tip = last && dgMt ? ws.gMi : nullptr;
+        SRI_TRY(launch_vjp(h, vp));
+        AdjointRefineParams rp{};
+        rp.batch = B; rp.N = N; rp.ptab = h->d_ptab; rp.gqe = dgqe; rp.gKd = gKd; rp.gKi = ws.gKi;
+        if (!last) {
+            rp.rhs = ws.rhs;
+        } else {
+            rp.resid = dres;
+            rp.gFi = ws.gFi; rp.gMd = ws.gMd; rp.gMi = ws.gMi; rp.gHw = ws.gHw;
+            rp.gF = dgF; rp.gM = dgMt; rp.gH = dgH;
+            rp.sinfo = ws.sinfo; rp.vinfo = ws.vinfo; rp.info = dinfo;
+        }
+        if (!last || dres || dgF || dgMt || dgH || dinfo) SRI_TRY(launch(refine_kernel, blocks, 256, 0, h->stream, rp));
+        if (!last) {
+            // lam -= J_a^-T (J_d^T lam - gqe), skipped for rods whose J_a^T is singular
+            SRI_TRY(solve_small_dev(h, B, n, ws.J, ws.rhs, ws.delta, ws.sinfo, true));
+            SRI_TRY(launch(newton_update_kernel, (unsigned)((tu + 255) / 256), 256, 0, h->stream, (long long)B, n, lam, ws.delta,
+                           ws.sinfo, (sri::NewtonState*)nullptr, (const int*)nullptr));
+        }
+    }
+    SRI_TRY(st.finish());
+    if (info && !is_device_pointer(info)) return singular_status(info, B, "sri_static_shape_vjp");
+    return SRI_OK;
 }
 
 // ---- NCCL, bound at run time --------------------------------------------------------------------------------------

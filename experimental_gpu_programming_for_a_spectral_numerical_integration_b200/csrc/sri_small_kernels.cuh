@@ -286,6 +286,177 @@ __global__ void __launch_bounds__(256, 4) galerkin_residual_kernel(long long bat
     }
 }
 
+// Reverse mode of galerkin_residual_kernel (sri_galerkin_residual_vjp), same lane layout: with the cotangent gg of g,
+//     rb[c][i] = w_i sum_k P_k(t_i) gg[c*ne+k]                     (the cotangent of rho)
+//     gK = H rb,  gK0 = -H rb,  gH[c] = sum_i rb[c][i] (K - K0)[c][i],  gm_i = -R(q_i) rb_i (node 0: gM_tip),
+//     gq_i = -d/dq (m_i^T R(q) rb_i) at q_i  (nodes 0..M-1: gQ, node N-1: gq0),
+// R the un-normalised rotation of q_rotate.  Every output pointer may be NULL (skipped); all are written, none accumulated.
+// gH is a per-rod shuffle tree over the G lanes in a fixed order: bitwise reproducible.
+template <int G, int NE>
+__global__ void __launch_bounds__(256, 2) galerkin_residual_vjp_kernel(
+        long long batch, int N, const double* __restrict__ ptab, const double* __restrict__ ccw, const double* __restrict__ K,
+        const double* __restrict__ K0, double h0, double h1, double h2, const double* __restrict__ Q,
+        const double* __restrict__ q0, const double* __restrict__ m, const double* __restrict__ M_tip,
+        const double* __restrict__ gg, double* __restrict__ gK, double* __restrict__ gK0, double* __restrict__ gH,
+        double* __restrict__ gQ, double* __restrict__ gq0, double* __restrict__ gm, double* __restrict__ gM_tip) {
+    constexpr int ne = NE;
+    const int M = N - 1;
+    const int sub = threadIdx.x & (G - 1);
+    const double hc[3] = {h0, h1, h2};
+    const long long nblk = (batch * G + blockDim.x - 1) / blockDim.x;
+    for (long long blk = blockIdx.x; blk < nblk; blk += gridDim.x) {
+    const long long b = (blk * blockDim.x + threadIdx.x) / G;
+    double hp[3] = {0.0, 0.0, 0.0};
+    if (b < batch) {
+        double gb[3][NE];
+#pragma unroll
+        for (int c = 0; c < 3; ++c)
+#pragma unroll
+            for (int k = 0; k < NE; ++k) gb[c][k] = gg[b * 3 * ne + c * ne + k];
+        for (int i = sub; i < N; i += G) {
+            const bool inner = i < M;
+            const double* qs = inner ? Q + b * 4 * M + i : (q0 ? q0 + b * 4 : nullptr);
+            const int qst = inner ? M : 1;
+            const double* ms = i == 0 ? M_tip + b * 3 : m + b * 3 * M + (i - 1);
+            const int mst = i == 0 ? 1 : M;
+            const double* kp = K + b * 3 * N + i;
+            sri::quat q; q.w = 1.0; q.x = 0.0; q.y = 0.0; q.z = 0.0;
+            if (qs) { q.w = qs[0]; q.x = qs[qst]; q.y = qs[2 * qst]; q.z = qs[3 * qst]; }
+            const double a0 = ms[0], a1 = ms[mst], a2 = ms[2 * mst];
+            double kd[3] = {kp[0], kp[N], kp[2 * N]};
+            if (K0) { const double* z = K0 + b * 3 * N + i; kd[0] -= z[0]; kd[1] -= z[N]; kd[2] -= z[2 * N]; }
+            const double w = ccw[i];
+            double rb[3] = {0.0, 0.0, 0.0};
+#pragma unroll
+            for (int k = 0; k < NE; ++k) {
+                const double pk = ptab[k * N + i];
+#pragma unroll
+                for (int c = 0; c < 3; ++c) rb[c] = fma(gb[c][k], pk, rb[c]);
+            }
+#pragma unroll
+            for (int c = 0; c < 3; ++c) {
+                rb[c] *= w;
+                hp[c] = fma(rb[c], kd[c], hp[c]);
+                if (gK) gK[b * 3 * N + c * N + i] = hc[c] * rb[c];
+                if (gK0) gK0[b * 3 * N + c * N + i] = -(hc[c] * rb[c]);
+            }
+            if (i == 0 ? gM_tip != nullptr : gm != nullptr) {
+                double r0, r1, r2;
+                sri::q_rotate(q, rb[0], rb[1], rb[2], r0, r1, r2);
+                double* d = i == 0 ? gM_tip + b * 3 : gm + b * 3 * M + (i - 1);
+                d[0] = -r0; d[mst] = -r1; d[2 * mst] = -r2;
+            }
+            double* dq = inner ? (gQ ? gQ + b * 4 * M + i : nullptr) : (gq0 ? gq0 + b * 4 : nullptr);
+            if (dq) {
+                // d/dq a^T R(q) g, R g = g + 2w (v x g) + 2 v x (v x g), v = (x, y, z), a = m_i, g = rb_i
+                const double g0 = rb[0], g1 = rb[1], g2 = rb[2];
+                const double vxg0 = q.y * g2 - q.z * g1, vxg1 = q.z * g0 - q.x * g2, vxg2 = q.x * g1 - q.y * g0;
+                const double gxa0 = g1 * a2 - g2 * a1, gxa1 = g2 * a0 - g0 * a2, gxa2 = g0 * a1 - g1 * a0;
+                const double av = a0 * q.x + a1 * q.y + a2 * q.z, vg = q.x * g0 + q.y * g1 + q.z * g2;
+                const double ag = a0 * g0 + a1 * g1 + a2 * g2;
+                dq[0] = -2.0 * (a0 * vxg0 + a1 * vxg1 + a2 * vxg2);
+                dq[qst] = -(2.0 * q.w * gxa0 + 2.0 * av * g0 + 2.0 * vg * a0 - 4.0 * ag * q.x);
+                dq[2 * qst] = -(2.0 * q.w * gxa1 + 2.0 * av * g1 + 2.0 * vg * a1 - 4.0 * ag * q.y);
+                dq[3 * qst] = -(2.0 * q.w * gxa2 + 2.0 * av * g2 + 2.0 * vg * a2 - 4.0 * ag * q.z);
+            }
+        }
+    }
+    if (gH) {
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+            double v = hp[c];
+#pragma unroll
+            for (int off = G / 2; off >= 1; off >>= 1) v += __shfl_xor_sync(0xffffffffu, v, off);
+            if (b < batch && sub == 0) gH[b * 3 + c] = v;
+        }
+    }
+    }  // chunks of this block
+}
+
+// NaN-propagating max (fmax drops a NaN operand; a non-finite residual must show)
+__device__ __forceinline__ double max_nan(double a, double b) { return (a > b || a != a) ? a : b; }
+
+// One refinement step of the implicit adjoint of the static shape solve (sri_static_shape_vjp).  jd = Phi^T (gKd + gKi) is
+// J_d^T lam, the exact transposed Jacobian of the discrete residual applied to lam (gKd: direct K-gradient of the
+// residual's VJP, gKi: K-gradient of the integration's VJP); rhs = jd - gqe (the negated residual r = gqe - jd, so that
+// the Newton update kernel lam -= J_a^-T rhs applies the step) and resid = max|r| / max|gqe| (max|r| when gqe = 0).  The
+// call after the last chain also writes the parameter gradients F-grad = -gFi, M-grad = -(gMd + gMi), H-grad = -gHw and
+// info = sinfo | vinfo << 8.  G lanes per rod as in galerkin_residual_kernel; NULL outputs are skipped.
+struct AdjointRefineParams {
+    long long batch;
+    int N;
+    const double* ptab;
+    const double* gqe;   // [B][3 ne] cotangent of qe*
+    const double* gKd;   // [B][3][N]
+    const double* gKi;   // [B][3][N]
+    double* rhs;         // [B][3 ne]
+    double* resid;       // [B]
+    const double *gFi, *gMd, *gMi, *gHw;   // [B][3] (final call)
+    double *gF, *gM, *gH;                  // [B][3] (final call)
+    const int *sinfo, *vinfo;              // [B]
+    int* info;                             // [B]
+};
+template <int G, int NE>
+__global__ void __launch_bounds__(256) static_adjoint_refine_kernel(AdjointRefineParams p) {
+    constexpr int ne = NE;
+    const int N = p.N;
+    const int sub = threadIdx.x & (G - 1);
+    const long long nblk = (p.batch * G + blockDim.x - 1) / blockDim.x;
+    for (long long blk = blockIdx.x; blk < nblk; blk += gridDim.x) {
+    const long long b = (blk * blockDim.x + threadIdx.x) / G;
+    double acc[3][NE];
+#pragma unroll
+    for (int c = 0; c < 3; ++c)
+#pragma unroll
+        for (int k = 0; k < NE; ++k) acc[c][k] = 0.0;
+    if (b < p.batch) {
+        for (int i = sub; i < N; i += G) {
+            const double* d = p.gKd + b * 3 * N + i;
+            const double* e = p.gKi + b * 3 * N + i;
+            const double s[3] = {d[0] + e[0], d[N] + e[N], d[2 * N] + e[2 * N]};
+#pragma unroll
+            for (int k = 0; k < NE; ++k) {
+                const double pk = p.ptab[k * N + i];
+#pragma unroll
+                for (int c = 0; c < 3; ++c) acc[c][k] = fma(s[c], pk, acc[c][k]);
+            }
+        }
+    }
+    double rmax = 0.0, gmax = 0.0;
+#pragma unroll
+    for (int c = 0; c < 3; ++c)
+#pragma unroll
+        for (int k = 0; k < NE; ++k) {
+            double v = acc[c][k];
+#pragma unroll
+            for (int off = G / 2; off >= 1; off >>= 1) v += __shfl_xor_sync(0xffffffffu, v, off);
+            const int j = c * ne + k;
+            if (b < p.batch && sub == (j & (G - 1))) {
+                const double gj = p.gqe[b * 3 * ne + j];
+                const double r = gj - v;
+                if (p.rhs) p.rhs[b * 3 * ne + j] = v - gj;
+                rmax = max_nan(rmax, fabs(r));
+                gmax = max_nan(gmax, fabs(gj));
+            }
+        }
+    if (p.resid) {
+#pragma unroll
+        for (int off = G / 2; off >= 1; off >>= 1) {
+            rmax = max_nan(rmax, __shfl_xor_sync(0xffffffffu, rmax, off));
+            gmax = max_nan(gmax, __shfl_xor_sync(0xffffffffu, gmax, off));
+        }
+        if (b < p.batch && sub == 0) p.resid[b] = gmax > 0.0 ? rmax / gmax : rmax;
+    }
+    if (b < p.batch && sub < 3) {
+        const long long o = b * 3 + sub;
+        if (p.gF) p.gF[o] = -p.gFi[o];
+        if (p.gM) p.gM[o] = -(p.gMd[o] + p.gMi[o]);
+        if (p.gH) p.gH[o] = -p.gHw[o];
+        if (p.info && sub == 0) p.info[b] = (p.sinfo ? p.sinfo[b] : 0) | ((p.vinfo ? p.vinfo[b] : 0) << 8);
+    }
+    }  // chunks of this block
+}
+
 // ---- analytic Jacobian of the Galerkin residual (sri_shape_jacobian) ---------------------------------------------------
 // J[b][j'][d] = d g_j' / d qe_d without any linear solve: the variation of the rotation is left-trivialised,
 // dR = [dtheta]x R with dtheta' = R dK, dtheta(base) = 0, so a direction dK = P_k(t) e_c costs two contractions with the
@@ -486,6 +657,9 @@ __global__ void assemble_A_kernel(long long batch, int N, const double* __restri
 
 // One thread per system: Gaussian elimination with partial pivoting.  The block's systems (contiguous in global memory)
 // are staged in shared memory element-major, a[e * (T + 1) + thread]: coalesced copies, conflict-free in both phases.
+// TRANS: solves A^T x = b (element (i, j) of A lands at (j, i) while staged, no copy of A), and a non-finite pivot counts
+// as singular too (the implicit adjoint of the static shape solve reports rods with non-finite loads through it).
+template <bool TRANS>
 __global__ void solve_small_kernel(long long batch, int n, const double* __restrict__ A, const double* __restrict__ b,
                                    double* __restrict__ x, int* __restrict__ info, const int* __restrict__ skip) {
     if (skip && *skip) return;
@@ -497,7 +671,12 @@ __global__ void solve_small_kernel(long long batch, int n, const double* __restr
     double* rhs = ssm + nn * LD + tid;
     {
         const double* src = A + s0 * nn;
-        for (int e = tid; e < count * nn; e += T) { const int sys = e / nn, el = e - sys * nn; ssm[el * LD + sys] = src[e]; }
+        for (int e = tid; e < count * nn; e += T) {
+            const int sys = e / nn;
+            int el = e - sys * nn;
+            if constexpr (TRANS) { const int r = el / n; el = (el - r * n) * n + r; }
+            ssm[el * LD + sys] = src[e];
+        }
         const double* bs = b + s0 * n;
         for (int e = tid; e < count * n; e += T) { const int sys = e / n, el = e - sys * n; ssm[(nn + el) * LD + sys] = bs[e]; }
     }
@@ -508,7 +687,7 @@ __global__ void solve_small_kernel(long long batch, int n, const double* __restr
             int p = k;
             double best = fabs(a[(k * n + k) * LD]);
             for (int i = k + 1; i < n; ++i) { const double v = fabs(a[(i * n + k) * LD]); if (v > best) { best = v; p = i; } }
-            if (best == 0.0) { if (!bad) bad = k + 1; continue; }
+            if (best == 0.0 || (TRANS && !isfinite(best))) { if (!bad) bad = k + 1; continue; }
             if (p != k) {
                 for (int j = k; j < n; ++j) { const double t = a[(k * n + j) * LD]; a[(k * n + j) * LD] = a[(p * n + j) * LD]; a[(p * n + j) * LD] = t; }
                 const double t = rhs[k * LD]; rhs[k * LD] = rhs[p * LD]; rhs[p * LD] = t;
@@ -536,8 +715,8 @@ __global__ void solve_small_kernel(long long batch, int n, const double* __restr
 // The same solve for the small orders of the shape problem (n = 3 ne, ne <= 3) with the whole system in registers: every
 // index is a compile-time constant, the row exchange of the partial pivoting is a chain of predicated swaps, and the
 // thread reads its own contiguous 8 n (n + 1) bytes straight from global memory (a warp's systems are one contiguous
-// region, so every fetched sector is consumed).  Same arithmetic as solve_small_kernel: identical results.
-template <int NN>
+// region, so every fetched sector is consumed).  Same arithmetic as solve_small_kernel: identical results.  TRANS as there.
+template <int NN, bool TRANS>
 __global__ void __launch_bounds__(64) solve_small_reg_kernel(long long batch, const double* __restrict__ A, const double* __restrict__ b,
                                                              double* __restrict__ x, int* __restrict__ info, const int* __restrict__ skip) {
     if (skip && *skip) return;
@@ -549,7 +728,7 @@ __global__ void __launch_bounds__(64) solve_small_reg_kernel(long long batch, co
 #pragma unroll
         for (int i = 0; i < NN; ++i)
 #pragma unroll
-            for (int j = 0; j < NN; ++j) a[i][j] = src[i * NN + j];
+            for (int j = 0; j < NN; ++j) a[i][j] = src[TRANS ? j * NN + i : i * NN + j];
         const double* bs = b + s * NN;
 #pragma unroll
         for (int e = 0; e < NN; ++e) r[e] = bs[e];
@@ -561,7 +740,7 @@ __global__ void __launch_bounds__(64) solve_small_reg_kernel(long long batch, co
         double best = fabs(a[k][k]);
 #pragma unroll
         for (int i = k + 1; i < NN; ++i) { const double v = fabs(a[i][k]); if (v > best) { best = v; p = i; } }
-        const bool ok = best != 0.0;   // a zero column is skipped (multipliers 0), as in solve_small_kernel
+        const bool ok = best != 0.0 && (!TRANS || isfinite(best));   // a zero column is skipped (multipliers 0), as in solve_small_kernel
         if (!ok && !bad) bad = k + 1;
 #pragma unroll
         for (int i = k + 1; i < NN; ++i) {  // row exchange k <-> p by selects: no branch, every index static

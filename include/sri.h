@@ -32,7 +32,7 @@ extern "C" {
 #endif
 
 #define SRI_VERSION_MAJOR 0
-#define SRI_VERSION_MINOR 3
+#define SRI_VERSION_MINOR 4
 
 typedef enum sri_status {
     SRI_OK = 0,
@@ -243,6 +243,18 @@ int sri_galerkin_residual(sri_handle h, int64_t batch, int ne, const double* K, 
                           const double* Q, const double* q0, const double* m, const double* M_tip, double* g,
                           double* norm2_and_max);
 
+/* Reverse mode of sri_galerkin_residual: given the cotangent gg [batch][3*ne] of g, with rb[c][i] = w_i sum_k P_k(2 x_i - 1)
+ * gg[c*ne+k] (the cotangent of rho), the gradients of <gg, g>:
+ *   gK = H rb,  gK0 = -H rb  ([batch][3][N]);  gH[b][c] = sum_i rb[c][i] (K - K0)[c][i]  ([batch][3], per rod: a caller with
+ *   one H for the batch sums over b);  gm[:, i-1] = -R(q_i) rb_i for i = 1..N-1  ([batch][3][M]),  gM_tip = -R(q_0) rb_0;
+ *   gQ[:, i] = -d/dq (m_i^T R(q) rb_i) at q_i for i = 0..M-1  ([batch][4][M]),  gq0 likewise at node N-1  ([batch][4]),
+ * R the un-normalised rotation of the forward.  Inputs as in sri_galerkin_residual (K0, q0 may be NULL); every output may be
+ * NULL (skipped) and is written, not accumulated.  One pass, the lane layout of sri_galerkin_residual; gH is reduced in a fixed
+ * order (bitwise reproducible). */
+int sri_galerkin_residual_vjp(sri_handle h, int64_t batch, int ne, const double* K, const double* K0, const double* H_diag,
+                              const double* Q, const double* q0, const double* m, const double* M_tip, const double* gg,
+                              double* gK, double* gK0, double* gH, double* gQ, double* gq0, double* gm, double* gM_tip);
+
 /* Jacobian of sri_galerkin_residual with respect to the modal strain coordinates, J[b][j][d] = d g_j / d qe_d, without
  * any linear solve: the variation of the rotation is left-trivialised (dR = [dtheta]x R, dtheta' = R dK, dtheta(0) = 0), so
  * every direction is two contractions with the cached integration matrices Dn_NN^-1 and D_TT^-1,
@@ -286,6 +298,24 @@ typedef struct sri_newton_report {
 int sri_newton_static_shape(sri_handle h, int64_t batch, int ne, const double* H_diag, const double* F_tip,
                             const double* M_tip, const double* K0, double* qe, double tol, int max_iter, double fd_step,
                             int64_t total_dof, sri_allreduce_fn reduce, void* reduce_ctx, sri_newton_report* report);
+/* Gradients of the static shape solution (implicit-function theorem): at an equilibrium qe* of sri_newton_static_shape
+ * (g(qe*; F_tip, M_tip, K0, H) = 0, q0 = identity, Gamma = e1, no distributed loads) and a cotangent gqe of qe*, solves
+ * J_d^T lam = gqe per rod, J_d the exact Jacobian of the discrete residual, and returns theta-grad = -(dg/dtheta)^T lam:
+ *   gF_tip, gM_tip [batch][3];  gK0 [batch][3][N];  gH [batch][3] (per rod: a caller with one H sums over the batch).
+ * qe [batch][3*ne] is the caller's converged solution: the call recomputes the four stages and the analytic Jacobian J_a of
+ * sri_shape_jacobian there, but does not check that g(qe) ~ 0; the result is the gradient of the equilibrium only when it is.
+ * J_d is never formed: lam_0 = J_a^-T gqe, then refine_steps steps lam += J_a^-T (gqe - J_d^T lam), each J_d^T lam being one
+ * residual VJP and one sri_integrate_all_vjp.  ||J_a^-1 J_d - I|| (ne = 4, tip loads up to 0.6) is 3e-2 at N = 5, 2e-6 at
+ * N = 9, 6e-14 at N = 16 and grows with the load: refine_steps = 3 reaches round-off for N >= 7, N = 5 needs about 12, 0 is
+ * enough for N >= 16 (DESIGN section 5e).
+ * K0 may be NULL (0); every output may be NULL.  lambda [batch][3*ne]: the adjoint solution; resid [batch]:
+ * max|gqe - J_d^T lam| / max|gqe| at the returned lam.  info [batch]: 0, or (s | v << 8) with s the zero / non-finite pivot
+ * step of the J_a^T solve (1..3*ne) and v that of the transposed stage-1 solve (as in sri_integrate_all_vjp); such a rod's
+ * outputs are not valid.  Host or device pointers, SRI_ERR_SINGULAR with host buffers as in sri_integrate_all_vjp.  The
+ * workspace is kept by the handle for the next call of the same shape. */
+int sri_static_shape_vjp(sri_handle h, int64_t batch, int ne, const double* H_diag, const double* F_tip, const double* M_tip,
+                         const double* K0, const double* qe, const double* gqe, int refine_steps, double* gF_tip,
+                         double* gM_tip, double* gK0, double* gH, double* lambda, double* resid, int* info);
 /* The same solve over all devices of mh from one host process: HOST pointers, rods sharded by index as in
  * sri_integrate_all_sharded, one host thread per device, the norms reduced between the threads (no NCCL, no MPI). */
 int sri_newton_static_shape_sharded(sri_multi_handle mh, int64_t batch, int ne, const double* H_diag, const double* F_tip,
