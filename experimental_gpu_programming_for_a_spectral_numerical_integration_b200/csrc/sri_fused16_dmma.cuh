@@ -1,5 +1,5 @@
 // sri_fused16_dmma.cuh -- fused four-stage kernel for N <= 16 with the quaternion elimination on the FP64 tensor
-// cores (DMMA m8n8k4).  ONE rod per warp.  Lane-exact numpy model of stage 1: tools/dmma_gj_emulator.py.
+// cores (DMMA m8n8k4).  ONE rod per warp.  Lane-exact numpy model of stage 1: tools/dmma_gj_emulator.py (solve_rod_lu).
 //
 // Replaces, per rod, the same reference code as sri_fused16.cuh (updateA main.cpp:55-88, A_NN.inverse()*(b-ivp)
 // main.cpp:113, updatePositionb main.cpp:121-140, Dn_NN_inv*(b_NN-ivp) main.cpp:172) plus rod_modeling.pdf 1.17-1.18.
@@ -8,14 +8,18 @@
 // what bounds it (DESIGN.md 2.1).  The DMMA data path does that broadcast for free.  The M x M quaternion system
 //      sum_j Q_j (x) c_ij = b_i
 // is stored as the REAL 64 x 16 matrix  Cr[4 i + r][j] = component r of c_ij  (column 15 = b_i), i.e. 8 x 2 DMMA
-// accumulator tiles of 8 x 8 = 32 doubles per lane.  With vec(a (x) b) = Rmat(b) vec(a), Gauss-Jordan step k is
+// accumulator tiles of 8 x 8 = 32 doubles per lane.  With vec(a (x) b) = Rmat(b) vec(a), elimination step k is
 //      U'  = Rmat(c_kk^-1) U            U = pivot row as a 4 x 16 matrix (one DMMA per column tile)
-//      Cr -= [Rmat(c_0k); Rmat(c_1k); ...; Rmat(c_kk - 1); ...] U'      (rank-4 update: 8 x 2 DMMAs, k = 4 exactly)
+//      Cr -= [...; Rmat(c_kk - 1); Rmat(c_k+1,k); ...] U'     (rank-4 update of the tile rows below the pivot, k = 4)
 // 4 x 4 real blocks appear only in the A operand (the multipliers); the matrix itself stays in quaternion (4-vector)
 // form, so the DMMAs execute exactly the 16 FMAs per quaternion multiply-add of the scalar kernel.
 // Per step the LSU only moves the pivot row into B-fragment layout (2 SHFL.64 per column tile), one component of the
 // pivot element and its squared norm to every lane (2 SHFL.64) and the pivot column into A-fragment layout (1 SHFL.64
-// per row tile).  Stages 2-4 are [16 x 16] x [16 x 3] DMMA contractions in the same warp (Q never leaves the SM).
+// per live row tile), and stores -U' to shared memory.  The back-substitution then runs with the rows on the n axis:
+//      -Q_i = -U'_i,15 + sum_{j>i} Lmat(-Q_j) (-U'_ij),    vec(a (x) b) = Lmat(a) vec(b),
+// so one DMMA (A = Lmat(-Q_j), B = column j of -U' over 8 rows) serves 8 rows.  Per rod: 107 updates, 23
+// normalisations, 20 back-substitution DMMAs.  Stages 2-4 are [16 x 16] x [16 x 3] DMMA contractions in the same
+// warp (16 DMMAs; Q never leaves the SM): 166 DMMAs in all.
 //
 // Pivoting: the order is static (pivot k = row k).  The left-preconditioned operator I - 1/2 S diag(kappa) has
 // |c_kk| >= 1 and measured sub-diagonal growth <= 0.15 for |K| <= 10 and <= 2.4 for |K| <= 300, so a search would
@@ -62,8 +66,15 @@ struct DmmaScratch {
     static constexpr int gam = lbs + 48;        // [3][16] Gamma by node
     static constexpr int ns = gam + 48;         // [3][16] n by reduced row
     static constexpr int qnode = ns + 48;       // [16][4] quaternions by node (slot M = base node)
-    static constexpr int total = qnode + 64;    // 624 doubles
+    static constexpr int ust = qnode + 64;      // -U' of every pivot row, [col j][row i][s] from ucol(j) (see below)
+    static constexpr int total = ust + 740;     // 1364 doubles
 };
+// Column j of the stored -U'.  Column j < 8 is written by steps k <= 6 and read for rows i < j only, so it needs 7
+// rows and shares a 92-double slot with column j + 8 (16 rows): one store pointer serves both column tiles.  The slot
+// stride is 12 mod 16 doubles, so the eight columns one B fragment stores start on distinct bank quads and a step's
+// store is conflict free.  A back-substitution read is 32 consecutive doubles (8 rows, those at or below j unused).
+__host__ __device__ constexpr int ucol(int j) { return j < 8 ? 92 * j + 64 : 92 * (j - 8); }
+static_assert(ucol(7) + 32 <= 740, "DmmaScratch::ust size");
 constexpr size_t kDmmaSmem = (kDmmaTabDoubles + (kDmmaThreads / 32) * DmmaScratch::total) * sizeof(double);
 
 #ifndef SRI_DMMA_VOLATILE
@@ -143,8 +154,7 @@ __global__ void __launch_bounds__(kDmmaThreads, SRI_DMMA_MINBLOCKS) fused16_dmma
     // Rmat(b)[r][s] = sg(r,s) b[r^s]: rows (+,-,-,-), (+,+,+,-), (+,-,+,+), (+,+,-,+)
     const unsigned neg_tab = 0x428Eu;  // bit (4r+s) set where sg(r,s) = -1: r0: s1,s2,s3; r1: s3; r2: s1; r3: s2
     const unsigned sgL_mask = ((neg_tab >> (4 * rr + cp)) & 1u) << 31;
-    const double dpiv0 = (hi == 0 && rr == cp) ? 1.0 : 0.0;
-    const double dpiv1 = (hi == 1 && rr == cp) ? 1.0 : 0.0;
+    const double dpiv0 = (hi == 0 && rr == cp) ? 1.0 : 0.0;  // the pivot's tile row is live only for even k
     const unsigned hi_mask = hi ? 0x7fffffffu : 0u;
     // normalisation operand: B[q = cp][n = rho]; even n = 2 s' carries Rmat(conj c)[s'][q] = sg(s',q) conj(c)[s'^q]
     // (odd columns feed C-fragment register 1, which is discarded: don't-care)
@@ -153,6 +163,8 @@ __global__ void __launch_bounds__(kDmmaThreads, SRI_DMMA_MINBLOCKS) fused16_dmma
     const unsigned sgN_mask = ((((neg_tab >> (4 * sp + cp)) & 1u) != 0) != (idxN != 0)) ? 0x80000000u : 0u;
     // identity entries of the assembly: tile (t, ct), register e holds delta_ij iff rr == 0, hi == e, cp == t - 4 ct
     const int diag_code = (rr == 0) ? (4 * hi + cp) : -1;
+    // -U' store of step k: lane (rho, cp) holds component cp of column 8 ct + rho
+    double* const ustl = scr + DmmaScratch::ust + 92 * rho + cp;
     // B-fragment read offset into a [4][20] right-hand side
     const int offb = (rho < 3 ? rho : 3) * 20 + cp;
     // stages 2+3 in one contraction: columns 0..2 = r' (bs), columns 3..5 = reversed fbar (fbs), the rest the zero row of bs
@@ -223,10 +235,13 @@ __global__ void __launch_bounds__(kDmmaThreads, SRI_DMMA_MINBLOCKS) fused16_dmma
                     }
                 }
         }
-        // ---- Gauss-Jordan over the quaternions on DMMA, static pivot order, software pipelined -----------------
-        // Iteration k issues the rank-4 update of step k and, behind it, everything step k+1 needs: its tile row is
-        // updated first, then the next pivot row is gathered and normalised; each la[t] is re-gathered for step k+1 as
-        // soon as tile row t has been updated.  k = -1 is the prologue (no update).
+        // ---- forward elimination over the quaternions on DMMA, static pivot order, software pipelined ----------
+        // Step k normalises pivot row k, stores it (-U'_k) to shared memory and eliminates column k from the rows
+        // below it.  A stored pivot row is never read from the tiles again, so step k updates only tile rows
+        // t >= (k+1)/2 (the pivot's own tile row only while row k+1 shares it), and the last step updates nothing.
+        // Iteration k issues the rank-4 update of step k and, behind it, everything step k+1 needs: its tile row, the
+        // first live one, is updated first, then the next pivot row is gathered and normalised; each la[t] is
+        // re-gathered for step k+1 as soon as tile row t has been updated.  k = -1 is the prologue (no update).
         // Scalar FP64 instructions share the pipe with the DMMAs and queue behind them, so the serial scalar chain is
         // kept to three operations per step: U (x) conj(c_kk) is itself a DMMA, whose (column k, w) entry is |c_kk|^2,
         // and its reciprocal (MUFU seed, e = 1 - nu r0, t2 = e + e^2) is folded into the scaling of that product.
@@ -236,10 +251,10 @@ __global__ void __launch_bounds__(kDmmaThreads, SRI_DMMA_MINBLOCKS) fused16_dmma
 #pragma unroll
         for (int k = -1; k < 15; ++k) {
             const int kn = k + 1;  // the step being prepared
-            const bool upd = (k >= 0) && (MS != 0 || k < M);
+            const bool upd = (k >= 0) && (k < 14) && (MS != 0 || k < M - 1);
             const bool prep = (kn < 15) && (MS != 0 || kn < M);
             const int nt = (kn >> 1) & 7, nh = kn & 1, nc = (kn >> 3) & 1, ncp = (kn & 7) >> 1, ne = kn & 1;
-            // 1. step k on the tile row of the next pivot
+            // 1. step k on the tile row of the next pivot (= its first live tile row)
             if (upd) {
 #pragma unroll
                 for (int ct = 0; ct < 2; ++ct)
@@ -272,26 +287,25 @@ __global__ void __launch_bounds__(kDmmaThreads, SRI_DMMA_MINBLOCKS) fused16_dmma
                 thr = (int)(((long long)hn + 0x3ff00000LL + (long long)growth_log) >> 1);
                 if (hn < 0x05000000 || hn >= 0x7ff00000) thr = -1;  // zero / tiny / negative / inf / NaN pivot norm
             }
-            // 2. step k on the other tile rows; la[t] is re-gathered for step k+1 once tile row t is done
+            // 2. step k on the other live tile rows; la[t] is re-gathered for step k+1 once tile row t is done (step
+            //    k+1 needs tile rows t >= (kn+1)/2: the next pivot's own tile row only when kn is even)
             const int srcL = srcL_base + ncp;
 #pragma unroll
-            for (int tt = 0; tt < 8; ++tt) {
-                const int t = (nt + tt) & 7;  // the next pivot's tile row first (already updated above)
-                if (upd && tt != 0) {
+            for (int t = nt; t < 8; ++t) {
+                if (upd && t != nt) {
 #pragma unroll
                     for (int ct = 0; ct < 2; ++ct)
                         if (8 * ct + 7 > k) dmma(c[t][ct][0], c[t][ct][1], la[t], un[ct]);
                 }
-                if (prep) {
+                if (prep && (t != nt || nh == 0)) {
                     const double v = __shfl_sync(0xffffffffu, c[t][nc][ne], srcL);
                     const unsigned h = (unsigned)__double2hiint(v) & 0x7fffffffu;
-                    if (t > nt) mx = max(mx, h);
-                    else if (t == nt && nh == 0) mx = max(mx, h & hi_mask);
+                    mx = max(mx, t != nt ? h : (h & hi_mask));
                     la[t] = flip_sign(v, sgL_mask);
-                    if (tt == 0) la[t] -= nh ? dpiv1 : dpiv0;  // pivot row: Rmat(c_kk - 1) leaves the normalised row
+                    if (t == nt) la[t] -= dpiv0;  // pivot row: Rmat(c_kk - 1) leaves the normalised row
                 }
             }
-            // 3. -U' = -(U (x) conj c_kk) / nu for the next step
+            // 3. -U' = -(U (x) conj c_kk) / nu for the next step, and into the store for the back-substitution
             if (prep) {
                 bad = bad || ((int)mx > thr);
 #pragma unroll
@@ -302,20 +316,49 @@ __global__ void __launch_bounds__(kDmmaThreads, SRI_DMMA_MINBLOCKS) fused16_dmma
 #else
                         const double a = un0[ct] * r0n; un[ct] = fma(a, t2, a);
 #endif
+                        ustl[(ct ? ucol(8) : ucol(0)) + 4 * kn] = un[ct];
                     }
             }
         }
         const bool flagged = __any_sync(0xffffffffu, bad);
+        __syncwarp();  // the -U' stores above are read across lanes below
+        // ---- back-substitution on DMMA: with W = -U' (stored) and C' = -Q,  C'_i = W_i,15 + sum_{j>i} Lmat(C'_j) W_ij
+        //      (vec(a (x) b) = Lmat(a) vec(b)).  C' lives in one C tile per 8-row block, component s on the m axis
+        //      (m >= 4 stays zero) and row 8b + n on the n axis, so one DMMA subtracts Q_j (x) U'_ij from 8 rows: the
+        //      A operand is Lmat(C'_j), one shuffle and a sign; the B operand is column j of W over the block.
+        //      C'_j is final once every j' > j has been applied, and is written to qnode as Q_j.
+        {
+            // the lane is re-read here so that its constants below are not held (and spilled) across the elimination
+            int ln;
+            asm volatile("mov.u32 %0, %%laneid;" : "=r"(ln));
+            const int qm = ln >> 2, qs = ln & 3;  // A: row m, k index s;  B: k index s, n = row within the block
+            const double* ust = scr + DmmaScratch::ust;
+            double y[2][2];
+#pragma unroll
+            for (int b = 0; b < 2; ++b)
+#pragma unroll
+                for (int e = 0; e < 2; ++e) y[b][e] = qm < 4 ? ust[ucol(15) + 4 * (8 * b + 2 * qs + e) + (qm & 3)] : 0.0;
+            // Lmat(a)[r][s] = sg(r,s) a[r^s]: rows (+,-,-,-), (+,+,-,+), (+,+,+,-), (+,-,+,+)
+            const unsigned sgQ_mask = ((0x284Eu >> (4 * (qm & 3) + qs)) & 1u) << 31;
+            const int srcQ_base = 4 * (qm ^ qs);  // m >= 4 reads the zero rows 4..7: the padded A rows stay zero
+#pragma unroll
+            for (int j = 14; j >= 0; --j) {
+                if (MS != 0 || j < M) {
+                    const int b = j >> 3, n = j & 7;
+                    const double v = __shfl_sync(0xffffffffu, y[b][n & 1], srcQ_base + (n >> 1));  // C'_j[qm ^ qs]
+                    if (qm < 4 && qs == 0) qnode[4 * j + qm] = flip_sign(v, 0x80000000u);
+                    const double a = flip_sign(v, sgQ_mask);
+#pragma unroll
+                    for (int bb = 0; bb <= b; ++bb)
+                        if (8 * bb < j) dmma(y[bb][0], y[bb][1], a, ust[ucol(j) + 32 * bb + ln]);
+                }
+            }
+        }
         cp_async_wait<0>();
         // a flagged rod needs row pivoting: it is handed to the scalar kernel; its stores below are suppressed (no
         // divergent `continue`, which would wrap every later shuffle in WARPSYNC/ENDCOLLECTIVE pairs)
         const bool keep = !(flagged && p.rod_list);
         if (!keep && lane == 0) p.rod_list[atomicAdd(p.rod_count, 1)] = (int)rod;
-        // ---- the solution is column 15: lanes cp == 3, register [t][1][1] -> qnode[i][r] ----------------------
-        if (cp == 3) {
-#pragma unroll
-            for (int t = 0; t < 8; ++t) qnode[4 * (2 * t + hi) + rr] = c[t][1][1];
-        }
         __syncwarp();
         if (lane < 4) qnode[4 * M + lane] = kb[16 * lane + 15];  // base node: q0
         if (p.info && keep && lane == 0) p.info[rod] = flagged ? -1 : 0;

@@ -15,6 +15,8 @@ Step k (static pivot order, growth check instead of a search):
     u'_j  = u_j (x) c_kk^-1                 (pivot row normalised: one DMMA per column tile)
     c_ij -= u'_j (x) c_ik   for all rows i  (vec(a (x) b) = Rmat(b) vec(a): [Rmat(c_ik) stacked] * [-U'] : DMMAs)
     pivot row itself: Rmat(c_kk - 1), which leaves exactly u'_j.
+`solve_rod` is that Gauss-Jordan over all rows; `solve_rod_lu` is the schedule the kernel runs: the same steps on the
+rows below the pivot only, then a back-substitution on DMMA.
 """
 from __future__ import annotations
 
@@ -118,6 +120,112 @@ def solve_rod(Stx, K, q0, M, growth=8.0):
     for t in range(8):
         sel = CP == 3
         Q[2 * t + HI[sel], R[sel]] = c[t, 1, 1][sel]
+    return Q[:M], flagged
+
+
+# ---- the shipped schedule: elimination below the pivot only, back-substitution with the solved quaternion as A -------
+# Lmat(a)[r][s] = SGL[r][s] * a[r ^ s]   (vec(a (x) b) = Lmat(a) vec(b))
+SGL = np.array([[1, -1, -1, -1], [1, 1, -1, 1], [1, 1, 1, -1], [1, -1, 1, 1]], dtype=np.float64)
+STAGE_DMMAS = 16  # stages 2-4 of the kernel: two [16 x 16] x [16 x 3] contractions, 2 row tiles x 4 k steps each
+
+
+def w_col(j):
+    """Start of column j of the per-warp store of -U' ([col j][row i][s], doubles).  Column j < 8 is only written by
+    steps k <= 6 and read for rows i < j: 7 rows, in the 92-double slot of column j + 8 (16 rows).  The slot stride is
+    12 mod 16, so the eight columns of one B fragment start on distinct bank quads (conflict-free stores)."""
+    j = np.asarray(j)
+    return np.where(j < 8, 92 * j + 64, 92 * (j - 8))
+
+
+W_DOUBLES = 740
+
+
+def solve_rod_lu(Stx, K, q0, M, growth=8.0, stats=None):
+    """Same system and same pivot order as solve_rod, on the kernel's schedule:
+    forward  step k updates only tile rows t >= (k+1)//2 (rows at or above a stored pivot row are dead); the
+             last step updates nothing; -U'_k (B-fragment layout: lane holds component CP of column 8ct+RHO) is
+             stored to W[w_col(8ct+RHO) + 4k + CP].
+    backward with C' = -Q accumulated in one C tile per 8-row block (C'[s][n] = row 8b+n, component s; m >= 4 zero):
+             -Q_i = W_i,15 + sum_{j>i} Lmat(-Q_j) W_ij, j = M-1..0; A = Lmat(C'_j) by one shuffle and a sign,
+             B = W column j over the block (one contiguous 32-double read).
+    Returns (Q [M][4], flagged); `stats` (dict) collects the DMMA count per kind."""
+    st = stats if stats is not None else {}
+    for key in ("update", "normalise", "backsub"):
+        st.setdefault(key, 0)
+    kx = np.zeros((4, 16))
+    kx[1:, :M] = K[:, :M]
+    kx[:, 15] = q0
+    c = np.zeros((8, 2, 2, 32))
+    for t in range(8):
+        for ct in range(2):
+            for e in range(2):
+                i = 2 * t + HI
+                j = 8 * ct + 2 * CP + e
+                diag = ((R == 0) & (i == j) & (j < 15)).astype(np.float64)
+                c[t, ct, e] = Stx[i, j] * kx[R, j] + diag
+    W = np.full(W_DOUBLES, np.nan)  # rows never written must never reach a live result
+    flagged = False
+    sgL = SG[R, CP]
+    srcL_base = 16 * (LANES >> 4) + 4 * (R ^ CP)
+    n_even = (RHO & 1) == 0
+    sp = RHO >> 1
+    idxN = sp ^ CP
+    conj = np.where(idxN == 0, 1.0, -1.0)
+    sgN = np.where(n_even, -SG[sp, CP] * conj, 0.0)
+    for k in range(M):
+        kt, kh, kc, kcp, ke = k >> 1, k & 1, k >> 3, (k & 7) >> 1, k & 1
+        cts = [ct for ct in range(2) if 8 * ct + 7 > k]
+        t0 = (k + 1) >> 1  # first live tile row: kt itself only while the row below the pivot (2kt + 1) shares it
+        src = 16 * kh + 4 * CP + (LANES >> 3)
+        Ub = {}
+        for ct in range(kc, 2):
+            v0 = shfl(c[kt, ct, 0], src)
+            v1 = shfl(c[kt, ct, 1], src)
+            Ub[ct] = np.where((RHO & 1) == 1, v1, v0)
+        pcs = shfl(c[kt, kc, ke], 16 * kh + 4 * idxN + kcp)
+        bn0 = sgN * pcs
+        un0 = {ct: mma_m8n8k4(np.zeros(32), np.zeros(32), Ub[ct], bn0)[0] for ct in Ub}
+        st["normalise"] += len(Ub)
+        nu = -shfl(un0[kc], np.full(32, 4 * (k & 7)))
+        inv = 1.0 / nu
+        srcL = srcL_base + kcp
+        La = {}
+        colmax = np.zeros(32)
+        for t in range(t0, 8):
+            v = shfl(c[t, kc, ke], srcL)
+            if t > kt:
+                colmax = np.maximum(colmax, np.abs(v))
+            else:  # t == kt, kh == 0: the row below the pivot in the same tile
+                colmax = np.maximum(colmax, np.where(HI > kh, np.abs(v), 0.0))
+            a = sgL * v
+            if t == kt:
+                a = a - ((HI == kh) & (R == CP)).astype(np.float64)
+            La[t] = a
+        if not (colmax.max() ** 2 <= growth * growth * nu[0]) or not (nu[0] > 1e-300):
+            flagged = True
+        for ct in cts:
+            d0 = un0[ct] * inv
+            W[w_col(8 * ct + RHO) + 4 * k + CP] = d0
+            if k < M - 1:
+                for t in range(t0, 8):
+                    c[t, ct, 0], c[t, ct, 1] = mma_m8n8k4(c[t, ct, 0], c[t, ct, 1], La[t], d0)
+                    st["update"] += 1
+    # ---- back-substitution --------------------------------------------------------------------------------------
+    sgLm = SGL[RHO & 3, CP]
+    y = {}
+    for b in range(2):
+        y[b] = [np.where(RHO < 4, W[w_col(15) + 4 * (8 * b + 2 * CP + e) + (RHO & 3)], 0.0) for e in range(2)]
+    Q = np.zeros((16, 4))
+    for j in range(M - 1, -1, -1):
+        b, n = j >> 3, j & 7
+        v = shfl(y[b][n & 1], 4 * (RHO ^ CP) + (n >> 1))  # lane (rho, cp) gets C'_j[rho ^ cp]; rho >= 4: zero rows
+        sel = (CP == 0) & (RHO < 4)
+        Q[j, RHO[sel]] = -v[sel]
+        a = sgLm * v
+        for bb in range(b + 1):
+            if 8 * bb < j:  # blocks holding a row i < j
+                y[bb][0], y[bb][1] = mma_m8n8k4(y[bb][0], y[bb][1], a, W[w_col(j) + 32 * bb + LANES])
+                st["backsub"] += 1
     return Q[:M], flagged
 
 
