@@ -59,6 +59,26 @@ class NewtonReport(ctypes.Structure):
     ]
 
 
+class StaticProblem(ctypes.Structure):
+    """struct sri_static_problem (include/sri.h)."""
+
+    _fields_ = [
+        ("batch", c_int64), ("ne", c_int),
+        ("H_diag", c_void_p), ("F_tip", c_void_p), ("M_tip", c_void_p), ("K0", c_void_p),
+        ("q0", c_void_p), ("Gamma", c_void_p), ("fbar", c_void_p), ("lbar", c_void_p),
+    ]
+
+
+class StaticProblemGrad(ctypes.Structure):
+    """struct sri_static_problem_grad (include/sri.h)."""
+
+    _fields_ = [
+        ("gF_tip", c_void_p), ("gM_tip", c_void_p), ("gK0", c_void_p), ("gH", c_void_p),
+        ("gq0", c_void_p), ("gGamma", c_void_p), ("gfbar", c_void_p), ("glbar", c_void_p),
+        ("lambda_", c_void_p), ("resid", c_void_p), ("info", c_void_p),
+    ]
+
+
 ALLREDUCE_FN = ctypes.CFUNCTYPE(c_int, POINTER(c_double), c_void_p)  # sri_allreduce_fn
 
 # every symbol include/sri.h declares: name -> (restype, argtypes)
@@ -88,6 +108,8 @@ SYMBOLS = {
     "sri_integrate_all_per_device": (c_int, [c_void_p, POINTER(RodBatch)]),
     "sri_newton_static_shape_sharded": (c_int, [c_void_p, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_double,
                                                 c_int, c_double, POINTER(NewtonReport)]),
+    "sri_newton_static_problem_sharded": (c_int, [c_void_p, POINTER(StaticProblem), c_void_p, c_double, c_int, c_double,
+                                                  POINTER(NewtonReport)]),
     "sri_nccl_unique_id": (c_int, [c_void_p]),
     "sri_nccl_init": (c_int, [c_void_p, c_int, c_int, c_void_p]),
     "sri_nccl_finalize": (c_int, [c_void_p]),
@@ -105,11 +127,14 @@ SYMBOLS = {
     "sri_galerkin_residual": (c_int, [c_void_p, c_int64, c_int] + [c_void_p] * 9),
     "sri_galerkin_residual_vjp": (c_int, [c_void_p, c_int64, c_int] + [c_void_p] * 15),
     "sri_static_shape_vjp": (c_int, [c_void_p, c_int64, c_int] + [c_void_p] * 6 + [c_int] + [c_void_p] * 7),
+    "sri_static_problem_vjp": (c_int, [c_void_p, POINTER(StaticProblem), c_void_p, c_void_p, c_int, POINTER(StaticProblemGrad)]),
     "sri_generalised_forces": (c_int, [c_void_p, c_int64, c_int, c_void_p, c_void_p]),
     "sri_shape_jacobian": (c_int, [c_void_p, c_int64, c_int] + [c_void_p] * 8),
     "sri_solve_small_batched": (c_int, [c_void_p, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
     "sri_newton_static_shape": (c_int, [c_void_p, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_double,
                                         c_int, c_double, c_int64, ALLREDUCE_FN, c_void_p, POINTER(NewtonReport)]),
+    "sri_newton_static_problem": (c_int, [c_void_p, POINTER(StaticProblem), c_void_p, c_double, c_int, c_double, c_int64,
+                                          ALLREDUCE_FN, c_void_p, POINTER(NewtonReport)]),
     "sri_generate_rods": (c_int, [c_void_p, c_uint64, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_void_p]),
     "sri_last_error_string": (c_char_p, []),
     "sri_set_timing": (c_int, [c_void_p, c_int]),

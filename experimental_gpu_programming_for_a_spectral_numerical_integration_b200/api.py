@@ -408,24 +408,33 @@ class SpectralRodIntegrator:
         return grads
 
     def static_shape_vjp(self, F_tip, M_tip, qe, gqe, H_diag=(1.0, 1.0, 0.77), K0=None, refine_steps: int = 3, info=None,
-                         want=("F_tip", "M_tip", "K0", "H"), out=None):
-        """sri_static_shape_vjp: gradients -(dg/dtheta)^T lam of the equilibrium qe [batch][3*ne] (the caller's converged
-        newton_static_shape solution) for the cotangent gqe, with respect to the parameters named in `want` among F_tip,
-        M_tip, K0, H (per rod, [batch][3]); "lambda" ([batch][3*ne], the adjoint solution) and "resid" ([batch], its relative
-        residual) may be requested too.  info: optional int32 [batch] pivot report.  Returns a dict of the requested arrays
-        (allocated unless given in the dict `out`)."""
+                         want=("F_tip", "M_tip", "K0", "H"), out=None, q0=None, Gamma=None, fbar=None, lbar=None):
+        """Gradients -(dg/dtheta)^T lam of the equilibrium qe [batch][3*ne] (the caller's converged newton_static_shape
+        solution, with the same q0, Gamma, fbar, lbar) for the cotangent gqe, with respect to the parameters named in `want`
+        among F_tip, M_tip, K0, H (per rod, [batch][3]), q0, Gamma, fbar, lbar; "lambda" ([batch][3*ne], the adjoint solution)
+        and "resid" ([batch], its relative residual) may be requested too.  info: optional int32 [batch] pivot report.
+        Returns a dict of the requested arrays (allocated unless given in the dict `out`).  sri_static_problem_vjp when a
+        clamp rotation, Gamma or a distributed load is given or its gradient wanted, else sri_static_shape_vjp."""
         self._follow_torch(qe)
-        batch, n = qe.shape[0], qe.shape[1]
+        batch, n, N = qe.shape[0], qe.shape[1], self.N
         H = np.ascontiguousarray(np.asarray(H_diag, dtype=np.float64))
-        shapes = {"F_tip": (batch, 3), "M_tip": (batch, 3), "K0": (batch, 3, self.N), "H": (batch, 3), "lambda": (batch, n),
-                  "resid": (batch,)}
+        shapes = {"F_tip": (batch, 3), "M_tip": (batch, 3), "K0": (batch, 3, N), "H": (batch, 3), "lambda": (batch, n),
+                  "resid": (batch,), "q0": (batch, 4), "Gamma": (batch, 3, N), "fbar": (batch, 3, N), "lbar": (batch, 3, N)}
         given = out or {}
         res = {key: given[key] if given.get(key) is not None else _empty_like_kind(qe, shapes[key]) for key in want}
         g = lambda key: _ptr(res.get(key), key)
-        _lib.check(self._lib.sri_static_shape_vjp(
-            self._h, batch, n // 3, H.ctypes.data, _ptr(F_tip, "F_tip"), _ptr(M_tip, "M_tip"), _ptr(K0, "K0"), _ptr(qe, "qe"),
-            _ptr(gqe, "gqe"), int(refine_steps), g("F_tip"), g("M_tip"), g("K0"), g("H"), g("lambda"), g("resid"),
-            _ptr(info, "info", np.int32)), "sri_static_shape_vjp")
+        if all(a is None for a in (q0, Gamma, fbar, lbar)) and not set(want) & set(_PROBLEM_INPUTS):
+            _lib.check(self._lib.sri_static_shape_vjp(
+                self._h, batch, n // 3, H.ctypes.data, _ptr(F_tip, "F_tip"), _ptr(M_tip, "M_tip"), _ptr(K0, "K0"),
+                _ptr(qe, "qe"), _ptr(gqe, "gqe"), int(refine_steps), g("F_tip"), g("M_tip"), g("K0"), g("H"), g("lambda"),
+                g("resid"), _ptr(info, "info", np.int32)), "sri_static_shape_vjp")
+            return res
+        prob = _problem(batch, n // 3, H, F_tip, M_tip, K0, q0, Gamma, fbar, lbar)
+        grads = _lib.StaticProblemGrad(gF_tip=g("F_tip"), gM_tip=g("M_tip"), gK0=g("K0"), gH=g("H"), gq0=g("q0"),
+                                       gGamma=g("Gamma"), gfbar=g("fbar"), glbar=g("lbar"), lambda_=g("lambda"),
+                                       resid=g("resid"), info=_ptr(info, "info", np.int32))
+        _lib.check(self._lib.sri_static_problem_vjp(self._h, ctypes.byref(prob), _ptr(qe, "qe"), _ptr(gqe, "gqe"),
+                                                    int(refine_steps), ctypes.byref(grads)), "sri_static_problem_vjp")
         return res
 
     def generalised_forces(self, Lambda, ne: int, out=None):
@@ -452,10 +461,13 @@ class SpectralRodIntegrator:
         return out
 
     def newton_static_shape(self, F_tip, M_tip, ne: int, H_diag=(1.0, 1.0, 0.77), qe=None, K0=None, tol: float = 1e-10,
-                            max_iter: int = 30, fd_step: float = 1e-6, total_dof: int = 0, allreduce=None):
-        """sri_newton_static_shape: the Newton loop of the static shape problem inside the library.  qe (in/out, zeros when
-        omitted) [batch][3*ne]; allreduce(norms) -- optional callable that replaces the 2-element float64 numpy array
-        [sum g^2, max |g|] by its reduction over the ranks.  Returns (qe, dict report)."""
+                            max_iter: int = 30, fd_step: float = 1e-6, total_dof: int = 0, allreduce=None, q0=None, Gamma=None,
+                            fbar=None, lbar=None):
+        """The Newton loop of the static shape problem inside the library: sri_newton_static_shape, or
+        sri_newton_static_problem when a clamp rotation q0 [batch][4], Gamma or a global-frame distributed load fbar / lbar
+        ([batch][3][N] each) is given.  qe (in/out, zeros when omitted) [batch][3*ne]; allreduce(norms) -- optional callable
+        that replaces the 2-element float64 numpy array [sum g^2, max |g|] by its reduction over the ranks.  Returns
+        (qe, dict report)."""
         self._follow_torch(F_tip)
         batch = F_tip.shape[0]
         if qe is None:
@@ -477,12 +489,19 @@ class SpectralRodIntegrator:
                 return 1
 
         cb = _lib.ALLREDUCE_FN(_cb) if allreduce is not None else _lib.ALLREDUCE_FN()
-        rc = self._lib.sri_newton_static_shape(self._h, batch, int(ne), H.ctypes.data, _ptr(F_tip, "F_tip"), _ptr(M_tip, "M_tip"),
-                                               _ptr(K0, "K0"), _ptr(qe, "qe"), float(tol), int(max_iter), float(fd_step),
-                                               int(total_dof), cb, None, ctypes.byref(rep))
+        if all(a is None for a in (q0, Gamma, fbar, lbar)):
+            where = "sri_newton_static_shape"
+            rc = self._lib.sri_newton_static_shape(self._h, batch, int(ne), H.ctypes.data, _ptr(F_tip, "F_tip"),
+                                                   _ptr(M_tip, "M_tip"), _ptr(K0, "K0"), _ptr(qe, "qe"), float(tol), int(max_iter),
+                                                   float(fd_step), int(total_dof), cb, None, ctypes.byref(rep))
+        else:
+            where = "sri_newton_static_problem"
+            prob = _problem(batch, ne, H, F_tip, M_tip, K0, q0, Gamma, fbar, lbar)
+            rc = self._lib.sri_newton_static_problem(self._h, ctypes.byref(prob), _ptr(qe, "qe"), float(tol), int(max_iter),
+                                                     float(fd_step), int(total_dof), cb, None, ctypes.byref(rep))
         if failure:
             raise failure[0]
-        _lib.check(rc, "sri_newton_static_shape")
+        _lib.check(rc, where)
         return qe, _report_dict(rep)
 
     def solve_small_batched(self, A, b, out=None, info=None):
@@ -551,6 +570,16 @@ def scale_for_length(length, K, Gamma=None, fbar=None, lbar=None):
     return sc(K), sc(Gamma), sc(fbar), sc(lbar)
 
 
+_PROBLEM_INPUTS = ("q0", "Gamma", "fbar", "lbar")
+
+
+def _problem(batch, ne, H, F_tip, M_tip, K0, q0, Gamma, fbar, lbar):
+    """struct sri_static_problem over the given buffers (H: a contiguous numpy array the caller keeps alive)."""
+    return _lib.StaticProblem(batch=batch, ne=int(ne), H_diag=H.ctypes.data, F_tip=_ptr(F_tip, "F_tip"),
+                              M_tip=_ptr(M_tip, "M_tip"), K0=_ptr(K0, "K0"), q0=_ptr(q0, "q0"), Gamma=_ptr(Gamma, "Gamma"),
+                              fbar=_ptr(fbar, "fbar"), lbar=_ptr(lbar, "lbar"))
+
+
 def _report_dict(rep) -> dict:
     return {"iterations": rep.iterations, "converged": bool(rep.converged), "integrations": rep.integrations,
             "rms": rep.rms, "max_abs": rep.max_abs, "rms_history": list(rep.rms_history[:rep.history_len]),
@@ -616,15 +645,23 @@ class MultiDeviceIntegrator:
         return {k: v for k, v in outs.items() if v is not None}
 
     def newton_static_shape(self, F_tip, M_tip, ne: int, H_diag=(1.0, 1.0, 0.77), qe=None, K0=None, tol: float = 1e-10,
-                            max_iter: int = 30, fd_step: float = 0.0):
+                            max_iter: int = 30, fd_step: float = 0.0, q0=None, Gamma=None, fbar=None, lbar=None):
+        """Host buffers, rods sharded over the devices: sri_newton_static_shape_sharded, or sri_newton_static_problem_sharded
+        when q0, Gamma, fbar or lbar is given."""
         batch = F_tip.shape[0]
         if qe is None:
             qe = np.zeros((batch, 3 * int(ne)))
         H = np.ascontiguousarray(np.asarray(H_diag, dtype=np.float64))
         rep = _lib.NewtonReport()
-        _lib.check(self._lib.sri_newton_static_shape_sharded(
-            self._mh, batch, int(ne), H.ctypes.data, _ptr(F_tip, "F_tip"), _ptr(M_tip, "M_tip"), _ptr(K0, "K0"), _ptr(qe, "qe"),
-            float(tol), int(max_iter), float(fd_step), ctypes.byref(rep)), "sri_newton_static_shape_sharded")
+        if all(a is None for a in (q0, Gamma, fbar, lbar)):
+            _lib.check(self._lib.sri_newton_static_shape_sharded(
+                self._mh, batch, int(ne), H.ctypes.data, _ptr(F_tip, "F_tip"), _ptr(M_tip, "M_tip"), _ptr(K0, "K0"),
+                _ptr(qe, "qe"), float(tol), int(max_iter), float(fd_step), ctypes.byref(rep)), "sri_newton_static_shape_sharded")
+        else:
+            prob = _problem(batch, ne, H, F_tip, M_tip, K0, q0, Gamma, fbar, lbar)
+            _lib.check(self._lib.sri_newton_static_problem_sharded(
+                self._mh, ctypes.byref(prob), _ptr(qe, "qe"), float(tol), int(max_iter), float(fd_step), ctypes.byref(rep)),
+                "sri_newton_static_problem_sharded")
         return qe, _report_dict(rep)
 
 

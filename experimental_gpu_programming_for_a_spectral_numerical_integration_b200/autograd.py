@@ -3,10 +3,11 @@
     Q, r, n, m = integrate_all(integ, K, F_tip, M_tip, q0=..., r0=..., Gamma=..., fbar=..., lbar=...)
     K = strain_from_modes(integ, qe, ne)
     g = galerkin_residual(integ, K, Q, m, M_tip, ne, H_diag, K0=..., q0=...)
-    qe = static_shape(integ, F_tip, M_tip, ne, H_diag, K0=..., qe0=...)      (the equilibrium, differentiated implicitly)
+    qe = static_shape(integ, F_tip, M_tip, ne, H_diag, K0=..., qe0=..., q0=..., Gamma=..., fbar=..., lbar=...)
+                                                                           (the equilibrium, differentiated implicitly)
 
 are differentiable with respect to every tensor argument: the backward pass is one sri_integrate_all_vjp launch (resp.
-sri_strain_from_modes_transpose, sri_galerkin_residual_vjp, sri_static_shape_vjp), enqueued on torch's current stream like the forward.  Only what the backward needs is
+sri_strain_from_modes_transpose, sri_galerkin_residual_vjp, sri_static_shape_vjp / sri_static_problem_vjp), enqueued on torch's current stream like the forward.  Only what the backward needs is
 saved (K, Q, n, and q0 / Gamma when given), not the graph of the forward.  Gradients are computed for the inputs that
 require them only, and outputs that receive no cotangent pass none to the library.  Tensors are CUDA float64 on the
 integrator's device; H_diag may be a 3-tensor (on any device) that requires grad, or a sequence of 3 floats.
@@ -110,33 +111,35 @@ class _GalerkinResidual(torch.autograd.Function):
 
 class _StaticShape(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, integ, ne, Hv, tol, max_iter, refine_steps, F_tip, M_tip, H_t, K0, qe0):
+    def forward(ctx, integ, ne, Hv, tol, max_iter, refine_steps, F_tip, M_tip, H_t, K0, qe0, q0, Gamma, fbar, lbar):
         qe = None if qe0 is None else qe0.detach().clone()
-        qe, rep = integ.newton_static_shape(F_tip, M_tip, ne, H_diag=Hv, qe=qe, K0=K0, tol=tol, max_iter=max_iter, fd_step=0.0)
+        qe, rep = integ.newton_static_shape(F_tip, M_tip, ne, H_diag=Hv, qe=qe, K0=K0, tol=tol, max_iter=max_iter, fd_step=0.0,
+                                            q0=q0, Gamma=Gamma, fbar=fbar, lbar=lbar)
         if not rep["converged"]:
             raise RuntimeError(f"static_shape: the Newton solve did not converge (rms {rep['rms']:.3e} after "
                                f"{rep['iterations']} iterations, tol {tol:.1e}); its gradient would not be that of an equilibrium")
         ctx.integ, ctx.Hv, ctx.refine_steps = integ, Hv, refine_steps
-        ctx.save_for_backward(F_tip, M_tip, K0, qe)
+        ctx.save_for_backward(F_tip, M_tip, K0, qe, q0, Gamma, fbar, lbar)
         return qe
 
     @staticmethod
     @once_differentiable
     def backward(ctx, gqe):
-        F_tip, M_tip, K0, qe = ctx.saved_tensors
-        names = ("F_tip", "M_tip", "H", "K0")
-        want = [name for name, need in zip(names, ctx.needs_input_grad[6:10]) if need]
+        F_tip, M_tip, K0, qe, q0, Gamma, fbar, lbar = ctx.saved_tensors
+        names = ("F_tip", "M_tip", "H", "K0", "qe0", "q0", "Gamma", "fbar", "lbar")
+        want = [name for name, need in zip(names, ctx.needs_input_grad[6:]) if need and name != "qe0"]
         grads = {}
         if want:
             info = torch.empty(qe.shape[0], dtype=torch.int32, device=qe.device)
             grads = ctx.integ.static_shape_vjp(F_tip, M_tip, qe, gqe.contiguous(), H_diag=ctx.Hv, K0=K0,
-                                               refine_steps=ctx.refine_steps, info=info, want=want)
+                                               refine_steps=ctx.refine_steps, info=info, want=want, q0=q0, Gamma=Gamma,
+                                               fbar=fbar, lbar=lbar)
             bad = int((info != 0).sum())
             if bad:
                 raise RuntimeError(f"static_shape backward: {bad} rod(s) met a zero or non-finite pivot in the adjoint solve")
             if "H" in grads:
                 grads["H"] = grads["H"].sum(0)
-        return (None,) * 6 + tuple(grads.get(name) for name in names) + (None,)
+        return (None,) * 6 + tuple(grads.get(name) for name in names)
 
 
 def galerkin_residual(integ, K, Q, m, M_tip, ne: int, H_diag, K0=None, q0=None):
@@ -147,10 +150,12 @@ def galerkin_residual(integ, K, Q, m, M_tip, ne: int, H_diag, K0=None, q0=None):
 
 
 def static_shape(integ, F_tip, M_tip, ne: int, H_diag, K0=None, qe0=None, tol: float = 1e-12, max_iter: int = 30,
-                 refine_steps: int = 3):
-    """Differentiable equilibrium qe* [batch][3*ne] of tip-loaded rods: the forward is newton_static_shape with the analytic
-    Jacobian (raises unless it converges), the backward one sri_static_shape_vjp with `refine_steps` refinement steps,
-    differentiating with respect to F_tip, M_tip, H_diag (when a tensor) and K0 -- not qe0, the starting point."""
+                 refine_steps: int = 3, q0=None, Gamma=None, fbar=None, lbar=None):
+    """Differentiable equilibrium qe* [batch][3*ne] of rods under tip loads, a clamp rotation q0 [batch][4], Gamma and the
+    global-frame distributed loads fbar, lbar ([batch][3][N] each; None: identity, e1, 0): the forward is newton_static_shape
+    with the analytic Jacobian (raises unless it converges), the backward one static_shape_vjp with `refine_steps` refinement
+    steps, differentiating with respect to F_tip, M_tip, H_diag (when a tensor), K0, q0, Gamma, fbar and lbar -- not qe0,
+    the starting point."""
     H_t, Hv = _H(H_diag)
     return _StaticShape.apply(integ, int(ne), Hv, float(tol), int(max_iter), int(refine_steps), _c(F_tip), _c(M_tip), H_t,
-                              _c(K0), _c(qe0))
+                              _c(K0), _c(qe0), _c(q0), _c(Gamma), _c(fbar), _c(lbar))

@@ -88,9 +88,10 @@ struct sri_context {
     double dmma_growth = sri::kDmmaGrowthDefault;
     bool use_dmma = false;       // DMMA elimination first, row-pivoting kernel for the rods it hands back (SRI_FUSED16_IMPL)
     struct NewtonWorkspace {  // buffers of sri_newton_static_shape, kept for the next call of the same shape
-        int64_t B = -1; int ne = 0; bool has_K0 = false, analytic = false;
+        int64_t B = -1; int ne = 0; unsigned present = 0; bool analytic = false;   // present: bits K0, q0, Gamma, fbar, lbar
         double* block = nullptr;
         double *K, *Q, *m, *nn, *g0, *J, *delta, *qe, *red, *F, *Mt, *K0, *qw, *Kw, *Qw, *mw, *gw, *Fw, *Mtw, *K0w;
+        double *q0, *G, *fb, *lb, *q0w, *Gw, *fbw, *lbw;   // optional inputs of the problem and their forward-difference replicas
         int* sinfo = nullptr;            // [B] zero-pivot report of the per-rod Newton solve
         sri::NewtonState* state = nullptr;       // device: convergence flag, singular count, norm history
         sri::NewtonState* host_state = nullptr;  // two pinned mirrors: test t is copied to mirror t & 1 (followed by event t & 1)
@@ -105,7 +106,7 @@ struct sri_context {
     struct AdjointWorkspace {  // buffers of sri_static_shape_vjp, kept for the next call of the same shape
         int64_t B = -1; int ne = 0;
         double* block = nullptr;
-        double *K, *Q, *n, *m, *J, *rhs, *delta, *gKd, *gKi, *gQ, *gm, *gMd, *gMi, *gFi, *gHw, *lam;
+        double *K, *Q, *n, *m, *J, *rhs, *delta, *gKd, *gKi, *gQ, *gm, *gMd, *gMi, *gFi, *gHw, *lam, *gq0d, *gq0i;
         int *sinfo, *vinfo;      // [B] pivot reports of the J_a^T solve and of the transposed stage-1 solve
     } adjoint;
     double* d_partial = nullptr;  // block partials of galerkin_residual_kernel's norms, and its ticket counter
@@ -1569,18 +1570,18 @@ int sri_solve_small_batched(sri_handle h, int64_t batch, int n, double* A, const
 //     lam_0 = J_a^-T gqe,   lam_{k+1} = lam_k + J_a^-T (gqe - J_d^T lam_k)   (refine_steps times),
 // where J_d^T lam = Phi^T (gK_dir + gK_int) comes from chain(lam): the residual's VJP (cotangent lam) followed by the
 // integration's VJP of its (gQ, gm).  A final chain(lam) gives the parameter gradients -(dg/dtheta)^T lam and the residual.
-int sri_static_shape_vjp(sri_handle h, int64_t batch, int ne, const double* H_diag, const double* F_tip, const double* M_tip,
-                         const double* K0, const double* qe, const double* gqe, int refine_steps, double* gF_tip,
-                         double* gM_tip, double* gK0, double* gH, double* lambda, double* resid, int* info) {
-    SRI_ENTER(h);
-    if (batch < 0 || ne < 1 || ne > 8 || !H_diag || refine_steps < 0 || refine_steps > 1000 ||
-        (batch > 0 && (!F_tip || !M_tip || !qe || !gqe)))
-        return fail(SRI_ERR_INVALID_ARGUMENT, "sri_static_shape_vjp: bad arguments (1 <= ne <= 8, 0 <= refine_steps <= 1000)");
-    if (batch == 0) return SRI_OK;
+// `who` names the entry point in error messages.
+static int static_problem_vjp(sri_context* h, const sri_static_problem& P, const double* qe, const double* gqe, int refine_steps,
+                              const sri_static_problem_grad& G, const char* who) {
+    const int64_t B = P.batch;
+    const int ne = P.ne;
+    if (B < 0 || ne < 1 || ne > 8 || !P.H_diag || refine_steps < 0 || refine_steps > 1000 ||
+        (B > 0 && (!P.F_tip || !P.M_tip || !qe || !gqe)))
+        return fail(SRI_ERR_INVALID_ARGUMENT, std::string(who) + ": bad arguments (1 <= ne <= 8, 0 <= refine_steps <= 1000)");
+    if (B == 0) return SRI_OK;
     const int N = h->N, M = h->M, n = 3 * ne;
-    const int64_t B = batch;
     double H[3];
-    SRI_TRY(read_H(H_diag, H));
+    SRI_TRY(read_H(P.H_diag, H));
     auto& ws = h->adjoint;
     if (ws.B != B || ws.ne != ne || !ws.block) {
         SRI_CUDA(cudaStreamSynchronize(h->stream));
@@ -1590,9 +1591,9 @@ int sri_static_shape_vjp(sri_handle h, int64_t batch, int ne, const double* H_di
         const size_t sz[] = {up((size_t)3 * N * B), up((size_t)4 * M * B), up((size_t)3 * M * B), up((size_t)3 * M * B),
                              up((size_t)n * n * B), up((size_t)n * B), up((size_t)n * B), up((size_t)3 * N * B), up((size_t)3 * N * B),
                              up((size_t)4 * M * B), up((size_t)3 * M * B), up((size_t)3 * B), up((size_t)3 * B), up((size_t)3 * B),
-                             up((size_t)3 * B), up((size_t)n * B)};
+                             up((size_t)3 * B), up((size_t)n * B), up((size_t)4 * B), up((size_t)4 * B)};
         double** fields[] = {&ws.K, &ws.Q, &ws.n, &ws.m, &ws.J, &ws.rhs, &ws.delta, &ws.gKd, &ws.gKi, &ws.gQ, &ws.gm, &ws.gMd,
-                             &ws.gMi, &ws.gFi, &ws.gHw, &ws.lam};
+                             &ws.gMi, &ws.gFi, &ws.gHw, &ws.lam, &ws.gq0d, &ws.gq0i};
         static_assert(sizeof(sz) / sizeof(sz[0]) == sizeof(fields) / sizeof(fields[0]), "one size per workspace field");
         size_t total = 2 * up(((size_t)B + 1) / 2);
         for (size_t v : sz) total += v;
@@ -1604,21 +1605,29 @@ int sri_static_shape_vjp(sri_handle h, int64_t batch, int ne, const double* H_di
         ws.B = B; ws.ne = ne;
     }
     Staging st(h);
-    const double *dF, *dMt, *dK0, *dqe, *dgqe;
-    double *dgF, *dgMt, *dgK0, *dgH, *dlam, *dres;
+    const double *dF, *dMt, *dK0, *dq0, *dG, *dfb, *dlb, *dqe, *dgqe;
+    double *dgF, *dgMt, *dgK0, *dgH, *dgq0, *dgG, *dgfb, *dglb, *dlam, *dres;
     int* dinfo;
-    SRI_TRY(st.in(F_tip, (size_t)B * 3, &dF));
-    SRI_TRY(st.in(M_tip, (size_t)B * 3, &dMt));
-    SRI_TRY(st.in(K0, (size_t)B * 3 * N, &dK0));
+    SRI_TRY(st.in(P.F_tip, (size_t)B * 3, &dF));
+    SRI_TRY(st.in(P.M_tip, (size_t)B * 3, &dMt));
+    SRI_TRY(st.in(P.K0, (size_t)B * 3 * N, &dK0));
+    SRI_TRY(st.in(P.q0, (size_t)B * 4, &dq0));
+    SRI_TRY(st.in(P.Gamma, (size_t)B * 3 * N, &dG));
+    SRI_TRY(st.in(P.fbar, (size_t)B * 3 * N, &dfb));
+    SRI_TRY(st.in(P.lbar, (size_t)B * 3 * N, &dlb));
     SRI_TRY(st.in(qe, (size_t)B * n, &dqe));
     SRI_TRY(st.in(gqe, (size_t)B * n, &dgqe));
-    SRI_TRY(st.out(gF_tip, (size_t)B * 3, &dgF));
-    SRI_TRY(st.out(gM_tip, (size_t)B * 3, &dgMt));
-    SRI_TRY(st.out(gK0, (size_t)B * 3 * N, &dgK0));
-    SRI_TRY(st.out(gH, (size_t)B * 3, &dgH));
-    SRI_TRY(st.out(lambda, (size_t)B * n, &dlam));
-    SRI_TRY(st.out(resid, (size_t)B, &dres));
-    SRI_TRY(st.out(info, (size_t)B, &dinfo));
+    SRI_TRY(st.out(G.gF_tip, (size_t)B * 3, &dgF));
+    SRI_TRY(st.out(G.gM_tip, (size_t)B * 3, &dgMt));
+    SRI_TRY(st.out(G.gK0, (size_t)B * 3 * N, &dgK0));
+    SRI_TRY(st.out(G.gH, (size_t)B * 3, &dgH));
+    SRI_TRY(st.out(G.gq0, (size_t)B * 4, &dgq0));
+    SRI_TRY(st.out(G.gGamma, (size_t)B * 3 * N, &dgG));
+    SRI_TRY(st.out(G.gfbar, (size_t)B * 3 * N, &dgfb));
+    SRI_TRY(st.out(G.glbar, (size_t)B * 3 * N, &dglb));
+    SRI_TRY(st.out(G.lambda, (size_t)B * n, &dlam));
+    SRI_TRY(st.out(G.resid, (size_t)B, &dres));
+    SRI_TRY(st.out(G.info, (size_t)B, &dinfo));
     double* lam = dlam ? dlam : ws.lam;
 
     // forward state at qe: K = Phi qe, the four stages (Q, n, m), the analytic Jacobian J_a
@@ -1626,26 +1635,35 @@ int sri_static_shape_vjp(sri_handle h, int64_t batch, int ne, const double* H_di
     {
         sri::FusedParams p{};
         p.batch = B; p.N = N; p.M = M; p.ops = h->d_ops16;
-        p.K = ws.K; p.F_tip = dF; p.M_tip = dMt; p.Q = ws.Q; p.n = ws.n; p.m = ws.m;
+        p.K = ws.K; p.q0 = dq0; p.Gamma = dG; p.fbar = dfb; p.lbar = dlb; p.F_tip = dF; p.M_tip = dMt;
+        p.Q = ws.Q; p.n = ws.n; p.m = ws.m;
         SRI_TRY(launch_fused(h, p));
     }
-    SRI_TRY(shape_jacobian_dev(h, B, ne, H, ws.Q, nullptr, nullptr, ws.n, ws.m, dMt, ws.J));
+    SRI_TRY(shape_jacobian_dev(h, B, ne, H, ws.Q, dq0, dG, ws.n, ws.m, dMt, ws.J));
     SRI_TRY(solve_small_dev(h, B, n, ws.J, dgqe, lam, ws.sinfo, true));
 
     sri::VjpParams vp{};
     SRI_TRY(vjp_params(h, B, &vp));
-    vp.K = ws.K; vp.Q = ws.Q; vp.n = ws.n; vp.gQ = ws.gQ; vp.gm = ws.gm; vp.gK = ws.gKi; vp.info = ws.vinfo;
+    vp.K = ws.K; vp.q0 = dq0; vp.Gamma = dG; vp.Q = ws.Q; vp.n = ws.n; vp.gQ = ws.gQ; vp.gm = ws.gm; vp.gK = ws.gKi;
+    vp.info = ws.vinfo;
     auto refine_kernel = pick_lanes_ne<PickAdjointRefine>(N, ne);
     const unsigned blocks = lane_group_blocks(h, B);
     const long long tu = (long long)n * B;
+    const bool finals = dres || dgF || dgMt || dgH || dgq0 || dgG || dgfb || dglb || dinfo;
     for (int step = 0; step <= refine_steps; ++step) {
         const bool last = step == refine_steps;
         // chain(lam): K0-gradient = H rho_bar = gK_dir, so the last chain writes gK_dir straight into that output
         double* gKd = last && dgK0 ? dgK0 : ws.gKd;
-        SRI_TRY(galerkin_residual_vjp_dev(h, B, ne, ws.K, dK0, H, ws.Q, nullptr, ws.m, dMt, lam, gKd, nullptr,
-                                          last && dgH ? ws.gHw : nullptr, ws.gQ, nullptr, ws.gm, last && dgMt ? ws.gMd : nullptr));
+        SRI_TRY(galerkin_residual_vjp_dev(h, B, ne, ws.K, dK0, H, ws.Q, dq0, ws.m, dMt, lam, gKd, nullptr,
+                                          last && dgH ? ws.gHw : nullptr, ws.gQ, last && dgq0 ? ws.gq0d : nullptr, ws.gm,
+                                          last && dgMt ? ws.gMd : nullptr));
         vp.gF_tip = last && dgF ? ws.gFi : nullptr;
         vp.gM_tip = last && dgMt ? ws.gMi : nullptr;
+        vp.gq0 = last && dgq0 ? ws.gq0i : nullptr;
+        // the last VJP writes the Gamma / fbar / lbar gradients into the outputs; the refine kernel negates them there
+        vp.gGamma = last ? dgG : nullptr;
+        vp.gfbar = last ? dgfb : nullptr;
+        vp.glbar = last ? dglb : nullptr;
         SRI_TRY(launch_vjp(h, vp));
         AdjointRefineParams rp{};
         rp.batch = B; rp.N = N; rp.ptab = h->d_ptab; rp.gqe = dgqe; rp.gKd = gKd; rp.gKi = ws.gKi;
@@ -1655,9 +1673,11 @@ int sri_static_shape_vjp(sri_handle h, int64_t batch, int ne, const double* H_di
             rp.resid = dres;
             rp.gFi = ws.gFi; rp.gMd = ws.gMd; rp.gMi = ws.gMi; rp.gHw = ws.gHw;
             rp.gF = dgF; rp.gM = dgMt; rp.gH = dgH;
+            rp.gq0d = ws.gq0d; rp.gq0i = ws.gq0i; rp.gq0 = dgq0;
+            rp.gGamma = dgG; rp.gfbar = dgfb; rp.glbar = dglb;
             rp.sinfo = ws.sinfo; rp.vinfo = ws.vinfo; rp.info = dinfo;
         }
-        if (!last || dres || dgF || dgMt || dgH || dinfo) SRI_TRY(launch(refine_kernel, blocks, 256, 0, h->stream, rp));
+        if (!last || finals) SRI_TRY(launch(refine_kernel, blocks, 256, 0, h->stream, rp));
         if (!last) {
             // lam -= J_a^-T (J_d^T lam - gqe), skipped for rods whose J_a^T is singular
             SRI_TRY(solve_small_dev(h, B, n, ws.J, ws.rhs, ws.delta, ws.sinfo, true));
@@ -1666,8 +1686,26 @@ int sri_static_shape_vjp(sri_handle h, int64_t batch, int ne, const double* H_di
         }
     }
     SRI_TRY(st.finish());
-    if (info && !is_device_pointer(info)) return singular_status(info, B, "sri_static_shape_vjp");
+    if (G.info && !is_device_pointer(G.info)) return singular_status(G.info, B, who);
     return SRI_OK;
+}
+
+int sri_static_shape_vjp(sri_handle h, int64_t batch, int ne, const double* H_diag, const double* F_tip, const double* M_tip,
+                         const double* K0, const double* qe, const double* gqe, int refine_steps, double* gF_tip,
+                         double* gM_tip, double* gK0, double* gH, double* lambda, double* resid, int* info) {
+    SRI_ENTER(h);
+    sri_static_problem P{};
+    P.batch = batch; P.ne = ne; P.H_diag = H_diag; P.F_tip = F_tip; P.M_tip = M_tip; P.K0 = K0;
+    sri_static_problem_grad G{};
+    G.gF_tip = gF_tip; G.gM_tip = gM_tip; G.gK0 = gK0; G.gH = gH; G.lambda = lambda; G.resid = resid; G.info = info;
+    return static_problem_vjp(h, P, qe, gqe, refine_steps, G, "sri_static_shape_vjp");
+}
+
+int sri_static_problem_vjp(sri_handle h, const sri_static_problem* problem, const double* qe, const double* gqe, int refine_steps,
+                           const sri_static_problem_grad* grads) {
+    SRI_ENTER(h);
+    if (!problem || !grads) return fail(SRI_ERR_INVALID_ARGUMENT, "sri_static_problem_vjp: problem and grads are required");
+    return static_problem_vjp(h, *problem, qe, gqe, refine_steps, *grads, "sri_static_problem_vjp");
 }
 
 // ---- NCCL, bound at run time --------------------------------------------------------------------------------------
@@ -1790,43 +1828,51 @@ int sri_nccl_allreduce_norms(sri_handle h, double* norm2_and_max) {
 // (8-12 stream operations) is ONE CUDA graph launch, captured once per workspace / H / tol (SRI_NEWTON_GRAPH=0 keeps eager
 // launches; so does a communicator of more than one rank, see below): worth 1 % at 10^5 rods and 5-8 % at 3 000-12 500.
 // reduce != NULL: the caller's host callback reduces the norms; the loop synchronises once per iteration.
-int sri_newton_static_shape(sri_handle h, int64_t batch, int ne, const double* H_diag, const double* F_tip,
-                            const double* M_tip, const double* K0, double* qe, double tol, int max_iter, double fd_step,
-                            int64_t total_dof, sri_allreduce_fn reduce, void* reduce_ctx, sri_newton_report* report) {
-    SRI_ENTER(h);
-    if (batch < 0 || ne < 1 || ne > 8 || !H_diag || max_iter < 0 || max_iter > 62 || !(fd_step >= 0.0) ||
-        (batch > 0 && (!F_tip || !M_tip || !qe)))
-        return fail(SRI_ERR_INVALID_ARGUMENT, "sri_newton_static_shape: bad arguments (1 <= ne <= 8, 0 <= max_iter <= 62, fd_step >= 0)");
+// `who` names the entry point in error messages.
+static int newton_static_problem(sri_context* h, const sri_static_problem& P, double* qe, double tol, int max_iter, double fd_step,
+                                 int64_t total_dof, sri_allreduce_fn reduce, void* reduce_ctx, sri_newton_report* report,
+                                 const char* who) {
+    const int64_t batch = P.batch;
+    const int ne = P.ne;
+    if (batch < 0 || ne < 1 || ne > 8 || !P.H_diag || max_iter < 0 || max_iter > 62 || !(fd_step >= 0.0) ||
+        (batch > 0 && (!P.F_tip || !P.M_tip || !qe)))
+        return fail(SRI_ERR_INVALID_ARGUMENT, std::string(who) + ": bad arguments (1 <= ne <= 8, 0 <= max_iter <= 62, fd_step >= 0)");
     const bool analytic = fd_step == 0.0;  // Jacobian from sri_shape_jacobian instead of forward differences
     const bool lagged = reduce == nullptr;
     const int N = h->N, M = h->M, n = 3 * ne;
     const int64_t B = batch, W = analytic ? 0 : (int64_t)n * B;
     double H[3];
-    SRI_TRY(read_H(H_diag, H));
+    SRI_TRY(read_H(P.H_diag, H));
     auto& ws = h->newton;
-    if (ws.B != B || ws.ne != ne || ws.has_K0 != (K0 != nullptr) || ws.analytic != analytic || !ws.block) {
+    // which optional arrays the problem has is part of the workspace key: a captured graph never points at a missing copy
+    const unsigned present = (P.K0 ? 1u : 0u) | (P.q0 ? 2u : 0u) | (P.Gamma ? 4u : 0u) | (P.fbar ? 8u : 0u) | (P.lbar ? 16u : 0u);
+    if (ws.B != B || ws.ne != ne || ws.present != present || ws.analytic != analytic || !ws.block) {
         SRI_CUDA(cudaStreamSynchronize(h->stream));
         if (ws.graph) { cudaGraphExecDestroy(ws.graph); ws.graph = nullptr; }
         if (ws.block) SRI_CUDA(cudaFree(ws.block));
         ws.block = nullptr; ws.B = -1;
-        const bool k0 = K0 != nullptr;
         auto up = [](size_t v) { return (v + 1) & ~(size_t)1; };  // 16-byte aligned pieces
+        // an optional array of `per_rod` doubles for `rods` rods, or nothing when the problem does not have it
+        auto opt = [&](unsigned bit, size_t per_rod, int64_t rods) { return (present & bit) ? up(per_rod * (size_t)rods) : (size_t)0; };
         const size_t state_doubles = up((sizeof(NewtonState) + 7) / 8);
         const size_t sz[] = {up((size_t)3 * N * B), up((size_t)4 * M * B), up((size_t)3 * M * B), up((size_t)3 * M * B), up((size_t)n * B), up((size_t)n * n * B),
-                             up((size_t)n * B), up((size_t)n * B), 8, up((size_t)3 * B), up((size_t)3 * B), k0 ? up((size_t)3 * N * B) : 0,
+                             up((size_t)n * B), up((size_t)n * B), 8, up((size_t)3 * B), up((size_t)3 * B), opt(1, 3 * N, B),
                              up((size_t)n * W), up((size_t)3 * N * W), up((size_t)4 * M * W), up((size_t)3 * M * W), up((size_t)n * W),
-                             up((size_t)3 * W), up((size_t)3 * W), k0 ? up((size_t)3 * N * W) : 0};
+                             up((size_t)3 * W), up((size_t)3 * W), opt(1, 3 * N, W),
+                             opt(2, 4, B), opt(4, 3 * N, B), opt(8, 3 * N, B), opt(16, 3 * N, B),
+                             opt(2, 4, W), opt(4, 3 * N, W), opt(8, 3 * N, W), opt(16, 3 * N, W)};
         size_t total = state_doubles + up(((size_t)B + 1) / 2);
         for (size_t v : sz) total += v;
         SRI_CUDA(cudaMalloc(&ws.block, total * sizeof(double)));
         double** fields[] = {&ws.K, &ws.Q, &ws.m, &ws.nn, &ws.g0, &ws.J, &ws.delta, &ws.qe, &ws.red, &ws.F, &ws.Mt, &ws.K0,
-                             &ws.qw, &ws.Kw, &ws.Qw, &ws.mw, &ws.gw, &ws.Fw, &ws.Mtw, &ws.K0w};
+                             &ws.qw, &ws.Kw, &ws.Qw, &ws.mw, &ws.gw, &ws.Fw, &ws.Mtw, &ws.K0w,
+                             &ws.q0, &ws.G, &ws.fb, &ws.lb, &ws.q0w, &ws.Gw, &ws.fbw, &ws.lbw};
         static_assert(sizeof(sz) / sizeof(sz[0]) == sizeof(fields) / sizeof(fields[0]), "one size per workspace field");
         size_t off = 0;
         for (size_t i = 0; i < sizeof(sz) / sizeof(sz[0]); ++i) { *fields[i] = sz[i] ? ws.block + off : nullptr; off += sz[i]; }
         ws.state = reinterpret_cast<NewtonState*>(ws.block + off); off += state_doubles;
         ws.sinfo = reinterpret_cast<int*>(ws.block + off);
-        ws.B = B; ws.ne = ne; ws.has_K0 = k0; ws.analytic = analytic;
+        ws.B = B; ws.ne = ne; ws.present = present; ws.analytic = analytic;
     }
     if (!ws.host_state) {
         SRI_CUDA(cudaMallocHost(reinterpret_cast<void**>(&ws.host_state), 2 * sizeof(NewtonState)));
@@ -1853,42 +1899,50 @@ int sri_newton_static_shape(sri_handle h, int64_t batch, int ne, const double* H
     SRI_CUDA(cudaMemsetAsync(ws.red, 0, 2 * sizeof(double), st));  // a rank without rods contributes (0, 0)
     if (B > 0) {
         SRI_CUDA(cudaMemcpyAsync(ws.qe, qe, sizeof(double) * n * B, cudaMemcpyDefault, st));
-        SRI_CUDA(cudaMemcpyAsync(ws.F, F_tip, sizeof(double) * 3 * B, cudaMemcpyDefault, st));
-        SRI_CUDA(cudaMemcpyAsync(ws.Mt, M_tip, sizeof(double) * 3 * B, cudaMemcpyDefault, st));
-        if (K0) SRI_CUDA(cudaMemcpyAsync(ws.K0, K0, sizeof(double) * 3 * N * B, cudaMemcpyDefault, st));
-        for (int d = 0; d < n && !analytic; ++d) {  // tip loads (and K0) of the forward-difference copies
-            SRI_CUDA(cudaMemcpyAsync(ws.Fw + (size_t)d * 3 * B, ws.F, sizeof(double) * 3 * B, cudaMemcpyDeviceToDevice, st));
-            SRI_CUDA(cudaMemcpyAsync(ws.Mtw + (size_t)d * 3 * B, ws.Mt, sizeof(double) * 3 * B, cudaMemcpyDeviceToDevice, st));
-            if (K0) SRI_CUDA(cudaMemcpyAsync(ws.K0w + (size_t)d * 3 * N * B, ws.K0, sizeof(double) * 3 * N * B, cudaMemcpyDeviceToDevice, st));
-        }
+        // the problem's inputs, and their replicas in each of the n forward-difference copies of the batch
+        struct Input { const double* src; double* dst; double* rep; size_t per_rod; };
+        const Input inputs[] = {{P.F_tip, ws.F, ws.Fw, 3}, {P.M_tip, ws.Mt, ws.Mtw, 3}, {P.K0, ws.K0, ws.K0w, (size_t)3 * N},
+                                {P.q0, ws.q0, ws.q0w, 4}, {P.Gamma, ws.G, ws.Gw, (size_t)3 * N}, {P.fbar, ws.fb, ws.fbw, (size_t)3 * N},
+                                {P.lbar, ws.lb, ws.lbw, (size_t)3 * N}};
+        for (const Input& in : inputs)
+            if (in.src) SRI_CUDA(cudaMemcpyAsync(in.dst, in.src, sizeof(double) * in.per_rod * B, cudaMemcpyDefault, st));
+        for (int d = 0; d < n && !analytic; ++d)
+            for (const Input& in : inputs)
+                if (in.src)
+                    SRI_CUDA(cudaMemcpyAsync(in.rep + (size_t)d * in.per_rod * B, in.dst, sizeof(double) * in.per_rod * B,
+                                             cudaMemcpyDeviceToDevice, st));
     }
     // every kernel launched from here on takes the device-side flag (lagged mode only); cleared on every way out
     struct SkipScope { sri_context* h; ~SkipScope() { h->skip = nullptr; } } skip_scope{h};
     h->skip = lagged ? &ws.state->done : nullptr;
 
-    auto evaluate = [&](int64_t rods, const double* q, double* K, double* Q, double* m, const double* F, const double* Mt,
-                        const double* k0, double* g, double* red, double* nout = nullptr) -> int {
+    // the loads of the batch (base) and of its forward-difference copies (w): workspace copies, NULL when absent
+    struct Loads { const double *F, *Mt, *K0, *q0, *G, *fb, *lb; };
+    const Loads base{ws.F, ws.Mt, ws.K0, ws.q0, ws.G, ws.fb, ws.lb}, w{ws.Fw, ws.Mtw, ws.K0w, ws.q0w, ws.Gw, ws.fbw, ws.lbw};
+    auto evaluate = [&](int64_t rods, const double* q, double* K, double* Q, double* m, const Loads& L, double* g, double* red,
+                        double* nout = nullptr) -> int {
         SRI_TRY(strain_from_modes_dev(h, rods, ne, q, K));
         sri::FusedParams p{};
         p.batch = rods; p.N = N; p.M = M; p.ops = h->d_ops16;
-        p.K = K; p.F_tip = F; p.M_tip = Mt; p.Q = Q; p.m = m; p.n = nout;
+        p.K = K; p.q0 = L.q0; p.Gamma = L.G; p.fbar = L.fb; p.lbar = L.lb; p.F_tip = L.F; p.M_tip = L.Mt;
+        p.Q = Q; p.m = m; p.n = nout;
         SRI_TRY(launch_fused(h, p));
-        return galerkin_residual_dev(h, rods, ne, K, k0, H, Q, nullptr, m, Mt, g, red);
+        return galerkin_residual_dev(h, rods, ne, K, L.K0, H, Q, L.q0, m, L.Mt, g, red);
     };
     // one Newton update + re-evaluation of the base point, all asynchronous on the handle's stream
     auto iterate = [&]() -> int {
         if (B == 0) return SRI_OK;
         const long long tq = (long long)n * W, tj = (long long)B * n * n, tu = (long long)n * B;
         if (analytic) {
-            SRI_TRY(shape_jacobian_dev(h, B, ne, H, ws.Q, nullptr, nullptr, ws.nn, ws.m, ws.Mt, ws.J));
+            SRI_TRY(shape_jacobian_dev(h, B, ne, H, ws.Q, ws.q0, ws.G, ws.nn, ws.m, ws.Mt, ws.J));
         } else {
             SRI_TRY(launch(fd_perturb_kernel, (unsigned)((tq + 255) / 256), 256, 0, st, B, n, fd_step, ws.qe, ws.qw, h->skip));
-            SRI_TRY(evaluate(W, ws.qw, ws.Kw, ws.Qw, ws.mw, ws.Fw, ws.Mtw, ws.K0w, ws.gw, nullptr));
+            SRI_TRY(evaluate(W, ws.qw, ws.Kw, ws.Qw, ws.mw, w, ws.gw, nullptr));
             SRI_TRY(launch(fd_jacobian_kernel, (unsigned)((tj + 255) / 256), 256, 0, st, B, n, fd_step, ws.gw, ws.g0, ws.J, h->skip));
         }
         SRI_TRY(solve_small_dev(h, B, n, ws.J, ws.g0, ws.delta, ws.sinfo));
         SRI_TRY(launch(newton_update_kernel, (unsigned)((tu + 255) / 256), 256, 0, st, B, n, ws.qe, ws.delta, ws.sinfo, ws.state, h->skip));
-        return evaluate(B, ws.qe, ws.K, ws.Q, ws.m, ws.F, ws.Mt, ws.K0, ws.g0, ws.red, analytic ? ws.nn : nullptr);
+        return evaluate(B, ws.qe, ws.K, ws.Q, ws.m, base, ws.g0, ws.red, analytic ? ws.nn : nullptr);
     };
     const double dof = (double)(total_dof > 0 ? total_dof : (int64_t)n * B);
     const int nranks = std::max(1, h->nccl_nranks);
@@ -1953,7 +2007,7 @@ int sri_newton_static_shape(sri_handle h, int64_t batch, int ne, const double* H
     };
 
     sri_newton_report rep{};
-    if (B > 0) SRI_TRY(evaluate(B, ws.qe, ws.K, ws.Q, ws.m, ws.F, ws.Mt, ws.K0, ws.g0, ws.red, analytic ? ws.nn : nullptr));
+    if (B > 0) SRI_TRY(evaluate(B, ws.qe, ws.K, ws.Q, ws.m, base, ws.g0, ws.red, analytic ? ws.nn : nullptr));
     rep.integrations = 1;
     unsigned long long singular = 0;
     int last_mirror = 0;
@@ -1992,7 +2046,7 @@ int sri_newton_static_shape(sri_handle h, int64_t batch, int ne, const double* H
             double red[2] = {0.0, 0.0};
             SRI_CUDA(cudaMemcpyAsync(red, ws.red, sizeof(red), cudaMemcpyDeviceToHost, st));
             SRI_CUDA(cudaStreamSynchronize(st));
-            if (reduce(red, reduce_ctx) != 0) return fail(SRI_ERR_INVALID_ARGUMENT, "sri_newton_static_shape: the reduction callback failed");
+            if (reduce(red, reduce_ctx) != 0) return fail(SRI_ERR_INVALID_ARGUMENT, std::string(who) + ": the reduction callback failed");
             rep.rms = dof > 0 ? std::sqrt(red[0] / dof) : 0.0;
             rep.max_abs = red[1];
             rep.rms_history[rep.history_len++] = rep.rms;
@@ -2013,6 +2067,24 @@ int sri_newton_static_shape(sri_handle h, int64_t batch, int ne, const double* H
     }
     if (report) *report = rep;
     return SRI_OK;
+}
+
+int sri_newton_static_shape(sri_handle h, int64_t batch, int ne, const double* H_diag, const double* F_tip,
+                            const double* M_tip, const double* K0, double* qe, double tol, int max_iter, double fd_step,
+                            int64_t total_dof, sri_allreduce_fn reduce, void* reduce_ctx, sri_newton_report* report) {
+    SRI_ENTER(h);
+    sri_static_problem P{};
+    P.batch = batch; P.ne = ne; P.H_diag = H_diag; P.F_tip = F_tip; P.M_tip = M_tip; P.K0 = K0;
+    return newton_static_problem(h, P, qe, tol, max_iter, fd_step, total_dof, reduce, reduce_ctx, report, "sri_newton_static_shape");
+}
+
+int sri_newton_static_problem(sri_handle h, const sri_static_problem* problem, double* qe, double tol, int max_iter,
+                              double fd_step, int64_t total_dof, sri_allreduce_fn reduce, void* reduce_ctx,
+                              sri_newton_report* report) {
+    SRI_ENTER(h);
+    if (!problem) return fail(SRI_ERR_INVALID_ARGUMENT, "sri_newton_static_problem: problem is required");
+    return newton_static_problem(h, *problem, qe, tol, max_iter, fd_step, total_dof, reduce, reduce_ctx, report,
+                                 "sri_newton_static_problem");
 }
 
 // ---- several devices in one process ------------------------------------------------------------------------------------
@@ -2186,14 +2258,19 @@ int sri_integrate_all_per_device(sri_multi_handle mh, const sri_rod_batch* per_d
     return SRI_OK;
 }
 
-int sri_newton_static_shape_sharded(sri_multi_handle mh, int64_t batch, int ne, const double* H_diag, const double* F_tip,
-                                    const double* M_tip, const double* K0, double* qe, double tol, int max_iter,
-                                    double fd_step, sri_newton_report* report) {
-    if (!mh) return fail(SRI_ERR_INVALID_ARGUMENT, "sri_newton_static_shape_sharded: null handle");
-    if (batch < 0 || ne < 1 || ne > 8 || !H_diag || (batch > 0 && (!F_tip || !M_tip || !qe)))
-        return fail(SRI_ERR_INVALID_ARGUMENT, "sri_newton_static_shape_sharded: bad arguments");
-    for (const void* p : {(const void*)H_diag, (const void*)F_tip, (const void*)M_tip, (const void*)K0, (const void*)qe})
-        if (p && is_device_pointer(p)) return fail(SRI_ERR_INVALID_ARGUMENT, "sri_newton_static_shape_sharded: host pointers only");
+}  // extern "C"
+
+// `who` names the entry point in error messages.
+static int newton_static_problem_sharded(sri_multi_handle mh, const sri_static_problem& P, double* qe, double tol, int max_iter,
+                                         double fd_step, sri_newton_report* report, const char* who) {
+    if (!mh) return fail(SRI_ERR_INVALID_ARGUMENT, std::string(who) + ": null handle");
+    const int64_t batch = P.batch;
+    const int ne = P.ne;
+    if (batch < 0 || ne < 1 || ne > 8 || !P.H_diag || (batch > 0 && (!P.F_tip || !P.M_tip || !qe)))
+        return fail(SRI_ERR_INVALID_ARGUMENT, std::string(who) + ": bad arguments");
+    for (const void* p : {(const void*)P.H_diag, (const void*)P.F_tip, (const void*)P.M_tip, (const void*)P.K0, (const void*)P.q0,
+                          (const void*)P.Gamma, (const void*)P.fbar, (const void*)P.lbar, (const void*)qe})
+        if (p && is_device_pointer(p)) return fail(SRI_ERR_INVALID_ARGUMENT, std::string(who) + ": host pointers only");
     const int G = (int)mh->handles.size(), N = mh->N, n = 3 * ne;
     ThreadReduce red;
     red.n = G;
@@ -2203,11 +2280,15 @@ int sri_newton_static_shape_sharded(sri_multi_handle mh, int64_t batch, int ne, 
         int64_t first = 0, last = 0;
         int r = sri_shard_range(batch, g, G, &first, &last);
         ThreadReduceCtx ctx{&red, g};
+        auto adv = [first](const double* p, size_t per_rod) { return p ? p + (size_t)first * per_rod : nullptr; };
+        sri_static_problem mine = P;
+        mine.batch = last - first;
+        mine.F_tip = adv(P.F_tip, 3); mine.M_tip = adv(P.M_tip, 3); mine.K0 = adv(P.K0, (size_t)3 * N);
+        mine.q0 = adv(P.q0, 4); mine.Gamma = adv(P.Gamma, (size_t)3 * N); mine.fbar = adv(P.fbar, (size_t)3 * N);
+        mine.lbar = adv(P.lbar, (size_t)3 * N);
         if (r == SRI_OK)
-            r = sri_newton_static_shape(mh->handles[g], last - first, ne, H_diag, F_tip ? F_tip + 3 * first : nullptr,
-                                        M_tip ? M_tip + 3 * first : nullptr, K0 ? K0 + (size_t)3 * N * first : nullptr,
-                                        qe ? qe + (size_t)n * first : nullptr, tol, max_iter, fd_step, (int64_t)n * batch,
-                                        thread_reduce_callback, &ctx, &reps[g]);
+            r = sri_newton_static_problem(mh->handles[g], &mine, qe ? qe + (size_t)n * first : nullptr, tol, max_iter, fd_step,
+                                          (int64_t)n * batch, thread_reduce_callback, &ctx, &reps[g]);
         if (r != SRI_OK) {  // release the shards waiting in the reduction
             std::lock_guard<std::mutex> lock(red.mu);
             red.failed = true;
@@ -2221,6 +2302,22 @@ int sri_newton_static_shape_sharded(sri_multi_handle mh, int64_t batch, int ne, 
         for (int g = 1; g < G; ++g) report->singular_solves += reps[g].singular_solves;
     }
     return SRI_OK;
+}
+
+extern "C" {
+
+int sri_newton_static_shape_sharded(sri_multi_handle mh, int64_t batch, int ne, const double* H_diag, const double* F_tip,
+                                    const double* M_tip, const double* K0, double* qe, double tol, int max_iter,
+                                    double fd_step, sri_newton_report* report) {
+    sri_static_problem P{};
+    P.batch = batch; P.ne = ne; P.H_diag = H_diag; P.F_tip = F_tip; P.M_tip = M_tip; P.K0 = K0;
+    return newton_static_problem_sharded(mh, P, qe, tol, max_iter, fd_step, report, "sri_newton_static_shape_sharded");
+}
+
+int sri_newton_static_problem_sharded(sri_multi_handle mh, const sri_static_problem* problem, double* qe, double tol,
+                                      int max_iter, double fd_step, sri_newton_report* report) {
+    if (!problem) return fail(SRI_ERR_INVALID_ARGUMENT, "sri_newton_static_problem_sharded: problem is required");
+    return newton_static_problem_sharded(mh, *problem, qe, tol, max_iter, fd_step, report, "sri_newton_static_problem_sharded");
 }
 
 int sri_generate_rods(sri_handle h, uint64_t seed, int64_t first_rod, int64_t batch, double* K, double* F_tip,

@@ -380,8 +380,10 @@ __device__ __forceinline__ double max_nan(double a, double b) { return (a > b ||
 // J_d^T lam, the exact transposed Jacobian of the discrete residual applied to lam (gKd: direct K-gradient of the
 // residual's VJP, gKi: K-gradient of the integration's VJP); rhs = jd - gqe (the negated residual r = gqe - jd, so that
 // the Newton update kernel lam -= J_a^-T rhs applies the step) and resid = max|r| / max|gqe| (max|r| when gqe = 0).  The
-// call after the last chain also writes the parameter gradients F-grad = -gFi, M-grad = -(gMd + gMi), H-grad = -gHw and
-// info = sinfo | vinfo << 8.  G lanes per rod as in galerkin_residual_kernel; NULL outputs are skipped.
+// call after the last chain also writes the parameter gradients F-grad = -gFi, M-grad = -(gMd + gMi), H-grad = -gHw,
+// q0-grad = -(gq0d + gq0i) and info = sinfo | vinfo << 8, and negates in place the Gamma, fbar and lbar gradients that the
+// last integration VJP wrote into the caller's buffers (no extra launch).  G lanes per rod as in galerkin_residual_kernel;
+// NULL outputs are skipped.
 struct AdjointRefineParams {
     long long batch;
     int N;
@@ -393,6 +395,9 @@ struct AdjointRefineParams {
     double* resid;       // [B]
     const double *gFi, *gMd, *gMi, *gHw;   // [B][3] (final call)
     double *gF, *gM, *gH;                  // [B][3] (final call)
+    const double *gq0d, *gq0i;             // [B][4] (final call)
+    double* gq0;                           // [B][4] (final call)
+    double *gGamma, *gfbar, *glbar;        // [B][3][N] (final call, negated in place)
     const int *sinfo, *vinfo;              // [B]
     int* info;                             // [B]
 };
@@ -419,6 +424,13 @@ __global__ void __launch_bounds__(256) static_adjoint_refine_kernel(AdjointRefin
                 const double pk = p.ptab[k * N + i];
 #pragma unroll
                 for (int c = 0; c < 3; ++c) acc[c][k] = fma(s[c], pk, acc[c][k]);
+            }
+#pragma unroll
+            for (int c = 0; c < 3; ++c) {
+                const long long o = b * 3 * N + c * N + i;
+                if (p.gGamma) p.gGamma[o] = -p.gGamma[o];
+                if (p.gfbar) p.gfbar[o] = -p.gfbar[o];
+                if (p.glbar) p.glbar[o] = -p.glbar[o];
             }
         }
     }
@@ -454,6 +466,7 @@ __global__ void __launch_bounds__(256) static_adjoint_refine_kernel(AdjointRefin
         if (p.gH) p.gH[o] = -p.gHw[o];
         if (p.info && sub == 0) p.info[b] = (p.sinfo ? p.sinfo[b] : 0) | ((p.vinfo ? p.vinfo[b] : 0) << 8);
     }
+    if (p.gq0 && b < p.batch && sub < 4) p.gq0[b * 4 + sub] = -(p.gq0d[b * 4 + sub] + p.gq0i[b * 4 + sub]);
     }  // chunks of this block
 }
 

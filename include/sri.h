@@ -32,7 +32,7 @@ extern "C" {
 #endif
 
 #define SRI_VERSION_MAJOR 0
-#define SRI_VERSION_MINOR 4
+#define SRI_VERSION_MINOR 5
 
 typedef enum sri_status {
     SRI_OK = 0,
@@ -295,10 +295,37 @@ typedef struct sri_newton_report {
     int64_t singular_solves; /* per-rod Newton systems found singular (zero pivot), summed over the iterations; those rods
                                 kept their qe in that iteration */
 } sri_newton_report;
+/* Tip-loaded rods with an identity clamp: sri_newton_static_problem with q0, Gamma, fbar and lbar NULL (the same kernels,
+ * results and launches). */
 int sri_newton_static_shape(sri_handle h, int64_t batch, int ne, const double* H_diag, const double* F_tip,
                             const double* M_tip, const double* K0, double* qe, double tol, int max_iter, double fd_step,
                             int64_t total_dof, sri_allreduce_fn reduce, void* reduce_ctx, sri_newton_report* report);
-/* Gradients of the static shape solution (implicit-function theorem): at an equilibrium qe* of sri_newton_static_shape
+
+/* A static shape problem with every input of the four-stage integration that the residual depends on (r0 moves the rod,
+ * not its shape, and is not part of it).  Distributed loads are dead loads: per unit length, in the global frame, independent
+ * of the shape (a follower load would make n depend on K).  Per-rod and per-node arrays are host or device pointers as
+ * everywhere. */
+typedef struct sri_static_problem {
+    int64_t batch;
+    int ne;                /* Legendre modes per strain component, 1..8: qe [batch][3*ne] */
+    const double* H_diag;  /* [3], host or device */
+    const double* F_tip;   /* [batch][3] */
+    const double* M_tip;   /* [batch][3] */
+    const double* K0;      /* [batch][3][N] or NULL (0) */
+    const double* q0;      /* [batch][4]    or NULL (identity): rotation of the clamped base */
+    const double* Gamma;   /* [batch][3][N] or NULL (e1) */
+    const double* fbar;    /* [batch][3][N] or NULL (0), global frame (e.g. the weight (0, 0, -g)) */
+    const double* lbar;    /* [batch][3][N] or NULL (0), global frame */
+} sri_static_problem;
+/* The Newton loop of sri_newton_static_shape (every argument, the report, both Jacobians, the lagged device-side test, the
+ * NCCL and callback reductions and the graph replay as documented there) for a sri_static_problem: q0, Gamma, fbar and lbar
+ * reach the integration, the residual and the analytic Jacobian, and the forward-difference copies carry them too.  The
+ * analytic Jacobian stays exact under dead loads: n does not depend on K, it only varies along the rod. */
+int sri_newton_static_problem(sri_handle h, const sri_static_problem* problem, double* qe, double tol, int max_iter,
+                              double fd_step, int64_t total_dof, sri_allreduce_fn reduce, void* reduce_ctx,
+                              sri_newton_report* report);
+/* Tip-loaded rods with an identity clamp: sri_static_problem_vjp with q0, Gamma, fbar and lbar NULL.
+ * Gradients of the static shape solution (implicit-function theorem): at an equilibrium qe* of sri_newton_static_shape
  * (g(qe*; F_tip, M_tip, K0, H) = 0, q0 = identity, Gamma = e1, no distributed loads) and a cotangent gqe of qe*, solves
  * J_d^T lam = gqe per rod, J_d the exact Jacobian of the discrete residual, and returns theta-grad = -(dg/dtheta)^T lam:
  *   gF_tip, gM_tip [batch][3];  gK0 [batch][3][N];  gH [batch][3] (per rod: a caller with one H sums over the batch).
@@ -316,11 +343,38 @@ int sri_newton_static_shape(sri_handle h, int64_t batch, int ne, const double* H
 int sri_static_shape_vjp(sri_handle h, int64_t batch, int ne, const double* H_diag, const double* F_tip, const double* M_tip,
                          const double* K0, const double* qe, const double* gqe, int refine_steps, double* gF_tip,
                          double* gM_tip, double* gK0, double* gH, double* lambda, double* resid, int* info);
+/* Outputs of sri_static_problem_vjp.  Every pointer may be NULL (skipped); each is written, not accumulated. */
+typedef struct sri_static_problem_grad {
+    double* gF_tip;  /* [batch][3] */
+    double* gM_tip;  /* [batch][3] */
+    double* gK0;     /* [batch][3][N] */
+    double* gH;      /* [batch][3], per rod: a caller with one H sums over the batch */
+    double* gq0;     /* [batch][4]    (at q0 = identity when problem->q0 is NULL) */
+    double* gGamma;  /* [batch][3][N] (at Gamma = e1 when problem->Gamma is NULL) */
+    double* gfbar;   /* [batch][3][N] (0 at node 0, whose sample the integration does not use) */
+    double* glbar;   /* [batch][3][N] (0 at node 0) */
+    double* lambda;  /* [batch][3*ne] the adjoint solution */
+    double* resid;   /* [batch] max|gqe - J_d^T lam| / max|gqe| */
+    int* info;       /* [batch] 0, or s | v << 8 as in sri_static_shape_vjp */
+} sri_static_problem_grad;
+/* sri_static_shape_vjp for a sri_static_problem: the forward state and J_a are those of the problem's inputs, J_d^T lam is the
+ * residual VJP and sri_integrate_all_vjp with q0 and Gamma, and theta-grad = -(dg/dtheta)^T lam also for theta = q0, Gamma,
+ * fbar, lbar (gq0 sums the residual's direct dependence on the base rotation and the integration's).  The refinement, its
+ * accuracy per N, the workspace, host / device buffers and SRI_ERR_SINGULAR are those of sri_static_shape_vjp; a rod with a
+ * non-finite load is flagged in its own info[b] and leaves the other rods' results unchanged. */
+int sri_static_problem_vjp(sri_handle h, const sri_static_problem* problem, const double* qe, const double* gqe, int refine_steps,
+                           const sri_static_problem_grad* grads);
 /* The same solve over all devices of mh from one host process: HOST pointers, rods sharded by index as in
- * sri_integrate_all_sharded, one host thread per device, the norms reduced between the threads (no NCCL, no MPI). */
+ * sri_integrate_all_sharded, one host thread per device, the norms reduced between the threads (no NCCL, no MPI).
+ * Tip-loaded rods with an identity clamp: sri_newton_static_problem_sharded with q0, Gamma, fbar and lbar NULL. */
 int sri_newton_static_shape_sharded(sri_multi_handle mh, int64_t batch, int ne, const double* H_diag, const double* F_tip,
                                     const double* M_tip, const double* K0, double* qe, double tol, int max_iter,
                                     double fd_step, sri_newton_report* report);
+/* sri_newton_static_problem over all devices of mh: every per-rod and per-node array of the problem and qe are HOST pointers,
+ * sharded by rod index as in sri_integrate_all_sharded; each rod's qe is bit for bit that of a one-device solve taking the same
+ * iterations (the norms are added in shard order, so the rms history agrees to round-off). */
+int sri_newton_static_problem_sharded(sri_multi_handle mh, const sri_static_problem* problem, double* qe, double tol,
+                                      int max_iter, double fd_step, sri_newton_report* report);
 
 /* ---- NCCL residual-norm reduction (BASELINE configs[4]; SURVEY 8e: the only collective, Newton driver only) -----------
  * libnccl.so.2 is opened at run time (dlopen), the library does not link against it.  One process per GPU:
