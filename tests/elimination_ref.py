@@ -69,7 +69,15 @@ def x_to_q(x, M):
 def system(tab: Tables, K, q0=None):
     """(C [B][4M][4M], b [B][4M]) in float64, entries rounded exactly as the kernels form them."""
     B, M = K.shape[0], tab.M
-    s = -0.5 * tab.S                                            # the kernels' table entry (exact)
+    C = quaternion_operator(-0.5 * tab.S, K)                    # the kernels' table entry -1/2 S_ij (exact)
+    q0 = np.tile([1.0, 0.0, 0.0, 0.0], (B, 1)) if q0 is None else q0
+    b = (tab.g[None, :, None] * q0[:, None, :]).reshape(B, 4 * M)
+    return C, b
+
+
+def quaternion_operator(s, K):
+    """The real 4M x 4M matrix [B][4M][4M] of x -> (sum_j x_j (x) c_ij)_i with c_ij = (delta_ij, fl(s_ij K_j)), node-major."""
+    B, M = K.shape[0], s.shape[0]
     v = s[None, :, :, None] * np.swapaxes(K[:, :, :M], 1, 2)[:, None, :, :]  # [B][i][j][3] = fl(s_ij K_j)
     w = np.broadcast_to(np.eye(M), (B, M, M))
     C = np.zeros((B, M, 4, M, 4))
@@ -78,9 +86,7 @@ def system(tab: Tables, K, q0=None):
     for r in range(4):
         for c in range(4):
             C[:, :, r, :, c] = rows[r][c]
-    q0 = np.tile([1.0, 0.0, 0.0, 0.0], (B, 1)) if q0 is None else q0
-    b = (tab.g[None, :, None] * q0[:, None, :]).reshape(B, 4 * M)
-    return C.reshape(B, 4 * M, 4 * M), b
+    return C.reshape(B, 4 * M, 4 * M)
 
 
 def residual(C, x, b):
@@ -109,8 +115,8 @@ def refine_step(C, x, b):
 
 def refined_solve(C, b, steps: int = 4, tol=1e-17):
     """float64 LAPACK solve, then `steps` refinement steps.  Raises unless the last correction is below tol relative
-    (scalar or one value per rod).  Returns x in long double."""
-    x = np.linalg.solve(C, b[..., None])[..., 0].astype(LD)
+    (scalar or one value per rod).  b may be float64 or long double.  Returns x in long double."""
+    x = np.linalg.solve(C, b.astype(np.float64)[..., None])[..., 0].astype(LD)
     for _ in range(steps):
         x, rel = refine_step(C, x, b)
     bad = np.nonzero(rel > tol)[0]
