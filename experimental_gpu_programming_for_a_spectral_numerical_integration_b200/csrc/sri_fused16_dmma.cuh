@@ -10,16 +10,17 @@
 // is stored as the REAL 64 x 16 matrix  Cr[4 i + r][j] = component r of c_ij  (column 15 = b_i), i.e. 8 x 2 DMMA
 // accumulator tiles of 8 x 8 = 32 doubles per lane.  With vec(a (x) b) = Rmat(b) vec(a), elimination step k is
 //      U'  = Rmat(c_kk^-1) U            U = pivot row as a 4 x 16 matrix (one DMMA per column tile)
-//      Cr -= [...; Rmat(c_kk - 1); Rmat(c_k+1,k); ...] U'     (rank-4 update of the tile rows below the pivot, k = 4)
+//      Cr -= [...; Rmat(c_k+1,k); Rmat(c_k+2,k); ...] U'      (rank-4 update of the tile rows below the pivot, k = 4)
 // 4 x 4 real blocks appear only in the A operand (the multipliers); the matrix itself stays in quaternion (4-vector)
 // form, so the DMMAs execute exactly the 16 FMAs per quaternion multiply-add of the scalar kernel.
 // Per step the LSU only moves the pivot row into B-fragment layout (2 SHFL.64 per column tile), one component of the
 // pivot element and its squared norm to every lane (2 SHFL.64) and the pivot column into A-fragment layout (1 SHFL.64
 // per live row tile), and stores -U' to shared memory.  The back-substitution then runs with the rows on the n axis:
 //      -Q_i = -U'_i,15 + sum_{j>i} Lmat(-Q_j) (-U'_ij),    vec(a (x) b) = Lmat(a) vec(b),
-// so one DMMA (A = Lmat(-Q_j), B = column j of -U' over 8 rows) serves 8 rows.  Per rod: 107 updates, 23
-// normalisations, 20 back-substitution DMMAs.  Stages 2-4 are [16 x 16] x [16 x 3] DMMA contractions in the same
-// warp (16 DMMAs; Q never leaves the SM): 166 DMMAs in all.
+// so one DMMA (A = Lmat(-Q_j), B = column j of -U' over 8 rows) serves 8 rows.  Per rod at N = 16: 96 updates (the
+// padding row sits above row 0, see kRowOff; the N < 16 instantiation keeps it below and issues up to 107), 23
+// normalisations, 20 back-substitution DMMAs.  Stages 2-4 are [16 x 16] x [16 x 3] DMMA contractions in the same warp
+// (16 DMMAs; Q never leaves the SM): 155 DMMAs in all.
 //
 // Pivoting: the order is static (pivot k = row k).  The left-preconditioned operator I - 1/2 S diag(kappa) has
 // |c_kk| >= 1 and measured sub-diagonal growth <= 0.15 for |K| <= 10 and <= 2.4 for |K| <= 300, so a search would
@@ -141,6 +142,11 @@ __global__ void __launch_bounds__(kDmmaThreads, SRI_DMMA_MINBLOCKS) fused16_dmma
 
     const int M = MS ? MS : p.M;
     const int N = M + 1;
+    // Tile position of quaternion row i: i + kRowOff (tile row (i + kRowOff) / 2, half (i + kRowOff) % 2).  At M = 15
+    // the padding row sits at position 0, above row 0, so the rows below pivot k fill exactly 7 - k/2 tile rows and the
+    // padding is never updated.  At runtime M (< 15) the rows keep positions 0..M-1 so that every tile index stays a
+    // compile-time constant.
+    constexpr int kRowOff = (MS == 15) ? 1 : 0;
     // fragment coordinates of this lane
     const int rho = lane >> 2, cp = lane & 3;  // C fragment: row rho, columns 2cp, 2cp+1
     const int hi = rho >> 2, rr = rho & 3;     // quaternion row within the tile, component
@@ -154,21 +160,12 @@ __global__ void __launch_bounds__(kDmmaThreads, SRI_DMMA_MINBLOCKS) fused16_dmma
     // Rmat(b)[r][s] = sg(r,s) b[r^s]: rows (+,-,-,-), (+,+,+,-), (+,-,+,+), (+,+,-,+)
     const unsigned neg_tab = 0x428Eu;  // bit (4r+s) set where sg(r,s) = -1: r0: s1,s2,s3; r1: s3; r2: s1; r3: s2
     const unsigned sgL_mask = ((neg_tab >> (4 * rr + cp)) & 1u) << 31;
-    const double dpiv0 = (hi == 0 && rr == cp) ? 1.0 : 0.0;  // the pivot's tile row is live only for even k
     const unsigned hi_mask = hi ? 0x7fffffffu : 0u;
     // normalisation operand: B[q = cp][n = rho]; even n = 2 s' carries Rmat(conj c)[s'][q] = sg(s',q) conj(c)[s'^q]
     // (odd columns feed C-fragment register 1, which is discarded: don't-care)
     const int sp = rho >> 1;
     const int idxN = sp ^ cp;
     const unsigned sgN_mask = ((((neg_tab >> (4 * sp + cp)) & 1u) != 0) != (idxN != 0)) ? 0x80000000u : 0u;
-    // identity entries of the assembly: tile (t, ct), register e holds delta_ij iff rr == 0, hi == e, cp == t - 4 ct
-    const int diag_code = (rr == 0) ? (4 * hi + cp) : -1;
-    // -U' store of step k: lane (rho, cp) holds component cp of column 8 ct + rho
-    double* const ustl = scr + DmmaScratch::ust + 92 * rho + cp;
-    // B-fragment read offset into a [4][20] right-hand side
-    const int offb = (rho < 3 ? rho : 3) * 20 + cp;
-    // stages 2+3 in one contraction: columns 0..2 = r' (bs), columns 3..5 = reversed fbar (fbs), the rest the zero row of bs
-    const int offb23 = (rho < 3 ? DmmaScratch::bs + rho * 20 : (rho < 6 ? DmmaScratch::fbs + (rho - 3) * 20 : DmmaScratch::bs + 60)) + cp;
 
     const long long stride = (long long)gridDim.x * kWarps;
     const long long rod0 = (long long)blockIdx.x * kWarps + warp;
@@ -191,11 +188,17 @@ __global__ void __launch_bounds__(kDmmaThreads, SRI_DMMA_MINBLOCKS) fused16_dmma
     cp_async_commit();
 
     int it = 0;
-    for (long long rod = rod0; rod < p.batch; rod += stride, ++it) {
+    for (long long rod = rod0; rod < p.batch; ++it) {
         const int cur = it & 1;
+        const long long next = rod + stride;
         // ---- prefetch: this rod's late inputs (nodal loads shifted to reduced rows, boundary values into k slot 15)
         //      and the next rod's strain samples -------------------------------------------------------------------
-        if (row < N) {
+        //      (the lane is re-read here, before the elimination and before the stages, so that the lane constants of
+        //      each phase are derived where they are used and not held, or spilled, across the elimination)
+        int lp;
+        asm volatile("mov.u32 %0, %%laneid;" : "=r"(lp));
+        if ((lp & 15) < N) {
+            const int row = lp & 15, half = lp >> 4;
             const int c0 = half ? 2 : 0, c1 = half ? 3 : 2;  // half 0: components 0, 1; half 1: component 2
             for (int c = c0; c < c1; ++c) {
                 if (p.fbar && row >= 1) cp_async8(scr + DmmaScratch::fbs + 20 * c + (M - row), p.fbar + (rod * 3 + c) * N + row);  // flipped, see stages 2+3
@@ -206,7 +209,7 @@ __global__ void __launch_bounds__(kDmmaThreads, SRI_DMMA_MINBLOCKS) fused16_dmma
         if (lane < 3) { if (p.F_tip) cp_async8(scr + DmmaScratch::fbs + 20 * lane + 15, p.F_tip + rod * 3 + lane); }
         else if (lane >= 4 && lane < 7) { if (p.M_tip) cp_async8(scr + DmmaScratch::xs + 20 * (lane - 4) + 15, p.M_tip + rod * 3 + lane - 4); }
         else if (lane >= 8 && lane < 11) { if (p.r0) cp_async8(scr + DmmaScratch::bs + 20 * (lane - 8) + 15, p.r0 + rod * 3 + lane - 8); }
-        if (rod + stride < p.batch) prefetch_K(rod + stride, cur ^ 1);
+        if (next < p.batch) prefetch_K(next, cur ^ 1);
         cp_async_commit();
         cp_async_wait<1>();  // everything but the group just committed: this rod's K and q0 have landed
         __syncwarp();
@@ -215,6 +218,12 @@ __global__ void __launch_bounds__(kDmmaThreads, SRI_DMMA_MINBLOCKS) fused16_dmma
         // ---- stage 1: assemble Cr = delta - 1/2 S_ij (0,K_j) | g_i q0 in C-fragment layout -------------------------
         double c[8][2][2];
         {
+            // identity entries: register e of tile (t, ct) holds delta_ij iff rr == 0 and 4 hi + cp equals the
+            // compile-time code of the diagonal entry in that register.  The lane is re-read here so that the eight
+            // selected 1.0s are not held (and spilled) across the rod loop.
+            int ln;
+            asm volatile("mov.u32 %0, %%laneid;" : "=r"(ln));
+            const int diag_code = ((ln >> 2) & 3) == 0 ? 4 * (ln >> 4) + (ln & 3) : -1;
             double kq[2][2];
 #pragma unroll
             for (int ct = 0; ct < 2; ++ct) {
@@ -225,11 +234,16 @@ __global__ void __launch_bounds__(kDmmaThreads, SRI_DMMA_MINBLOCKS) fused16_dmma
             for (int t = 0; t < 8; ++t)
 #pragma unroll
                 for (int ct = 0; ct < 2; ++ct) {
-                    const double2 s = *reinterpret_cast<const double2*>(stx + (2 * t + hi) * 16 + 8 * ct + 2 * cp);
+                    // position 2t + hi holds row 2t + hi - kRowOff; the padding row reads Stx row 15, which is zero
+                    const double2 s = *reinterpret_cast<const double2*>(stx + ((2 * t + hi - kRowOff) & 15) * 16 + 8 * ct + 2 * cp);
 #pragma unroll
                     for (int e = 0; e < 2; ++e) {
-                        const int dcode = 4 * e + (t - 4 * ct);  // compile-time
-                        const bool candidate = (t - 4 * ct >= 0) && (t - 4 * ct < 4) && !(ct == 1 && t == 7 && e == 1);
+                        // compile-time: register e of tile (t, ct) holds column j = 8 ct + 2 cp + e, and j is the
+                        // row of half dh = (e + kRowOff) & 1 in lane column cp = dcp + 4 ct; no identity at j = 15
+                        const int dh = (e + kRowOff) & 1;
+                        const int dcp = (2 * t + dh - kRowOff - e) / 2 - 4 * ct;
+                        const int dcode = 4 * dh + dcp;
+                        const bool candidate = (dcp >= 0) && (dcp < 4) && (8 * ct + 2 * dcp + e < 15);
                         const double d = (candidate && diag_code == dcode) ? 1.0 : 0.0;
                         c[t][ct][e] = fma(e ? s.y : s.x, kq[ct][e], d);
                     }
@@ -238,13 +252,17 @@ __global__ void __launch_bounds__(kDmmaThreads, SRI_DMMA_MINBLOCKS) fused16_dmma
         // ---- forward elimination over the quaternions on DMMA, static pivot order, software pipelined ----------
         // Step k normalises pivot row k, stores it (-U'_k) to shared memory and eliminates column k from the rows
         // below it.  A stored pivot row is never read from the tiles again, so step k updates only tile rows
-        // t >= (k+1)/2 (the pivot's own tile row only while row k+1 shares it), and the last step updates nothing.
+        // t >= (k+1+kRowOff)/2, the tile row of row k+1 and those below it, and the last step updates nothing.
         // Iteration k issues the rank-4 update of step k and, behind it, everything step k+1 needs: its tile row, the
         // first live one, is updated first, then the next pivot row is gathered and normalised; each la[t] is
         // re-gathered for step k+1 as soon as tile row t has been updated.  k = -1 is the prologue (no update).
         // Scalar FP64 instructions share the pipe with the DMMAs and queue behind them, so the serial scalar chain is
         // kept to three operations per step: U (x) conj(c_kk) is itself a DMMA, whose (column k, w) entry is |c_kk|^2,
         // and its reciprocal (MUFU seed, e = 1 - nu r0, t2 = e + e^2) is folded into the scaling of that product.
+        // -U' store of step k: lane (rho, cp) holds component cp of column 8 ct + rho
+        int lu;
+        asm volatile("mov.u32 %0, %%laneid;" : "=r"(lu));
+        double* const ustl = scr + DmmaScratch::ust + 92 * (lu >> 2) + (lu & 3);
         bool bad = false;
         const int growth_log = p.growth_log;
         double la[8], un[2];
@@ -253,7 +271,9 @@ __global__ void __launch_bounds__(kDmmaThreads, SRI_DMMA_MINBLOCKS) fused16_dmma
             const int kn = k + 1;  // the step being prepared
             const bool upd = (k >= 0) && (k < 14) && (MS != 0 || k < M - 1);
             const bool prep = (kn < 15) && (MS != 0 || kn < M);
-            const int nt = (kn >> 1) & 7, nh = kn & 1, nc = (kn >> 3) & 1, ncp = (kn & 7) >> 1, ne = kn & 1;
+            // the next pivot row sits at tile position kn + kRowOff; its column is kn
+            const int nt = ((kn + kRowOff) >> 1) & 7, nh = (kn + kRowOff) & 1;
+            const int nc = (kn >> 3) & 1, ncp = (kn & 7) >> 1, ne = kn & 1;
             // 1. step k on the tile row of the next pivot (= its first live tile row)
             if (upd) {
 #pragma unroll
@@ -288,7 +308,8 @@ __global__ void __launch_bounds__(kDmmaThreads, SRI_DMMA_MINBLOCKS) fused16_dmma
                 if (hn < 0x05000000 || hn >= 0x7ff00000) thr = -1;  // zero / tiny / negative / inf / NaN pivot norm
             }
             // 2. step k on the other live tile rows; la[t] is re-gathered for step k+1 once tile row t is done (step
-            //    k+1 needs tile rows t >= (kn+1)/2: the next pivot's own tile row only when kn is even)
+            //    k+1 needs tile rows t >= (kn+1+kRowOff)/2: the next pivot's own tile row only when the pivot is its
+            //    upper half, nh == 0)
             const int srcL = srcL_base + ncp;
 #pragma unroll
             for (int t = nt; t < 8; ++t) {
@@ -301,8 +322,8 @@ __global__ void __launch_bounds__(kDmmaThreads, SRI_DMMA_MINBLOCKS) fused16_dmma
                     const double v = __shfl_sync(0xffffffffu, c[t][nc][ne], srcL);
                     const unsigned h = (unsigned)__double2hiint(v) & 0x7fffffffu;
                     mx = max(mx, t != nt ? h : (h & hi_mask));
+                    // on the pivot's own tile this also updates the pivot row, which is stored and never read again
                     la[t] = flip_sign(v, sgL_mask);
-                    if (t == nt) la[t] -= dpiv0;  // pivot row: Rmat(c_kk - 1) leaves the normalised row
                 }
             }
             // 3. -U' = -(U (x) conj c_kk) / nu for the next step, and into the store for the back-substitution
@@ -390,6 +411,14 @@ __global__ void __launch_bounds__(kDmmaThreads, SRI_DMMA_MINBLOCKS) fused16_dmma
                 if (row < 15) { double* b = scr + DmmaScratch::bs + row; b[0] = bv0; b[20] = bv1; b[40] = bv2; }
             }
             __syncwarp();
+            // B-fragment read offsets (the lane is re-read so that they are not held across the elimination):
+            // into a [4][20] right-hand side, and for stages 2+3 in one contraction: columns 0..2 = r' (bs),
+            // columns 3..5 = reversed fbar (fbs), the rest the zero row of bs
+            int ls;
+            asm volatile("mov.u32 %0, %%laneid;" : "=r"(ls));
+            const int brho = ls >> 2, bcp = ls & 3;
+            const int offb = (brho < 3 ? brho : 3) * 20 + bcp;
+            const int offb23 = (brho < 3 ? DmmaScratch::bs + brho * 20 : (brho < 6 ? DmmaScratch::fbs + (brho - 3) * 20 : DmmaScratch::bs + 60)) + bcp;
             double acc[2][2];
             // stages 2 and 3 in ONE contraction against Dn_NN^-1: the Chebyshev matrix is centro-antisymmetric, so
             // -D_TT^-1 = J Dn_NN^-1 J (J = exchange matrix; 4e-16 on the as-built inverses, SURVEY T11) and gT = J g, hence
@@ -444,6 +473,7 @@ __global__ void __launch_bounds__(kDmmaThreads, SRI_DMMA_MINBLOCKS) fused16_dmma
             }
         }
         __syncwarp();  // scratch is reused by the next iteration
+        rod = next;
     }
     cp_async_wait<0>();
 }

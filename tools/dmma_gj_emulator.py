@@ -140,11 +140,15 @@ def w_col(j):
 W_DOUBLES = 740
 
 
-def solve_rod_lu(Stx, K, q0, M, growth=8.0, stats=None):
+def solve_rod_lu(Stx, K, q0, M, growth=8.0, stats=None, row_offset=0):
     """Same system and same pivot order as solve_rod, on the kernel's schedule:
-    forward  step k updates only tile rows t >= (k+1)//2 (rows at or above a stored pivot row are dead); the
-             last step updates nothing; -U'_k (B-fragment layout: lane holds component CP of column 8ct+RHO) is
-             stored to W[w_col(8ct+RHO) + 4k + CP].
+    layout   quaternion row i sits at tile position p = i + row_offset (tile row p // 2, half p % 2); the kernel uses
+             row_offset = 1 at M = 15 (fused16_dmma_kernel<15>: the padding row above row 0, position 0, reading the
+             all-zero Stx row 15) and 0 otherwise (<0>: rows 0..M-1 at positions 0..M-1).  Columns do not move.
+    forward  step k updates only tile rows t >= (k+1+row_offset)//2, the tile row of row k+1 and those below it (rows
+             at or above a stored pivot row are dead, and the pivot row itself is never read from the tiles again, so
+             its multiplier is plain Rmat(c_kk)); the last step updates nothing; -U'_k (B-fragment layout: lane holds
+             component CP of column 8ct+RHO) is stored to W[w_col(8ct+RHO) + 4k + CP].
     backward with C' = -Q accumulated in one C tile per 8-row block (C'[s][n] = row 8b+n, component s; m >= 4 zero):
              -Q_i = W_i,15 + sum_{j>i} Lmat(-Q_j) W_ij, j = M-1..0; A = Lmat(C'_j) by one shuffle and a sign,
              B = W column j over the block (one contiguous 32-double read).
@@ -159,7 +163,7 @@ def solve_rod_lu(Stx, K, q0, M, growth=8.0, stats=None):
     for t in range(8):
         for ct in range(2):
             for e in range(2):
-                i = 2 * t + HI
+                i = (2 * t + HI - row_offset) & 15  # position 0 at row_offset 1: Stx row 15, all zero
                 j = 8 * ct + 2 * CP + e
                 diag = ((R == 0) & (i == j) & (j < 15)).astype(np.float64)
                 c[t, ct, e] = Stx[i, j] * kx[R, j] + diag
@@ -173,9 +177,10 @@ def solve_rod_lu(Stx, K, q0, M, growth=8.0, stats=None):
     conj = np.where(idxN == 0, 1.0, -1.0)
     sgN = np.where(n_even, -SG[sp, CP] * conj, 0.0)
     for k in range(M):
-        kt, kh, kc, kcp, ke = k >> 1, k & 1, k >> 3, (k & 7) >> 1, k & 1
+        kt, kh = (k + row_offset) >> 1, (k + row_offset) & 1  # tile row and half of the pivot row
+        kc, kcp, ke = k >> 3, (k & 7) >> 1, k & 1  # tile, lane column and register of the pivot column
         cts = [ct for ct in range(2) if 8 * ct + 7 > k]
-        t0 = (k + 1) >> 1  # first live tile row: kt itself only while the row below the pivot (2kt + 1) shares it
+        t0 = (k + 1 + row_offset) >> 1  # tile row of row k + 1: kt itself only while the pivot is its upper half
         src = 16 * kh + 4 * CP + (LANES >> 3)
         Ub = {}
         for ct in range(kc, 2):
@@ -197,10 +202,7 @@ def solve_rod_lu(Stx, K, q0, M, growth=8.0, stats=None):
                 colmax = np.maximum(colmax, np.abs(v))
             else:  # t == kt, kh == 0: the row below the pivot in the same tile
                 colmax = np.maximum(colmax, np.where(HI > kh, np.abs(v), 0.0))
-            a = sgL * v
-            if t == kt:
-                a = a - ((HI == kh) & (R == CP)).astype(np.float64)
-            La[t] = a
+            La[t] = sgL * v
         if not (colmax.max() ** 2 <= growth * growth * nu[0]) or not (nu[0] > 1e-300):
             flagged = True
         for ct in cts:
